@@ -231,8 +231,11 @@ void orc_grid_posterior(int M, int S, const double* lj, double* post, double* ma
   }
 }
 
-/* inverse normal cdf: Acklam's rational start + two Halley steps on erfc => ~1 ulp */
+/* inverse normal cdf: Acklam's rational start + two Halley steps on erfc => ~1 ulp.  Upper half
+ * by symmetry: 1 - p is exact there, while a Halley residual formed against p itself keeps only
+ * the absolute precision of p (~1e-16), i.e. ~1e-16 / pdf(x) in x (1e-10 at x = 5). */
 static double ndtri_(double p) {
+  if (p > 0.5) return -ndtri_(1.0 - p);
   static const double a[] = {-3.969683028665376e+01, 2.209460984245205e+02, -2.759285104469687e+02,
                              1.383577518672690e+02, -3.066479806614716e+01, 2.506628277459239e+00};
   static const double b[] = {-5.447609879822406e+01, 1.615858368580409e+02, -1.556989798598866e+02,

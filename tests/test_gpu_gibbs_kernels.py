@@ -1,0 +1,448 @@
+"""K5 Gibbs, one compiled kernel at a time, against the numpy oracle.
+
+``pbx_gibbs_mvn_run`` picks one of 38 instantiations (36 reachable) of
+``gibbs_mvn_kernel<DQ, kSweepRec, false, NT>`` and ``gibbs_mvn_mma_kernel<DQ, kPair, NT, kDens>``
+from the dimension, the step alignment, the chain count and whether densities are recorded.
+``_instantiation`` restates that choice; the parity cases below run every reachable
+instantiation with injected uniforms, a model with real truncation limits in every draw regime
+of the table ndtri, and the native Philox stream at nonzero ``step0`` / ``chain0``."""
+import numpy as np
+import pytest
+from conftest import relerr
+from gpu_util import engine, dev, tcd_to_tdc, host
+from oracle import np_oracle as o
+from oracle import philox
+
+# trajectories against scipy's ndtri; see test_gpu_gibbs.py and the band model below
+GTOL = 1e-12
+LIN_TOL = 1e-11
+
+GB, GM = "gibbs_mvn_kernel", "gibbs_mvn_mma_kernel"
+
+
+# ---------------------------------------------------------------------------------------------
+# dispatch mirror (pbx_gibbs_mvn_run -> gibbs_launch<DQ> -> gibbs_launch_nt<DQ, NT>)
+# ---------------------------------------------------------------------------------------------
+def _dq(d):
+    for dq in (1, 2, 4, 8, 16):
+        if d <= 4 * dq:
+            return dq
+    return 32
+
+
+def _nt(C, sm_count):
+    """128 threads while there are too few chains for 3 CTAs of 64 chains per SM, else 256."""
+    return 128 if C < 3 * 64 * sm_count else 256
+
+
+def _instantiation(d, C, T, thin, step0, want_prob, sm_count):
+    """(kernel, DQ, flag, NT, kDens) launched for ``T >= 1`` steps of ``C`` chains in ``d``
+    dimensions from ``step0``, recording every ``thin`` steps (densities too if
+    ``want_prob``).  ``flag`` is kSweepRec for gibbs_mvn_kernel and kPair for
+    gibbs_mvn_mma_kernel."""
+    assert 1 <= d <= 128 and C >= 1 and T >= 1 and thin >= 1 and step0 >= 0
+    dq, nt = _dq(d), _nt(C, sm_count)
+    whole = thin % d == 0 and step0 % d == 0 and T % d == 0
+    if dq >= 2 and whole:
+        return (GM, dq, d % 8 == 0, nt, dq == 16 and d == 64 and bool(want_prob))
+    return (GB, dq, dq == 1 and whole, nt, False)
+
+
+COMPILED = {(GB, dq, sr, nt, False) for dq in (1, 2, 4, 8, 16, 32)
+            for sr in ((False, True) if dq == 1 else (False,)) for nt in (128, 256)} | \
+           {(GM, dq, kp, nt, kd) for dq in (2, 4, 8, 16, 32) for kp in (False, True)
+            for nt in (128, 256) for kd in ((False, True) if dq == 16 else (False,))}
+# kDens without kPair needs d = 64 with d % 8 != 0
+UNREACHABLE = {(GM, 16, False, nt, True) for nt in (128, 256)}
+REACHABLE = COMPILED - UNREACHABLE
+
+
+def _chains(size, sm_count):
+    """A ragged chain count: partial last warp and partial last CTA at either width."""
+    return 101 if size == "small" else 3 * 64 * sm_count + 37
+
+
+def _cta_chains(C, sm_count):
+    return _nt(C, sm_count) // 32 * 8
+
+
+def _sample(C, width, n=96, seed=0):
+    """Chains replayed on the CPU: all of them when there are few, else chain 0, the last
+    chain, both sides of three CTA boundaries (the first, one in the middle and the start of
+    the partial last CTA) and random others."""
+    if C <= n:
+        return np.arange(C)
+    nb = C // width
+    must = {0, C - 1, width - 1, width, nb // 2 * width - 1, nb // 2 * width,
+            nb * width - 1, min(nb * width, C - 1)}
+    rest = np.setdiff1d(np.arange(C), sorted(must))
+    pick = np.random.default_rng(seed).choice(rest, n - len(must), replace=False)
+    return np.sort(np.concatenate([sorted(must), pick]))
+
+
+def test_dispatch_mirror_rules():
+    sm = 148
+    big = 3 * 64 * sm
+    assert len(COMPILED) == 38 and len(REACHABLE) == 36
+    cases = [
+        ((3, 10, 9, 3, 0, True), (GB, 1, True, 128, False)),
+        ((3, 10, 9, 3, 1, True), (GB, 1, False, 128, False)),
+        ((4, 10, 8, 2, 0, True), (GB, 1, False, 128, False)),      # thin % d != 0
+        ((5, 10, 10, 5, 0, True), (GM, 2, False, 128, False)),
+        ((8, big - 1, 16, 8, 8, True), (GM, 2, True, 128, False)),
+        ((8, big, 16, 8, 8, True), (GM, 2, True, 256, False)),
+        ((8, 10, 15, 8, 8, True), (GB, 2, False, 128, False)),     # T % d != 0
+        ((16, 10, 32, 16, 4, True), (GB, 4, False, 128, False)),   # step0 % d != 0
+        ((16, 10, 32, 16, 16, False), (GM, 4, True, 128, False)),
+        ((17, 10, 34, 17, 0, True), (GM, 8, False, 128, False)),
+        ((32, 10, 64, 32, 0, True), (GM, 8, True, 128, False)),
+        ((33, big, 66, 33, 0, True), (GM, 16, False, 256, False)),
+        ((64, 10, 128, 64, 0, False), (GM, 16, True, 128, False)),
+        ((64, 10, 128, 64, 0, True), (GM, 16, True, 128, True)),
+        ((64, big, 128, 64, 64, True), (GM, 16, True, 256, True)),
+        ((64, 10, 128, 1, 0, True), (GB, 16, False, 128, False)),  # unfused density
+        ((63, 10, 126, 63, 0, True), (GM, 16, False, 128, False)),
+        ((65, 10, 130, 65, 0, True), (GM, 32, False, 128, False)),
+        ((128, big, 128, 128, 0, True), (GM, 32, True, 256, False)),
+        ((128, big, 129, 128, 0, True), (GB, 32, False, 256, False)),
+    ]
+    for args, want in cases:
+        assert _instantiation(*args, sm_count=sm) == want, args
+    # exhaustively: every compiled kernel but the two kDens && !kPair ones is reached
+    seen = set()
+    for d in range(1, 129):
+        for C in (1, big - 1, big):
+            for T, thin, step0 in ((d, d, 0), (2 * d, d, d), (d + 1, 1, 0), (d, 1, 1), (d, d, 3)):
+                for wp in (False, True):
+                    seen.add(_instantiation(d, C, T, thin, step0, wp, sm_count=sm))
+    assert seen == REACHABLE
+    assert not seen & UNREACHABLE
+
+
+# ---------------------------------------------------------------------------------------------
+# models
+# ---------------------------------------------------------------------------------------------
+def _model(d, seed):
+    rng = np.random.default_rng(seed)
+    A = rng.standard_normal((d, d))
+    cov = A @ A.T / d + np.eye(d)
+    mean = rng.standard_normal(d)
+    return mean, cov, rng
+
+
+# Standardised truncation bands z = (lim - mean_i) / stdv_i of the band model.  With p the
+# smaller of u and 1 - u: central (table rows in shared memory), half-infinite both ways,
+# lower tail p in (3e-7, 2.4e-4) (below the shared rows, p < 2^-11: draw_fix on the global
+# table), deep lower tail p < 8e-24 (below the table, p < 2^-64: normcdfinv) and upper tail.
+BANDS = [(-0.5, 1.0), (-np.inf, 0.3), (-5.0, -3.5), (-0.2, np.inf), (-12.0, -10.0), (3.0, 10.0)]
+
+
+def _band_of(i):
+    """Band index of coordinate i: the two draws of a lane (i, i + 4) and coordinates 8 apart
+    (the next block of the tensor-core kernel) fall in different bands."""
+    return (i + i // 4) % len(BANDS)
+
+
+def _band_model(d, seed):
+    """A d-dimensional normal whose coordinate i is truncated to band _band_of(i).
+    The conditional stdv does not depend on the limits, so it is read off a first CondCov."""
+    from probayes_b200.cond_cov import CondCov
+    mean, cov, rng = _model(d, seed)
+    sd = CondCov(mean, cov, np.tile([-10., 10.], (d, 1))).stdv
+    z = np.array([BANDS[_band_of(i)] for i in range(d)])
+    lims = mean[:, None] + z * sd[:, None]
+    return mean, cov, lims, rng
+
+
+def test_band_model_reaches_every_draw_path():
+    from probayes_b200.cond_cov import CondCov
+    mean, cov, lims, _ = _band_model(24, 5)
+    cdfs = CondCov(mean, cov, lims).cdfs
+    ref = o.CondCovOracle(mean, cov, lims).cdfs
+    assert np.abs(cdfs - ref).max() <= 1e-15
+    lo, hi = cdfs[:, 0], cdfs[:, 1]
+    kind = np.array([_band_of(i) for i in range(24)])
+    assert (lo[kind == 1] == 0.0).all() and (hi[kind == 3] == 1.0).all()
+    assert (lo[kind == 2] > 2.0 ** -64).all() and (hi[kind == 2] < 2.0 ** -11).all()
+    assert (hi[kind == 4] < 2.0 ** -64).all() and (lo[kind == 4] > 0.0).all()
+    assert ((1.0 - lo[kind == 5]) < 2.0 ** -9).all()
+    for i in range(20):
+        assert _band_of(i) != _band_of(i + 4) and _band_of(i) != _band_of(i + 1)
+    for i in range(16):
+        assert _band_of(i) != _band_of(i + 8)
+
+
+def test_band_model_c_oracle_matches_numpy():
+    """The C restatement's native stream under real truncation (every draw regime) at nonzero
+    step0 and chain0, against the numpy restatement fed with oracle/philox.py's replay."""
+    from oracle.c import build, liboracle
+    from probayes_b200.cond_cov import CondCov
+    build.build()
+    d, Cn, T, seed, step0, chain0 = 24, 3000, 3 * 24 + 5, 4321, 12, 1001
+    mean, cov, lims, rng = _band_model(d, 6)
+    cc = CondCov(mean, cov, lims)
+    init = mean + rng.standard_normal((Cn, d))
+    x = liboracle.gibbs_mvn_walk(init, mean, cc.coef_matrix(), cc.stdv, cc.cdfs, T, seed=seed,
+                                 step0=step0, chain0=chain0)
+    t = (np.arange(T, dtype=np.uint64) + np.uint64(step0))[:, None]
+    c = (np.arange(Cn, dtype=np.uint64) + np.uint64(chain0))[None, :]
+    ref = o.gibbs_mvn_walk(init, philox.gibbs_uniforms(seed, t, c), mean, cov, lims, start=step0)
+    want = ref["x"][-1]
+    assert np.isfinite(want).all()
+    assert np.abs(x - want).max() <= GTOL * max(1.0, np.abs(want).max())
+
+
+# ---------------------------------------------------------------------------------------------
+# device runs against the oracle
+# ---------------------------------------------------------------------------------------------
+def _check(out, state, ref, thin, sel, want_prob, cov, mean, lin=None):
+    """Recorded states, log densities, final state and running sums of the chains ``sel``
+    against the oracle's walk ``ref`` of those chains; ``lin`` is the output of the same run
+    with linear densities."""
+    X = tcd_to_tdc(ref["x"])[thin - 1::thin]                     # [R, d, n]
+    R = X.shape[0]
+    assert R >= 2                                                  # sums over several records
+    scale = max(1.0, float(np.abs(X).max()))
+    xd = host(out["x"])[:, :, sel]
+    assert np.abs(xd - X).max() <= GTOL * scale
+    assert np.abs(host(state)[:, sel] - ref["x"][-1].T).max() <= GTOL * scale
+    assert np.abs(host(out["stat_sum"])[:, sel] - X.sum(axis=0)).max() <= (R + 1) * GTOL * scale
+    assert np.abs(host(out["stat_sumsq"])[:, sel] - (X * X).sum(axis=0)).max() <= \
+        2 * (R + 1) * GTOL * scale * scale
+    if want_prob:
+        assert relerr(host(out["prob"])[:, sel], ref["prob"][thin - 1::thin]) <= GTOL
+    if lin is not None:
+        # same uniforms, same trajectory; the density of each recorded state in linear pscale
+        assert np.array_equal(host(lin["x"]), host(out["x"]))
+        U, lpd = o.mvn_whiten(cov)
+        pts = np.transpose(xd, (0, 2, 1))[..., o.mvn_value_order(len(mean))]
+        want = np.exp(o.mvn_logpdf(pts, mean, U, lpd))
+        assert (want > 1e-300).all()
+        assert relerr(host(lin["prob"])[:, sel], want) <= LIN_TOL
+
+
+# (d, T, thin, step0, want_prob): each reaches one instantiation per chain-count size
+INJ_CASES = [
+    # per-coordinate kernel (any step range)
+    (3, 9, 3, 0, True),            # DQ = 1, whole sweeps: kSweepRec
+    (4, 11, 2, 1, True),           # DQ = 1
+    (7, 17, 3, 5, True),           # DQ = 2, odd step0
+    (13, 30, 4, 12, True),         # DQ = 4, step0 = 4 mod 8
+    (27, 61, 6, 9, True),          # DQ = 8
+    (50, 103, 10, 20, True),       # DQ = 16
+    (100, 205, 41, 3, True),       # DQ = 32
+    # tensor-core kernel (whole sweeps)
+    (6, 12, 6, 6, True),           # DQ = 2
+    (8, 16, 8, 0, True),           # DQ = 2, kPair
+    (13, 26, 13, 13, True),        # DQ = 4
+    (16, 32, 16, 0, True),         # DQ = 4, kPair
+    (27, 54, 27, 0, True),         # DQ = 8
+    (32, 64, 32, 32, True),        # DQ = 8, kPair
+    (45, 90, 45, 0, True),         # DQ = 16
+    (64, 128, 64, 0, False),       # DQ = 16, kPair, no density
+    (64, 128, 64, 64, True),       # DQ = 16, kPair, fused density
+    (100, 200, 100, 0, True),      # DQ = 32
+    (128, 256, 128, 128, True),    # DQ = 32, kPair
+]
+SIZES = ["small", "big"]
+
+
+@pytest.mark.gpu
+def test_case_list_reaches_every_instantiation():
+    sm = engine().info.sm_count
+    got = {_instantiation(d, _chains(size, sm), T, thin, step0, wp, sm)
+           for size in SIZES for d, T, thin, step0, wp in INJ_CASES}
+    assert got == REACHABLE, sorted(REACHABLE - got)
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("size", SIZES)
+@pytest.mark.parametrize("d,T,thin,step0,want_prob", INJ_CASES)
+def test_injected_every_instantiation(d, T, thin, step0, want_prob, size):
+    from probayes_b200.cond_cov import CondCov
+    eng = engine()
+    sm = eng.info.sm_count
+    C = _chains(size, sm)
+    mean, cov, rng = _model(d, 1000 * d + T)
+    lims = np.tile([-10., 10.], (d, 1))
+    cc = CondCov(mean, cov, lims)
+    init = mean + rng.standard_normal((C, d))
+    Ru = rng.random((T, C))
+    sel = _sample(C, _cta_chains(C, sm))
+    ref = o.gibbs_mvn_walk(init[sel], Ru[:, sel], mean, cov, lims, log_pscale=True, start=step0)
+    Rd = dev(eng, Ru)
+    state = dev(eng, init.T)
+    out = eng.gibbs_mvn(state, cc, T, thin=thin, step0=step0, log_pscale=True, inj_runif=Rd,
+                        want_prob=want_prob, stats=True)
+    lin = None
+    if want_prob:
+        lin = eng.gibbs_mvn(dev(eng, init.T), cc, T, thin=thin, step0=step0, log_pscale=False,
+                            inj_runif=Rd)
+    eng.sync()
+    _check(out, state, ref, thin, sel, want_prob, cov, mean, lin)
+
+
+# Band model runs: (d, T, thin, step0, want_prob) for the per-coordinate kernel and the
+# tensor-core kernel with and without kPair and with the fused density.
+#
+# Why 1e-12 holds under truncation: the table ndtri is accurate to <= 7e-16 relative (normcdfinv,
+# below 2^-64, to ~1e-14), and the kernels form u = cdf_lo + (cdf_hi - cdf_lo) r with one fused
+# multiply-add where the reference rounds the product first.  u then differs by one ulp in up to
+# a fifth of the draws.  Below the median that moves x by < 1e-14; above it p = 1 - u carries
+# the ulp of u and x moves by about (ulp / p) / x: at most 7e-13 (2e-13 relative) over the draws
+# of these tests.  That move grows without bound as p -> 0 -- about 2 in 10^6 upper-tail draws
+# move x by more than 1e-11 -- so the bound holds for these fixed streams, not for every stream.
+BAND_CASES = {
+    "per-coordinate": (24, 2 * 24 + 5, 5, 12, True),
+    "mma-kpair": (24, 48, 24, 24, True),
+    "mma-nopair": (21, 42, 21, 0, True),
+    "mma-density": (64, 128, 64, 0, True),
+}
+BAND_KERNELS = {"per-coordinate": (GB, False), "mma-kpair": (GM, True),
+                "mma-nopair": (GM, False), "mma-density": (GM, True)}
+
+
+def _band_run(eng, path, size, native, seed=0, step0=None, chain0=0):
+    """Band model through ``path``: returns (out, state, ref, thin, sel, want_prob)."""
+    from probayes_b200.cond_cov import CondCov
+    sm = eng.info.sm_count
+    d, T, thin, s0, want_prob = BAND_CASES[path]
+    step0 = s0 if step0 is None else step0
+    C = _chains(size, sm)
+    inst = _instantiation(d, C, T, thin, step0, want_prob, sm)
+    assert (inst[0], inst[2]) == BAND_KERNELS[path] and inst[3] == _nt(C, sm)
+    assert inst[4] == (path == "mma-density")
+    mean, cov, lims, rng = _band_model(d, 77 + d)
+    cc = CondCov(mean, cov, lims)
+    init = mean + rng.standard_normal((C, d))
+    sel = _sample(C, _cta_chains(C, sm))
+    state = dev(eng, init.T)
+    if native:
+        t = (np.arange(T, dtype=np.uint64) + np.uint64(step0))[:, None]
+        Ru = philox.gibbs_uniforms(seed, t, (sel.astype(np.uint64) + np.uint64(chain0))[None, :])
+        out = eng.gibbs_mvn(state, cc, T, thin=thin, step0=step0, chain0=chain0, seed=seed,
+                            log_pscale=True, want_prob=want_prob, stats=True)
+    else:
+        Ru = rng.random((T, C))
+        out = eng.gibbs_mvn(state, cc, T, thin=thin, step0=step0, log_pscale=True,
+                            inj_runif=dev(eng, Ru), want_prob=want_prob, stats=True)
+        Ru = Ru[:, sel]
+    eng.sync()
+    ref = o.gibbs_mvn_walk(init[sel], Ru, mean, cov, lims, log_pscale=True, start=step0)
+    assert np.isfinite(ref["x"]).all()
+    return out, state, ref, thin, sel, want_prob, cov, mean
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("size", SIZES)
+@pytest.mark.parametrize("path", list(BAND_CASES))
+def test_band_injected(path, size):
+    eng = engine()
+    out, state, ref, thin, sel, wp, cov, mean = _band_run(eng, path, size, native=False)
+    _check(out, state, ref, thin, sel, wp, cov, mean)
+
+
+# native stream: whole-sweep kernels at step0 a nonzero multiple of d, the per-coordinate
+# kernel at an odd step0 and at step0 = 4 (mod 8); chain ids offset
+NATIVE_CASES = [("per-coordinate", 29), ("per-coordinate", 36), ("mma-kpair", 72),
+                ("mma-nopair", 42), ("mma-density", 128)]
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("size", SIZES)
+@pytest.mark.parametrize("path,step0", NATIVE_CASES)
+def test_band_native_replay(path, step0, size):
+    eng = engine()
+    out, state, ref, thin, sel, wp, cov, mean = _band_run(eng, path, size, native=True,
+                                                          seed=0x5EED0 + step0, step0=step0,
+                                                          chain0=1000003)
+    _check(out, state, ref, thin, sel, wp, cov, mean)
+
+
+def _native(eng, cc, init, T, step0, chain0, seed, thin=1, record=True):
+    state = dev(eng, init.T)
+    out = eng.gibbs_mvn(state, cc, T, thin=thin, step0=step0, chain0=chain0, seed=seed,
+                        want_prob=False, record=record)
+    return state, out
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("size", SIZES)
+@pytest.mark.parametrize("d,T,thin", [(24, 53, 5), (24, 48, 24), (21, 42, 21)])
+def test_native_sharding_is_bit_exact(d, T, thin, size):
+    """Two calls over the chains [0, C1) and [C1, C) with chain0 offset equal one call bit
+    for bit (at "big" both halves keep the 256-thread kernel)."""
+    from probayes_b200.cond_cov import CondCov
+    eng = engine()
+    sm = eng.info.sm_count
+    C1 = _chains(size, sm)
+    C = 2 * C1 + 1
+    mean, cov, lims, rng = _band_model(d, 11)
+    cc = CondCov(mean, cov, lims)
+    assert _instantiation(d, C, T, thin, 0, False, sm) == \
+        _instantiation(d, C1, T, thin, 0, False, sm) == _instantiation(d, C - C1, T, thin, 0, False, sm)
+    init = mean + rng.standard_normal((C, d))
+    chain0, seed = 555, 2024
+    s_all, o_all = _native(eng, cc, init, T, 0, chain0, seed, thin)
+    s_a, o_a = _native(eng, cc, init[:C1], T, 0, chain0, seed, thin)
+    s_b, o_b = _native(eng, cc, init[C1:], T, 0, chain0 + C1, seed, thin)
+    eng.sync()
+    assert np.array_equal(host(s_all), np.concatenate([host(s_a), host(s_b)], axis=1))
+    assert np.array_equal(host(o_all["x"]), np.concatenate([host(o_a["x"]), host(o_b["x"])], axis=2))
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("size", SIZES)
+@pytest.mark.parametrize("d", [24, 21])
+def test_native_resume(d, size):
+    """Resuming at a sweep boundary (same tensor-core kernel) equals one call bit for bit;
+    resuming mid-sweep (two per-coordinate calls) equals it within the oracle tolerance."""
+    from probayes_b200.cond_cov import CondCov
+    eng = engine()
+    C = _chains(size, eng.info.sm_count)
+    mean, cov, lims, rng = _band_model(d, 12)
+    cc = CondCov(mean, cov, lims)
+    init = mean + rng.standard_normal((C, d))
+    chain0, seed = 99991, 31337
+    s_one, o_one = _native(eng, cc, init, 3 * d, 0, chain0, seed, thin=d)
+    s_sw = dev(eng, init.T)
+    o_a = eng.gibbs_mvn(s_sw, cc, d, thin=d, chain0=chain0, seed=seed, want_prob=False)
+    o_b = eng.gibbs_mvn(s_sw, cc, 2 * d, thin=d, step0=d, chain0=chain0, seed=seed,
+                        want_prob=False)
+    s_mid = dev(eng, init.T)
+    h = d + 5
+    eng.gibbs_mvn(s_mid, cc, h, chain0=chain0, seed=seed, record=False)
+    eng.gibbs_mvn(s_mid, cc, 3 * d - h, step0=h, chain0=chain0, seed=seed, record=False)
+    eng.sync()
+    one = host(s_one)
+    assert np.array_equal(host(s_sw), one)
+    assert np.array_equal(np.concatenate([host(o_a["x"]), host(o_b["x"])]), host(o_one["x"]))
+    assert np.abs(host(s_mid) - one).max() <= GTOL * max(1.0, np.abs(one).max())
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("d,idx", [(4, 2), (6, 5), (13, 4)])
+def test_condcov_interp_native(d, idx):
+    """CondCov.interp (one coordinate, native stream at step0 = idx, seed drawn from
+    np.random) under real truncation equals the oracle's draw."""
+    from probayes_b200.cond_cov import CondCov
+    engine()
+    mean, cov, lims, rng = _band_model(d, 13 + d)
+    cc = CondCov(mean, cov, lims)
+    C = 37
+    vals = mean + rng.standard_normal((C, d))
+    args = [vals[:, j] if j != idx else {0} for j in range(d)]
+    np.random.seed(4242)
+    seed = int(np.random.randint(0, 2 ** 31 - 1))
+    np.random.seed(4242)
+    got = cc.interp(*args)
+    init = vals.copy()
+    init[:, idx] = mean[idx]
+    R = philox.gibbs_uniforms(seed, np.uint64(idx), np.arange(C, dtype=np.uint64))[None, :]
+    ref = o.gibbs_mvn_walk(init, R, mean, cov, lims, start=idx)
+    want = ref["x"][0][:, idx]
+    assert np.abs(got - want).max() <= GTOL * max(1.0, np.abs(want).max())
+    # scalar arguments: one chain, chain id 0
+    np.random.seed(4242)
+    got1 = cc.interp(*[float(a[0]) if not isinstance(a, set) else a for a in args])
+    assert isinstance(got1, float) and abs(got1 - want[0]) <= GTOL * max(1.0, abs(want[0]))
