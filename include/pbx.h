@@ -241,36 +241,30 @@ PBX_API int pbx_grid_norm_logjoint(pbx_ctx* ctx, const double* x_obs, int64_t n_
                            const double* sigma, int32_t n_sigma,
                            const double* logprior_mu, const double* logprior_sigma,
                            double* out);
-/* out[0] = max over n entries (device scalar) */
 /* opt-in: the same values (<= 1e-15) from centred sufficient statistics of the
  * observations: one reduction over x_obs, then O(1) per cell instead of O(N) */
 PBX_API int pbx_grid_norm_logjoint_ss(pbx_ctx* ctx, const double* x_obs, int64_t n_obs,
                                       const double* mu, int32_t n_mu, const double* sigma,
                                       int32_t n_sigma, const double* logprior_mu,
                                       const double* logprior_sigma, double* out);
-PBX_API int pbx_grid_max(pbx_ctx* ctx, const double* logjoint, int64_t n, double* out);
-/* out[0] = sum exp_logp(logjoint - gmax[0]) (device scalars) */
-PBX_API int pbx_grid_sumexp(pbx_ctx* ctx, const double* logjoint, int64_t n,
-                    const double* gmax, double* out);
-/* post[m][s] = log_prob( exp_logp(lj - gmax) / max(tiny, gsum) )   (pd.py:285-295)
- * marg_mu_lin[m]    = sum_s exp_logp(post[m][s])                    (pd.py:162-163)
- * marg_sigma_lin[s] = sum_m exp_logp(post[m][s])  (partial over this slab's rows)
- * post may be NULL (marginals only) or alias logjoint (in place). */
-PBX_API int pbx_grid_posterior(pbx_ctx* ctx, const double* logjoint, int32_t n_mu, int32_t n_sigma,
-                       const double* gmax, const double* gsum,
-                       double* post, double* marg_mu_lin, double* marg_sigma_lin);
-/* The same algebra in TWO passes over the grid (PD.conditionalise + both PD.marginal calls,
- * pd.py:214-295,136-165), for log-pscale (linear = 0) or linear-pscale (linear = 1) input:
- * out2[0] = max (0 for linear input), out2[1] = sum exp_logp(v - max) (plain sum for linear
- * input), from ONE read of v with online rescaling (device scalars) */
+/* The PD normalise / marginal algebra (PD.conditionalise + both PD.marginal calls,
+ * pd.py:214-295,136-165) in TWO passes over the grid, for log-pscale (linear = 0) or
+ * linear-pscale (linear = 1) input.  First pass: out2[0] = max (0 for linear input),
+ * out2[1] = sum exp_logp(v - max) (plain sum for linear input), from ONE read of v with
+ * online rescaling (device scalars) */
 PBX_API int pbx_grid_max_sumexp(pbx_ctx* ctx, const double* v, int64_t n, int32_t linear,
                                 double* out2);
 /* slab-sharded grids: sum_inout[0] *= exp(local_max[0] - global_max[0]) (device scalars), so
  * that per-rank sums taken against the local maxima can be all-reduced */
 PBX_API int pbx_grid_rescale_sumexp(pbx_ctx* ctx, const double* local_max,
                                     const double* global_max, double* sum_inout);
-/* pbx_grid_posterior with linear-pscale support (post = p / max(tiny, sum), marginals plain
- * sums) and the marginals' clamped logs fused: marg_log_flags bit 0 -> marg_mu = log_prob(sum),
+/* Second pass over the grid prob [n_mu, n_sigma] (device):
+ *   post[m][s] = log_prob( exp_logp(prob - gmax) / max(tiny, gsum) )   (pd.py:285-295)
+ *   marg_mu[m]    = sum_s exp_logp(post[m][s])                          (pd.py:162-163)
+ *   marg_sigma[s] = sum_m exp_logp(post[m][s])   (partial over this slab's rows)
+ * linear = 1: post = prob / max(tiny, gsum) and the marginals are plain sums (gmax unused).
+ * post may be NULL (marginals only) or alias prob (in place).  The marginals' clamped logs
+ * are fused: marg_log_flags bit 0 -> marg_mu = log_prob(sum),
  * bit 1 -> marg_sigma likewise (leave a bit clear where the sum must be all-reduced first);
  * bit 2 -> PD.marginalise semantics (pd.py:162-164): the terms exp_logp(p) are summed as they
  * are, subnormals included, instead of conditionalise's clamp of q < tiny to zero */

@@ -124,11 +124,6 @@ SIGNATURES = {
     "pbx_grid_norm_logjoint_ss": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p,
                                             C.c_int32, C.c_void_p, C.c_int32, C.c_void_p,
                                             C.c_void_p, C.c_void_p]),
-    "pbx_grid_max": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
-    "pbx_grid_sumexp": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]),
-    "pbx_grid_posterior": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32,
-                                     C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
-                                     C.c_void_p]),
     "pbx_grid_max_sumexp": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p]),
     "pbx_grid_rescale_sumexp": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "pbx_grid_posterior2": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32,

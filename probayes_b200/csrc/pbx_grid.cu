@@ -12,7 +12,7 @@
 //     [N, M, S] temporary.  FP64-pipe bound: 2 instructions per (cell, observation).
 // K4  PD.conditionalise (pd.py:285-295): p - max; exp; / max(tiny, sum); clamped log
 //     PD.marginalise   (pd.py:162-164): exp (no shift); sum over an axis; clamped log
-//     as deterministic two-stage reductions; HBM bound.
+//     in two deterministic passes over the grid (below); HBM bound.
 #include <math.h>
 #include "pbx_common.cuh"
 
@@ -110,139 +110,6 @@ __global__ void __launch_bounds__(GR_THREADS)
 }
 
 // ---------------------------------------------------------------------------
-// deterministic two-stage reductions over n entries
-// ---------------------------------------------------------------------------
-#define RD_THREADS 256
-enum { RD_MAX = 0, RD_SUMEXP = 1 };
-
-template <int OP>
-__device__ __forceinline__ double rd_combine(double a, double b) {
-  return OP == RD_MAX ? fmax(a, b) : a + b;
-}
-
-template <int OP>
-__global__ void __launch_bounds__(RD_THREADS)
-    grid_reduce_stage1(const double* __restrict__ v, int64_t n, const double* __restrict__ gmax,
-                       double* __restrict__ partial) {
-  const double shift = OP == RD_SUMEXP ? gmax[0] : 0.0;
-  double acc = OP == RD_MAX ? -INFINITY : 0.0, acc2 = acc;
-  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
-  const int64_t tid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if ((((uintptr_t)v) & 15) == 0) {                     // 128-bit loads, 4 in flight per thread
-    const double2* v2 = reinterpret_cast<const double2*>(v);
-    const int64_t n2 = n / 2;
-#pragma unroll 4
-    for (int64_t i = tid; i < n2; i += stride) {
-      const double2 e = __ldcs(v2 + i);
-      acc = rd_combine<OP>(acc, OP == RD_MAX ? e.x : pbx_exp_logp(e.x - shift));
-      acc2 = rd_combine<OP>(acc2, OP == RD_MAX ? e.y : pbx_exp_logp(e.y - shift));
-    }
-    if ((n & 1) && tid == 0)
-      acc = rd_combine<OP>(acc, OP == RD_MAX ? v[n - 1] : pbx_exp_logp(v[n - 1] - shift));
-  } else {
-    for (int64_t i = tid; i < n; i += stride) {
-      const double e = v[i];
-      acc = rd_combine<OP>(acc, OP == RD_MAX ? e : pbx_exp_logp(e - shift));
-    }
-  }
-  acc = rd_combine<OP>(acc, acc2);
-  __shared__ double sh[RD_THREADS];
-  sh[threadIdx.x] = acc;
-  __syncthreads();
-  for (int o = RD_THREADS / 2; o > 0; o >>= 1) {
-    if (threadIdx.x < o) sh[threadIdx.x] = rd_combine<OP>(sh[threadIdx.x], sh[threadIdx.x + o]);
-    __syncthreads();
-  }
-  if (threadIdx.x == 0) partial[blockIdx.x] = sh[0];
-}
-
-template <int OP>
-__global__ void __launch_bounds__(RD_THREADS)
-    grid_reduce_stage2(const double* __restrict__ partial, int np, double* __restrict__ out) {
-  double acc = OP == RD_MAX ? -INFINITY : 0.0;
-  for (int i = threadIdx.x; i < np; i += RD_THREADS) acc = rd_combine<OP>(acc, partial[i]);
-  __shared__ double sh[RD_THREADS];
-  sh[threadIdx.x] = acc;
-  __syncthreads();
-  for (int o = RD_THREADS / 2; o > 0; o >>= 1) {
-    if (threadIdx.x < o) sh[threadIdx.x] = rd_combine<OP>(sh[threadIdx.x], sh[threadIdx.x + o]);
-    __syncthreads();
-  }
-  if (threadIdx.x == 0) out[0] = sh[0];
-}
-
-// ---------------------------------------------------------------------------
-// posterior + marginals: CTA = PR_ROWS rows x 256 columns, thread = one column
-// ---------------------------------------------------------------------------
-#define PR_ROWS 32
-#define PR_COLS 256
-
-__global__ void __launch_bounds__(PR_COLS)
-    grid_posterior_kernel(const double* lj, int M, int S,
-                          const double* __restrict__ gmax, const double* __restrict__ gsum,
-                          double* post, double* __restrict__ row_partial,
-                          double* __restrict__ col_partial, int n_colblocks) {
-  __shared__ double s_row[PR_ROWS][PR_COLS / 32];
-  const int s = blockIdx.x * PR_COLS + threadIdx.x;
-  const int m0 = blockIdx.y * PR_ROWS;
-  const double mx = gmax[0];
-  const double den = fmax(PBX_TINY, gsum[0]);
-  const double lden = log(den);
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  double col = 0.0;
-  for (int r = 0; r < PR_ROWS; ++r) {
-    const int m = m0 + r;
-    double q = 0.0;
-    if (m < M && s < S) {
-      // reference: q = exp_logp(lj - max) / max(tiny, sum); post = log_prob(q);
-      // marginal term = exp_logp(post).  log(q) is evaluated as (lj - max) - log(den)
-      // and exp(log q) as q itself: same values to ~1e-16 relative, a third of the
-      // transcendental work; the clamp decision (q < tiny -> -1.797e308) is the
-      // reference's, taken on q.
-      const double sh = lj[(int64_t)m * S + s] - mx;
-      const double e = pbx_exp_logp(sh);
-      q = e / den;
-      const bool keep = q >= PBX_TINY;
-      if (post) post[(int64_t)m * S + s] = keep ? sh - lden : -PBX_HUGE;
-      q = keep ? q : 0.0;                                 // exp_logp(-1.797e308) = 0
-    }
-    col += q;
-    double w = q;
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) w += __shfl_xor_sync(0xffffffffu, w, o);
-    if (lane == 0) s_row[r][warp] = w;
-  }
-  if (s < S) col_partial[(int64_t)blockIdx.y * S + s] = col;
-  __syncthreads();
-  if (threadIdx.x < PR_ROWS) {
-    const int m = m0 + threadIdx.x;
-    if (m < M) {
-      double w = 0.0;
-#pragma unroll
-      for (int k = 0; k < PR_COLS / 32; ++k) w += s_row[threadIdx.x][k];
-      row_partial[(int64_t)m * n_colblocks + blockIdx.x] = w;
-    }
-  }
-}
-
-__global__ void __launch_bounds__(256)
-    grid_marginal_finish(const double* __restrict__ row_partial, int M, int n_colblocks,
-                         const double* __restrict__ col_partial, int n_rowblocks, int S,
-                         double* __restrict__ marg_mu, double* __restrict__ marg_sigma) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < M && marg_mu) {
-    double w = 0.0;
-    for (int k = 0; k < n_colblocks; ++k) w += row_partial[(int64_t)i * n_colblocks + k];
-    marg_mu[i] = w;
-  }
-  if (i < S && marg_sigma) {
-    double w = 0.0;
-    for (int k = 0; k < n_rowblocks; ++k) w += col_partial[(int64_t)k * S + i];
-    marg_sigma[i] = w;
-  }
-}
-
-// ---------------------------------------------------------------------------
 // C ABI
 // ---------------------------------------------------------------------------
 extern "C" int pbx_grid_norm_logjoint(pbx_ctx* ctx, const double* x_obs, int64_t n_obs,
@@ -316,64 +183,8 @@ extern "C" int pbx_grid_norm_logjoint_ss(pbx_ctx* ctx, const double* x_obs, int6
   return PBX_OK;
 }
 
-template <int OP>
-static int grid_reduce(pbx_ctx* ctx, const double* v, int64_t n, const double* gmax, double* out) {
-  PBX_CUDA(cudaSetDevice(ctx->device));
-  int64_t want = (n + RD_THREADS * 16 - 1) / (RD_THREADS * 16);
-  int np = (int)(want < 1 ? 1 : (want > ctx->sm_count * 8 ? ctx->sm_count * 8 : want));
-  int rc = pbx_ws_reserve(ctx, (size_t)np * 8);
-  if (rc) return rc;
-  double* partial = (double*)ctx->ws;
-  PBX_CUDA(cudaEventRecord(ctx->ev0, ctx->stream));
-  grid_reduce_stage1<OP><<<np, RD_THREADS, 0, ctx->stream>>>(v, n, gmax, partial);
-  PBX_LAUNCH_CHECK(ctx);
-  grid_reduce_stage2<OP><<<1, RD_THREADS, 0, ctx->stream>>>(partial, np, out);
-  PBX_LAUNCH_CHECK(ctx);
-  PBX_CUDA(cudaEventRecord(ctx->ev1, ctx->stream));
-  return PBX_OK;
-}
-
-extern "C" int pbx_grid_max(pbx_ctx* ctx, const double* logjoint, int64_t n, double* out) {
-  PBX_REQUIRE(ctx && logjoint && out && n >= 1, "pbx_grid_max: bad argument");
-  return grid_reduce<RD_MAX>(ctx, logjoint, n, nullptr, out);
-}
-
-extern "C" int pbx_grid_sumexp(pbx_ctx* ctx, const double* logjoint, int64_t n,
-                               const double* gmax, double* out) {
-  PBX_REQUIRE(ctx && logjoint && gmax && out && n >= 1, "pbx_grid_sumexp: bad argument");
-  return grid_reduce<RD_SUMEXP>(ctx, logjoint, n, gmax, out);
-}
-
-extern "C" int pbx_grid_posterior(pbx_ctx* ctx, const double* logjoint, int32_t n_mu,
-                                  int32_t n_sigma, const double* gmax, const double* gsum,
-                                  double* post, double* marg_mu_lin, double* marg_sigma_lin) {
-  PBX_REQUIRE(ctx && logjoint && gmax && gsum, "pbx_grid_posterior: null argument");
-  PBX_REQUIRE(n_mu >= 1 && n_sigma >= 1, "pbx_grid_posterior: sizes must be positive");
-  PBX_CUDA(cudaSetDevice(ctx->device));
-  const int ncb = (n_sigma + PR_COLS - 1) / PR_COLS, nrb = (n_mu + PR_ROWS - 1) / PR_ROWS;
-  PBX_REQUIRE(nrb <= 65535, "pbx_grid_posterior: too many rows per call (slab it)");
-  const size_t rp = ((size_t)n_mu * ncb * 8 + 255) / 256 * 256;
-  const size_t cp = (size_t)nrb * n_sigma * 8;
-  int rc = pbx_ws_reserve(ctx, rp + cp);
-  if (rc) return rc;
-  double* row_partial = (double*)ctx->ws;
-  double* col_partial = (double*)((char*)ctx->ws + rp);
-  PBX_CUDA(cudaEventRecord(ctx->ev0, ctx->stream));
-  grid_posterior_kernel<<<dim3(ncb, nrb), PR_COLS, 0, ctx->stream>>>(
-      logjoint, n_mu, n_sigma, gmax, gsum, post, row_partial, col_partial, ncb);
-  PBX_LAUNCH_CHECK(ctx);
-  if (marg_mu_lin || marg_sigma_lin) {
-    const int n = n_mu > n_sigma ? n_mu : n_sigma;
-    grid_marginal_finish<<<(n + 255) / 256, 256, 0, ctx->stream>>>(
-        row_partial, n_mu, ncb, col_partial, nrb, n_sigma, marg_mu_lin, marg_sigma_lin);
-    PBX_LAUNCH_CHECK(ctx);
-  }
-  PBX_CUDA(cudaEventRecord(ctx->ev1, ctx->stream));
-  return PBX_OK;
-}
-
 // ---------------------------------------------------------------------------
-// K4 in two passes over the grid (was max, sum-exp, posterior: three reads + a write).
+// K4 in two passes over the grid.
 //
 // Pass A  pbx_grid_max_sumexp: ONE read.  Every thread keeps an online (max, sum-exp)
 //         pair: per chunk of 8 entries held in registers, the running maximum is raised

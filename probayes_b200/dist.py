@@ -44,12 +44,21 @@ def default_chain0(chains):
     return world()[0] * int(chains)
 
 
+def _sharded(group=None):
+    """``torch.distributed`` when ``group`` (None: the default group) has more than one
+    rank, else None."""
+    import torch.distributed as dist
+    if dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1:
+        return dist
+    return None
+
+
 def allreduce_chain_stats(stats, group=None):
     """stats [D, 4] = (sum_c mean, sum_c mean^2, sum_c var, C) per dimension, as
     produced by ``Engine.chain_stats`` on this rank's chains -> summed over ranks
     (in place)."""
-    import torch.distributed as dist
-    if dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1:
+    dist = _sharded(group)
+    if dist is not None:
         dist.all_reduce(stats, op=dist.ReduceOp.SUM, group=group)
     return stats
 
@@ -73,19 +82,20 @@ def pooled_moments(stats):
     return st[:, 0] / st[:, 3], st[:, 2] / st[:, 3]
 
 
-def grid_normaliser(local_max, local_sumexp_fn, group=None):
-    """Two-phase normaliser of a slab-sharded log-joint.
+def allreduce_max_sumexp(gmax, gsum, rescale, linear=False, group=None):
+    """Normaliser of a slab-sharded log-joint: (gmax, gsum) = this slab's (max, sum exp(v -
+    max)) as 1-element tensors, updated in place to the same pair over all ranks.
 
-    local_max: 1-element tensor (this slab's max).  local_sumexp_fn(gmax) -> 1-element
-    tensor sum exp(lj - gmax) over this slab.  Returns (gmax, gsum) identical on
-    every rank: all-reduce(max) then all-reduce(sum)."""
-    import torch.distributed as dist
-    on = dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1
-    gmax = local_max.clone()
-    if on:
-        dist.all_reduce(gmax, op=dist.ReduceOp.MAX, group=group)
-    gsum = local_sumexp_fn(gmax)
-    if on:
+    All-reduce(max) of gmax; rescale(local_max, gmax, gsum) turns the local sum into the
+    sum against the global maximum (``Engine.grid_rescale_sumexp_`` on the device: 0 stays
+    0, else gsum * exp(local_max - gmax)); all-reduce(sum) of gsum.  ``linear`` input (plain
+    sums): only gsum is reduced.  Identical on every rank; a no-op on one rank."""
+    dist = _sharded(group)
+    if dist is not None:
+        if not linear:
+            lmax = gmax.clone()
+            dist.all_reduce(gmax, op=dist.ReduceOp.MAX, group=group)
+            rescale(lmax, gmax, gsum)
         dist.all_reduce(gsum, op=dist.ReduceOp.SUM, group=group)
     return gmax, gsum
 
@@ -94,8 +104,8 @@ def gather_slabs(local, counts, group=None):
     """All-gather of per-rank 1-D slabs of (possibly) different lengths ``counts``
     into one vector (the mu marginal of a slab-sharded grid)."""
     import torch
-    import torch.distributed as dist
-    if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size(group) == 1:
+    dist = _sharded(group)
+    if dist is None:
         return local
     m = max(counts)
     pad = torch.zeros(m, dtype=local.dtype, device=local.device)
@@ -110,7 +120,6 @@ def dgei_sharded(engine, x_obs, mu, sigma, logprior_mu, logprior_sigma, group=No
     log-joint of its mu rows, the ranks agree on the normaliser, and each returns
     dict(post=[M_local, S] slab, marg_mu=[M] (gathered), marg_sigma=[S], rows=(start,
     count)).  All inputs are full-size host arrays."""
-    import torch.distributed as dist
     rank, ws = world()
     M = len(mu)
     start, count = shard_range(M, rank, ws)
@@ -118,11 +127,11 @@ def dgei_sharded(engine, x_obs, mu, sigma, logprior_mu, logprior_sigma, group=No
     lj = engine.grid_norm_logjoint(engine.to_device(x_obs), engine.to_device(mu[sl]),
                                    engine.to_device(sigma), engine.to_device(logprior_mu[sl]),
                                    engine.to_device(logprior_sigma))
-    import torch.distributed as tdist
-    on = tdist.is_available() and tdist.is_initialized() and tdist.get_world_size(group) > 1
-    if on and group is None:
-        group = tdist.group.WORLD
-    r = engine.grid_conditionalise(lj, want_post=True, inplace=True, group=group if on else None)
+    dist = _sharded(group)
+    if dist is not None and group is None:
+        group = dist.group.WORLD
+    r = engine.grid_conditionalise(lj, want_post=True, inplace=True,
+                                   group=group if dist is not None else None)
     counts = [shard_range(M, q, ws)[1] for q in range(ws)]
     mm = gather_slabs(r["marg_mu"], counts, group)
     return dict(post=r["post"], marg_mu=mm, marg_sigma=r["marg_sigma"], rows=(start, count),
@@ -133,8 +142,8 @@ def allreduce_expectation(sums, group=None):
     """sums [1 + K] = (sum p, sum p*v_1, ...) over this rank's cells (Engine.
     expectation_sums) -> expectations [K] over all ranks: all-reduce(sum), then the
     reference's safe division (probayes/pd.py:402, pscales.py:219-236)."""
-    import torch.distributed as dist
-    if dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1:
+    dist = _sharded(group)
+    if dist is not None:
         dist.all_reduce(sums, op=dist.ReduceOp.SUM, group=group)
     st = np.asarray(sums.detach().cpu().numpy() if hasattr(sums, "detach") else sums,
                     dtype=np.float64)
@@ -154,9 +163,13 @@ def omc_sharded(engine, y_obs, lims, open_end, log_ufun, n_samples, seed=0, x_ob
     y = engine.to_device(np.ravel(np.asarray(y_obs, dtype=np.float64)))
     x = None if x_obs is None else engine.to_device(np.ravel(np.asarray(x_obs, np.float64)))
     logp = engine.normreg_logjoint(theta, y, x, lims, open_end, log_ufun)
-    gmax, gsum = grid_normaliser(engine.grid_max(logp),
-                                 lambda g: engine.grid_sumexp(logp, g), group)
-    post, _, _ = engine.grid_posterior(logp.reshape(1, -1), gmax, gsum, inplace=True)
+    ms = engine.grid_max_sumexp(logp)
+    gmax, gsum = allreduce_max_sumexp(ms[0:1], ms[1:2], engine.grid_rescale_sumexp_,
+                                      group=group)
+    # Engine.grid_conditionalise without its marginals: the per-sample "column" sums differ
+    # in length from rank to rank and must not be all-reduced
+    post, _, _ = engine.grid_posterior2(logp.reshape(1, -1), gmax, gsum, inplace=True,
+                                        marg_log=0)
     sums = engine.expectation_sums(post.reshape(-1), True, None, theta)
     return dict(theta=theta, logpost=post.reshape(-1), samples=(start, count),
                 expectation=allreduce_expectation(sums, group))

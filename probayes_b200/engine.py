@@ -452,29 +452,6 @@ class Engine:
                 self._ptr(out[m0:m1])), what)
         return out
 
-    def grid_max(self, lj):
-        out = self.empty(1)
-        _lib.check(self.lib.pbx_grid_max(self.ctx, self._ptr(lj), int(lj.numel()),
-                                         self._ptr(out)), "pbx_grid_max")
-        return out
-
-    def grid_sumexp(self, lj, gmax):
-        out = self.empty(1)
-        _lib.check(self.lib.pbx_grid_sumexp(self.ctx, self._ptr(lj), int(lj.numel()),
-                                            self._ptr(gmax), self._ptr(out)), "pbx_grid_sumexp")
-        return out
-
-    def grid_posterior(self, lj, gmax, gsum, want_post=True, inplace=False):
-        """(post [M, S] or None, marg_mu_lin [M], marg_sigma_lin [S]) -- the
-        marginals are linear sums still to be passed through ``log_prob_``."""
-        M, S = lj.shape
-        post = (lj if inplace else self.empty(M, S)) if want_post else None
-        mm, ms = self.empty(M), self.empty(S)
-        _lib.check(self.lib.pbx_grid_posterior(self.ctx, self._ptr(lj), M, S, self._ptr(gmax),
-                                               self._ptr(gsum), self._ptr(post), self._ptr(mm),
-                                               self._ptr(ms)), "pbx_grid_posterior")
-        return post, mm, ms
-
     def log_prob_(self, v):
         """In-place clamped log (probayes/pscales.py:44-53)."""
         _lib.check(self.lib.pbx_log_prob_inplace(self.ctx, self._ptr(v), int(v.numel())),
@@ -495,6 +472,13 @@ class Engine:
                                                 1 if linear else 0, self._ptr(out)),
                    "pbx_grid_max_sumexp")
         return out
+
+    def grid_rescale_sumexp_(self, lmax, gmax, gsum):
+        """gsum = sum exp(v - lmax) -> sum exp(v - gmax) in place (1-element device tensors;
+        a zero sum stays zero): a slab's sum against the maximum over all slabs."""
+        _lib.check(self.lib.pbx_grid_rescale_sumexp(self.ctx, self._ptr(lmax), self._ptr(gmax),
+                                                    self._ptr(gsum)), "pbx_grid_rescale_sumexp")
+        return gsum
 
     def grid_posterior2(self, prob, gmax, gsum, linear=False, want_post=True, inplace=False,
                         marg_log=3):
@@ -518,19 +502,13 @@ class Engine:
         Returns dict(post, marg_mu, marg_sigma, gmax, gsum) in the input's pscale."""
         ms = self.grid_max_sumexp(lj, linear)
         gmax, gsum = ms[0:1], ms[1:2]
-        dist = None
+        if group is not None:
+            from .dist import allreduce_max_sumexp
+            allreduce_max_sumexp(gmax, gsum, self.grid_rescale_sumexp_, linear, group)
+        log_bits = 0 if linear else (1 if group is not None else 3)
+        post, mm, msig = self.grid_posterior2(lj, gmax, gsum, linear, want_post, inplace, log_bits)
         if group is not None:
             import torch.distributed as dist
-            if not linear:
-                lmax = gmax.clone()
-                dist.all_reduce(gmax, op=dist.ReduceOp.MAX, group=group)
-                _lib.check(self.lib.pbx_grid_rescale_sumexp(self.ctx, self._ptr(lmax),
-                                                            self._ptr(gmax), self._ptr(gsum)),
-                           "pbx_grid_rescale_sumexp")
-            dist.all_reduce(gsum, op=dist.ReduceOp.SUM, group=group)
-        log_bits = 0 if linear else (1 if dist is not None else 3)
-        post, mm, msig = self.grid_posterior2(lj, gmax, gsum, linear, want_post, inplace, log_bits)
-        if dist is not None:
             dist.all_reduce(msig, op=dist.ReduceOp.SUM, group=group)
             if not linear:
                 self.log_prob_(msig)

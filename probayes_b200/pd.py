@@ -273,8 +273,14 @@ class PD(collections.OrderedDict):
                 if linear:
                     tot = eng.grid_max_sumexp(self._prob_dev.reshape(-1), linear=True)[1:2]
                 else:
+                    one = torch.ones(1, dtype=torch.float64, device=self._prob_dev.device)
                     zero = torch.zeros(1, dtype=torch.float64, device=self._prob_dev.device)
-                    tot = eng.log_prob_(eng.grid_sumexp(self._prob_dev.reshape(-1), zero))
+                    # row sums of exp_logp(prob) from the posterior pass (max = 0, sum = 1,
+                    # marginalise semantics), then their plain sum.  A 2-D PD keeps its rows:
+                    # one warp finishes a row, from one partial per 128 columns
+                    p2 = self._prob_dev if self.ndim == 2 else self._prob_dev.reshape(1, -1)
+                    _, rows, _ = eng.grid_posterior2(p2, zero, one, want_post=False, marg_log=4)
+                    tot = eng.log_prob_(eng.grid_max_sumexp(rows, linear=True)[1:2])
                 return self._new(name, vals, dims, float(tot.item()))
             if self.ndim == 2 and len(axes) == 1:
                 one = torch.ones(1, dtype=torch.float64, device=self._prob_dev.device)

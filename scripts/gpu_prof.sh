@@ -8,7 +8,7 @@ prof() {  # name regex which
 prof tiles nr_tiles tiles
 prof stream nr_stream stream
 prof gridlj grid_logjoint grid
-prof gridpost grid_posterior grid
+prof gridpost grid_posterior2 grid
 prof gibbs gibbs_mvn_kernel gibbs
 prof dmma mvn_logpdf_mma gibbs
 ls -la gpurun_out/*.ncu-rep; du -sh gpurun_out

@@ -12,14 +12,8 @@ def t(fn, n=5):
     for _ in range(n):
         fn(); ms.append(eng.last_kernel_ms())
     return float(np.median(ms))
-print("max (old)        %.4f ms" % t(lambda: eng.grid_max(lj)))
-gm = eng.grid_max(lj)
-print("sumexp (old)     %.4f ms" % t(lambda: eng.grid_sumexp(lj, gm)))
-gs = eng.grid_sumexp(lj, gm)
-print("posterior (old)  %.4f ms" % t(lambda: eng.grid_posterior(lj, gm, gs)))
 print("max_sumexp       %.4f ms" % t(lambda: eng.grid_max_sumexp(lj)))
 ms = eng.grid_max_sumexp(lj)
-print("  check", float(ms[0] - gm), float(ms[1] / gs - 1))
 print("posterior2       %.4f ms" % t(lambda: eng.grid_posterior2(lj, ms[0:1], ms[1:2])))
 print("posterior2 inpl  %.4f ms" % t(lambda: eng.grid_posterior2(lj.clone(), ms[0:1], ms[1:2], inplace=True)))
 print("posterior2 nopost %.4f ms" % t(lambda: eng.grid_posterior2(lj, ms[0:1], ms[1:2], want_post=False)))

@@ -1,7 +1,8 @@
 """Multi-rank host logic on CPU with the gloo backend (world_size 2 and 3): chain
 sharding, summary all-reduce -> R-hat, slab-sharded grid normaliser and marginal
 gathering.  The device kernels are not involved (no GPU here); the per-rank slab
-arithmetic is stood in for by the numpy oracle."""
+arithmetic, including the rescaling of a local sum to the global maximum, is stood in for
+by the numpy oracle."""
 import os
 import sys
 import numpy as np
@@ -53,6 +54,18 @@ def test_rhat_allreduce(world, port):
         assert np.allclose(pm, wm, rtol=1e-12)
 
 
+def _rescale(lmax, gmax, gsum):
+    """Engine.grid_rescale_sumexp_ (grid_rescale_sumexp_kernel) on host tensors."""
+    s = float(gsum[0])
+    gsum[0] = 0.0 if s == 0 else s * np.exp(float(lmax[0]) - float(gmax[0]))
+
+
+def _local_max_sumexp(v):
+    """This rank's (max, sum exp(v - max)) pair, as Engine.grid_max_sumexp returns it."""
+    from oracle import np_oracle as o
+    return torch.tensor([v.max()]), torch.tensor([o.exp_logp(v - v.max()).sum()])
+
+
 def _grid_job(rank, world):
     from probayes_b200 import dist as pd_
     from oracle import np_oracle as o
@@ -61,9 +74,12 @@ def _grid_job(rank, world):
     lj = rng.normal(-500, 30, (M, S))
     start, count = pd_.shard_range(M, rank, world)
     slab = lj[start:start + count]
-    gmax, gsum = pd_.grid_normaliser(
-        torch.tensor([slab.max()]),
-        lambda g: torch.tensor([o.exp_logp(slab - float(g)).sum()]))
+    gmax, gsum = pd_.allreduce_max_sumexp(*_local_max_sumexp(slab), _rescale)
+    # linear-pscale slabs: only the plain sum is reduced
+    p = np.exp(lj - lj.max())
+    lin_max, lin_sum = pd_.allreduce_max_sumexp(
+        torch.zeros(1), torch.tensor([p[start:start + count].sum()]), _rescale, linear=True)
+    lin_ok = float(lin_max) == 0.0 and abs(float(lin_sum) - p.sum()) <= 1e-12 * p.sum()
     post = o.log_prob(o.exp_logp(slab - float(gmax)) / max(o.NEARLY_POSITIVE_ZERO, float(gsum)))
     lin = o.exp_logp(post)
     ms = torch.tensor(lin.sum(axis=0))
@@ -74,13 +90,14 @@ def _grid_job(rank, world):
     return (np.abs(post - whole[start:start + count]).max(),
             np.abs(o.log_prob(mm.numpy()) - o.grid_marginal(whole, 1)).max(),
             np.abs(o.log_prob(ms.numpy()) - o.grid_marginal(whole, 0)).max(),
-            float(gmax) == lj.max())
+            float(gmax) == lj.max(), lin_ok)
 
 
 @pytest.mark.parametrize("world,port", [(2, 29615), (3, 29617)])
-def test_slab_sharded_grid_normaliser(world, port):
-    for e_post, e_mm, e_ms, max_ok in _spawn(_grid_job, world, port):
+def test_slab_sharded_allreduce_max_sumexp(world, port):
+    for e_post, e_mm, e_ms, max_ok, lin_ok in _spawn(_grid_job, world, port):
         assert max_ok and e_post <= 1e-9 and e_mm <= 1e-9 and e_ms <= 1e-9
+        assert lin_ok
 
 
 def _omc_job(rank, world):
@@ -95,8 +112,7 @@ def _omc_job(rank, world):
     start, count = pd_.shard_range(T, rank, world)
     th = o.box_sample(lims, logu, philox.uniforms(seed, count, 1, 2, step0=start)[:, 0, :])
     lj = o.normreg_logjoint(th.T, None, data, lims, np.ones((2, 2), int), logu, has_slope=False)
-    gmax, gsum = pd_.grid_normaliser(torch.tensor([lj.max()]),
-                                     lambda g: torch.tensor([o.exp_logp(lj - float(g)).sum()]))
+    gmax, gsum = pd_.allreduce_max_sumexp(*_local_max_sumexp(lj), _rescale)
     lin = o.exp_logp(lj - float(gmax)) / max(o.NEARLY_POSITIVE_ZERO, float(gsum))
     sums = torch.tensor([lin.sum(), (lin * th[0]).sum(), (lin * th[1]).sum()])
     e = pd_.allreduce_expectation(sums)
@@ -109,7 +125,7 @@ def _omc_job(rank, world):
 
 
 @pytest.mark.parametrize("world,port", [(2, 29619), (3, 29621)])
-def test_sample_sharded_omc_expectation(world, port):
+def test_sample_sharded_omc_expectation_allreduce_max_sumexp(world, port):
     for e, want, same_stream in _spawn(_omc_job, world, port):
         assert same_stream                       # results do not depend on the rank count
         assert np.allclose(e, want, rtol=1e-12)

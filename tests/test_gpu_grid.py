@@ -83,7 +83,7 @@ def test_oracle_ragged(N, M, S):
     assert _abs_masked(host(r["marg_sigma"]), o.grid_marginal(post, 0)) <= atol
 
 
-def test_slab_sharded_equals_whole():
+def test_slab_sharded_two_pass_equals_whole():
     """mu-row slabs (the multi-GPU partitioning) reproduce the whole-grid result:
     max of maxes, sum of sums, summed sigma marginal, concatenated mu marginal."""
     import torch
@@ -99,11 +99,12 @@ def test_slab_sharded_equals_whole():
                                                           lpsd))
     slabs = [eng.grid_norm_logjoint(xd, dev(eng, mu[a:b]), sd, dev(eng, lpm[a:b]), lpsd)
              for a, b in [(0, 40), (40, 41), (41, 96)]]
-    gmax = torch.stack([eng.grid_max(s) for s in slabs]).max(dim=0).values
-    gsum = torch.stack([eng.grid_sumexp(s, gmax) for s in slabs]).sum(dim=0)
-    parts = [eng.grid_posterior(s, gmax, gsum) for s in slabs]
+    pairs = [eng.grid_max_sumexp(s) for s in slabs]
+    gmax = torch.stack([p[0:1] for p in pairs]).max(dim=0).values
+    gsum = torch.stack([eng.grid_rescale_sumexp_(p[0:1], gmax, p[1:2]) for p in pairs]).sum(dim=0)
+    parts = [eng.grid_posterior2(s, gmax, gsum, marg_log=1) for s in slabs]
     post = torch.cat([p[0] for p in parts])
-    mm = eng.log_prob_(torch.cat([p[1] for p in parts]))
+    mm = torch.cat([p[1] for p in parts])
     ms = eng.log_prob_(torch.stack([p[2] for p in parts]).sum(dim=0))
     eng.sync()
     assert float(gmax) == float(whole["gmax"])

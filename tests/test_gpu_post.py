@@ -274,6 +274,30 @@ def test_api_omc_large_native_rng():
     assert abs(e['mu'] - data.mean()) < 0.5
 
 
+def test_omc_sharded_single_rank_matches_oracle():
+    """dist.omc_sharded outside a process group: the Philox draws, the log posterior
+    normalised over all samples (an odd count, off every CTA tile) and the posterior means
+    against the oracle on the replayed stream."""
+    from probayes_b200 import dist as pd_
+    eng = engine()
+    data = np.random.default_rng(4).normal(50., 10., 300)
+    T, seed, ex = 100003, 21, np.ones((2, 2), int)
+    r = pd_.omc_sharded(eng, data, LIMS, ex, LOGU, T, seed=seed)
+    eng.sync()
+    assert r["samples"] == (0, T)
+    th = o.box_sample(LIMS, LOGU, philox.uniforms(seed, T, 1, 2)[:, 0, :])
+    got = host(r["theta"])
+    assert np.array_equal(got[0], th[0]) and relerr(got[1], th[1]) <= 4e-16
+    lj = o.normreg_logjoint(th.T, None, data, LIMS, ex, LOGU, has_slope=False)
+    want = o.grid_conditionalise(lj)
+    post = host(r["logpost"])
+    clamp = want == o.NEARLY_NEGATIVE_INF
+    assert np.array_equal(post == o.NEARLY_NEGATIVE_INF, clamp) and not clamp.all()
+    assert np.abs(post[~clamp] - want[~clamp]).max() <= TOL * np.abs(lj).max()
+    lin = o.exp_logp(want)
+    assert relerr(r["expectation"], (lin * th).sum(axis=1) / lin.sum()) <= 1e-10
+
+
 def test_api_dgei_posterior_postprocessing():
     """The steps right after the DGEI posterior (dgei_norm1d_improved.py:38-46) on the
     device-backed grid PD: expectation over both axes, quantiles of the marginals and
@@ -481,6 +505,40 @@ def test_linear_pscale_device_pds_stay_on_the_device():
         odd.conditionalise('x')
     with pytest.raises(NotImplementedError):
         odd.marginalise('mu')
+
+
+@pytest.mark.parametrize("shape", [(1,), (1000,), (5000,), (37, 29), (3, 5000)])
+def test_full_marginalise_log_pscale_matches_oracle(shape):
+    """PD.marginalise over every array axis of a log-pscale device PD (1-D and 2-D, one and
+    several 1024-column blocks): log_prob(sum exp_logp(p)) without a max shift, against the
+    oracle.  Ordinary values; every term underflowing (-> -1.797e308); a subnormal total;
+    subnormal terms with a normal total; one term above log(huge) (clamped to huge); two of
+    them (the sum overflows -> inf)."""
+    eng = engine()
+    import probayes_b200 as pb
+    n = int(np.prod(shape))
+    rng = np.random.default_rng(n)
+    vals = {k: np.arange(m, dtype=float) for k, m in zip("xy", shape)}
+    name = ",".join(vals)
+    cases = {"ordinary": rng.normal(-3., 2., n),
+             "underflow": np.concatenate([[o.NEARLY_NEGATIVE_INF, -np.inf],
+                                          rng.uniform(-3000., -746., n)])[:n],
+             "subnormal_total": rng.uniform(-745., -720., n),
+             "subnormal_terms": rng.uniform(-712., -709.5, n),
+             "huge_term": np.concatenate([[1e4], rng.normal(-3., 2., n)])[:n]}
+    if n > 1:
+        cases["overflow"] = np.concatenate([[709.9, 1e4], rng.normal(-3., 2., n)])[:n]
+    for case, p in cases.items():
+        p = rng.permutation(p)
+        pd = pb.PD(name, dict(vals), prob=dev(eng, p.reshape(shape)), pscale='log')
+        got = float(pd.marginalise(list(vals)).prob)
+        with np.errstate(over='ignore'):
+            want = float(o.log_prob(o.exp_logp(p).sum()))
+        if case in ("underflow", "subnormal_total"):
+            assert want == o.NEARLY_NEGATIVE_INF, case
+        if case == "overflow":
+            assert want == np.inf, case
+        assert got == want or abs(got - want) <= 1e-13, (case, got, want)
 
 
 # ---- full-size properties (no CPU oracle at these sizes) --------------------------------------
