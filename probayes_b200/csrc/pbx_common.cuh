@@ -73,6 +73,17 @@ __device__ __forceinline__ double pbx_exp_logp(double l) {
   return (l <= PBX_LOG_HUGE) ? exp(l) : PBX_HUGE;
 }
 
+// Variable.apply_delta(bound=True), scalar branch (variable.py:700-727): proposal v of a
+// coordinate whose current value is cur, inside [lo, hi]; closed ends clip, beyond an open
+// end the proposal bounces back to the current value
+__device__ __forceinline__ double pbx_bound(double v, double cur, double lo, double hi,
+                                            bool olo, bool ohi) {
+  if (!olo && !ohi) return fmax(lo, fmin(hi, v));
+  if (olo && ohi) return (v > lo && v < hi) ? v : cur;
+  if (olo) return (v < lo) ? cur : fmin(hi, v);
+  return (v > hi) ? cur : fmax(lo, v);
+}
+
 // ---------------------------------------------------------------------------
 // Philox4x32-10 counter RNG.  Stream layout documented in oracle/philox.py:
 //   key = (seed lo, seed hi); counter = (step lo, step hi, chain, slot)

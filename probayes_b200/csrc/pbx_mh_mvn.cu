@@ -325,19 +325,10 @@ __global__ void __launch_bounds__(128) mh_mvn_kernel(const MhMvnArgs a,
 #pragma unroll
     for (int j = 0; j < D; ++j) xp[j] = x[j] + dv[j];
     if (m.bound) {
-      // Variable.apply_delta(bound=True), scalar branch (variable.py:700-727): closed
-      // ends clip; beyond an open end the proposal bounces back to the current value
 #pragma unroll
-      for (int j = 0; j < D; ++j) {
-        const double lo = m.lims[j][0], hi = m.lims[j][1];
-        const bool olo = m.open_end[j][0] != 0, ohi = m.open_end[j][1] != 0;
-        double v = xp[j];
-        if (!olo && !ohi) v = fmax(lo, fmin(hi, v));
-        else if (olo && ohi) v = (v > lo && v < hi) ? v : x[j];
-        else if (olo) v = (v < lo) ? x[j] : fmin(hi, v);
-        else v = (v > hi) ? x[j] : fmax(lo, v);
-        xp[j] = v;
-      }
+      for (int j = 0; j < D; ++j)
+        xp[j] = pbx_bound(xp[j], x[j], m.lims[j][0], m.lims[j][1], m.open_end[j][0] != 0,
+                          m.open_end[j][1] != 0);
     }
     // ---- evaluate target ----------------------------------------------------
     const double maha = mvn_maha<D>(xp, m);

@@ -24,7 +24,6 @@
 //          128-bit coalesced loads, updates all chains' sums, warp-shuffle + block
 //          reduce.  This is the HBM-roofline regime (16 B per observation per step).
 #include <math.h>
-#include <stdlib.h>
 #include <string.h>
 #include <algorithm>
 #include "pbx_common.cuh"
@@ -136,28 +135,92 @@ __device__ __forceinline__ double nr_threshold(const NrArgs& a, int64_t gstep, i
   return pbx_t44(w.w, w.y);
 }
 
-// kExtras gates the rarely used per-step extras (bounded deltas, proposal outputs) at
-// compile time, so that adding to them never perturbs the register allocation of the
-// hot likelihood loops of the common configuration (a 9 % effect when it happened)
+// ----------------------------------------------------------------------------
+// one MH step, shared by every walk path: only the likelihood sum differs between them
+// ----------------------------------------------------------------------------
+// coordinate j of the proposal: ufun^-1(ufun(th) + dl) (variable.py:693-697), then the bound
+// rule.  kBound = false compiles the bound rule out: the one-launch-per-step kernels pass their
+// kExtras there, so that the rarely used per-step extras (bounded deltas, proposal outputs)
+// never perturb the register allocation of the hot likelihood loops of the common
+// configuration (a 9 % effect when it happened)
+template <bool kBound>
+__device__ __forceinline__ double nr_move(const NrModel& m, int j, double th, double dl) {
+  const double v = m.log_ufun[j] ? exp(log(th) + dl) : th + dl;
+  if (!kBound || !m.bound) return v;
+  return pbx_bound(v, th, m.lims[j][0], m.lims[j][1], m.open_end[j][0] != 0,
+                   m.open_end[j][1] != 0);
+}
+
+// accept decision for the proposal's log-joint lpp against the current lp and threshold t
+// (sp_utils.py:19-64 / pscales.py:219-236); logt() gives log(t) and is called under the log
+// rule only.  Global step 0 always accepts (sp.py:253, sp_utils.py:24-25), with score NaN;
+// the log rule computes its score only when want_score
+template <class LogT>
+__device__ __forceinline__ bool nr_decide(const NrModel& m, double lpp, double lp, double t,
+                                          LogT logt, int64_t gstep, bool want_score, double& s) {
+  bool acc;
+  s = nan("");
+  if (gstep == 0) {
+    acc = true;
+  } else if (m.accept_mode == PBX_ACCEPT_REFERENCE) {
+    // hastings_scores multiplies the linear proposal density into the LOG target
+    // (sp_utils.py:62-64); coef = 1 for metropolis
+    const double num = pbx_exp_logp(lpp * m.coef), den = pbx_exp_logp(lp * m.coef);
+    s = fmin(1.0, num / fmax(PBX_TINY, den));
+    acc = (s >= t);
+  } else {
+    const double d = m.coef * (lpp - lp);
+    acc = (d >= logt());
+    if (want_score) s = fmin(1.0, exp(fmin(d, 0.0)));
+  }
+  return acc;
+}
+
+// per-step outputs of step k (decision, score, proposal thp and its lpp) and, every thin-th
+// step, the record of the state th / lp after it; kExtras = false leaves out the proposal
+template <bool kExtras, int kP = 0>
+__device__ __forceinline__ void nr_record(const NrArgs& a, const NrModel& m, int k, int c,
+                                          bool acc, double s, const double* thp, double lpp,
+                                          const double* th, double lp) {
+  const int64_t C = a.C;
+  const int P = kP ? kP : m.P;
+  if (a.out_accept) a.out_accept[(int64_t)k * C + c] = acc ? 1 : 0;
+  if (a.out_score) a.out_score[(int64_t)k * C + c] = s;
+  if (kExtras && a.out_xprop)
+    for (int j = 0; j < P; ++j) a.out_xprop[((int64_t)k * P + j) * C + c] = thp[j];
+  if (kExtras && a.out_pprop) a.out_pprop[(int64_t)k * C + c] = lpp;
+  if ((k + 1) % a.thin == 0) {
+    const int64_t r = (k + 1) / a.thin - 1;
+    if (a.out_x)
+      for (int j = 0; j < P; ++j) a.out_x[(r * P + j) * C + c] = th[j];
+    if (a.out_prob) a.out_prob[r * C + c] = lp;
+  }
+}
+
+// end of a one-launch walk: the state, its log-joint, the running sums and the accept count
+template <int kP = 0>
+__device__ __forceinline__ void nr_write_back(const NrArgs& a, const NrModel& m, int c,
+                                              const double* th, double lp, const double* ssum,
+                                              const double* ssq, int64_t nacc) {
+  const int64_t C = a.C;
+  const int P = kP ? kP : m.P;
+  for (int j = 0; j < P; ++j) {
+    a.state[(int64_t)j * C + c] = th[j];
+    if (a.stat_sum) a.stat_sum[(int64_t)j * C + c] += ssum[j];
+    if (a.stat_sumsq) a.stat_sumsq[(int64_t)j * C + c] += ssq[j];
+  }
+  a.state_lp[c] = lp;
+  if (a.accept_count) a.accept_count[c] += nacc;
+}
+
+// proposal of step kk (global step gstep) of chain c from its state th, into a.prop
 template <bool kExtras>
 __device__ __forceinline__ void nr_propose(const NrArgs& a, const NrModel& m, int64_t gstep,
                                            int kk, int c, const double* th) {
   double dl[PBX_MAX_PARAMS];
   nr_draw_delta(a, m, gstep, kk, c, dl);
-  for (int j = 0; j < m.P; ++j) {
-    double v = m.log_ufun[j] ? exp(log(th[j]) + dl[j]) : th[j] + dl[j];
-    if (kExtras && m.bound) {
-      // Variable.apply_delta(bound=True), scalar branch (variable.py:700-727): closed
-      // ends clip; beyond an open end the proposal bounces back to the current value
-      const double lo = m.lims[j][0], hi = m.lims[j][1];
-      const bool olo = m.open_end[j][0] != 0, ohi = m.open_end[j][1] != 0;
-      if (!olo && !ohi) v = fmax(lo, fmin(hi, v));
-      else if (olo && ohi) v = (v > lo && v < hi) ? v : th[j];
-      else if (olo) v = (v < lo) ? th[j] : fmin(hi, v);
-      else v = (v > hi) ? th[j] : fmax(lo, v);
-    }
-    a.prop[(int64_t)j * a.C + c] = v;
-  }
+  for (int j = 0; j < m.P; ++j)
+    a.prop[(int64_t)j * a.C + c] = nr_move<kExtras>(m, j, th[j], dl[j]);
 }
 
 // log-joint from the residual sum of squares S (see file header)
@@ -195,21 +258,9 @@ __device__ void nr_phase_b(const NrArgs& a, const NrModel& m, int c, double S) {
   for (int j = 0; j < m.P; ++j) th[j] = a.state[(int64_t)j * C + c];
   double lp = a.state_lp[c];
   const double t = nr_threshold(a, a.gstep, a.k, c);
-  bool acc;
-  double s = nan("");
-  if (a.gstep == 0) {
-    acc = true;                                            // sp.py:253, sp_utils.py:24-25
-  } else if (m.accept_mode == PBX_ACCEPT_REFERENCE) {
-    // hastings_scores multiplies the linear proposal density into the LOG target
-    // (sp_utils.py:62-64); coef = 1 for metropolis
-    const double num = pbx_exp_logp(lpp * m.coef), den = pbx_exp_logp(lp * m.coef);
-    s = fmin(1.0, num / fmax(PBX_TINY, den));
-    acc = (s >= t);
-  } else {
-    const double d = m.coef * (lpp - lp);
-    acc = (d >= log(t));
-    if (a.out_score) s = fmin(1.0, exp(fmin(d, 0.0)));
-  }
+  double s;
+  const bool acc = nr_decide(m, lpp, lp, t, [&] { return log(t); }, a.gstep,
+                             a.out_score != nullptr, s);
   if (acc) {
     for (int j = 0; j < m.P; ++j) {
       th[j] = thp[j];
@@ -223,17 +274,7 @@ __device__ void nr_phase_b(const NrArgs& a, const NrModel& m, int c, double S) {
     if (a.stat_sum) a.stat_sum[(int64_t)j * C + c] += th[j];
     if (a.stat_sumsq) a.stat_sumsq[(int64_t)j * C + c] = fma(th[j], th[j], a.stat_sumsq[(int64_t)j * C + c]);
   }
-  if (a.out_accept) a.out_accept[(int64_t)a.k * C + c] = acc ? 1 : 0;
-  if (a.out_score) a.out_score[(int64_t)a.k * C + c] = s;
-  if (kExtras && a.out_xprop)
-    for (int j = 0; j < m.P; ++j) a.out_xprop[((int64_t)a.k * m.P + j) * C + c] = thp[j];
-  if (kExtras && a.out_pprop) a.out_pprop[(int64_t)a.k * C + c] = lpp;
-  if ((a.k + 1) % a.thin == 0) {
-    const int64_t r = (a.k + 1) / a.thin - 1;
-    if (a.out_x)
-      for (int j = 0; j < m.P; ++j) a.out_x[(r * m.P + j) * C + c] = th[j];
-    if (a.out_prob) a.out_prob[r * C + c] = lp;
-  }
+  nr_record<kExtras>(a, m, a.k, c, acc, s, thp, lpp, th, lp);
   // draw the proposal of the NEXT step (none after the last step of the call)
   if (a.k + 1 < a.T) nr_propose<kExtras>(a, m, a.gstep + 1, a.k + 1, c, th);
 }
@@ -531,10 +572,6 @@ static NrPlan nr_plan(pbx_ctx* ctx, const pbx_mh_normreg_params* p) {
   pl.smem = 0;
   if (variant == 1) {
     pl.kc = (C >= 4 * NR_THREADS * 8) ? 4 : ((C >= 2 * NR_THREADS * 8) ? 2 : 1);
-    if (const char* e = getenv("PBX_NR_KC")) {           // tuning experiments only
-      const int v = atoi(e);
-      if (v == 1 || v == 2 || v == 4) pl.kc = v;
-    }
     pl.n_groups = (C + NR_THREADS * pl.kc - 1) / (NR_THREADS * pl.kc);
     pl.smem = (size_t)NR_STAGES * 2 * NR_TILE * sizeof(double);     // 48 KB -> 4 CTAs / SM
     const int64_t n_full = p->n_obs / NR_TILE;
@@ -796,33 +833,12 @@ __global__ void __launch_bounds__(128) ss_walk_kernel(const NrArgs a, const __gr
     const int64_t gstep = a.step0 + k;
     double dl[PBX_MAX_PARAMS], thp[PBX_MAX_PARAMS];
     nr_draw_delta(a, m, gstep, k, c, dl);
-    for (int j = 0; j < m.P; ++j) {
-      double v = m.log_ufun[j] ? exp(log(th[j]) + dl[j]) : th[j] + dl[j];
-      if (m.bound) {                                   // variable.py:700-727
-        const double lo = m.lims[j][0], hi = m.lims[j][1];
-        const bool olo = m.open_end[j][0] != 0, ohi = m.open_end[j][1] != 0;
-        if (!olo && !ohi) v = fmax(lo, fmin(hi, v));
-        else if (olo && ohi) v = (v > lo && v < hi) ? v : th[j];
-        else if (olo) v = (v < lo) ? th[j] : fmin(hi, v);
-        else v = (v > hi) ? th[j] : fmax(lo, v);
-      }
-      thp[j] = v;
-    }
+    for (int j = 0; j < m.P; ++j) thp[j] = nr_move<true>(m, j, th[j], dl[j]);
     const double lpp = nr_logjoint(a, m, thp, ss_rss(st, m, thp));
     const double t = nr_threshold(a, gstep, k, c);
-    bool acc;
-    double s = nan("");
-    if (gstep == 0) {
-      acc = true;
-    } else if (m.accept_mode == PBX_ACCEPT_REFERENCE) {
-      const double num = pbx_exp_logp(lpp * m.coef), den = pbx_exp_logp(lp * m.coef);
-      s = fmin(1.0, num / fmax(PBX_TINY, den));
-      acc = (s >= t);
-    } else {
-      const double d = m.coef * (lpp - lp);
-      acc = (d >= log(t));
-      if (a.out_score) s = fmin(1.0, exp(fmin(d, 0.0)));
-    }
+    double s;
+    const bool acc = nr_decide(m, lpp, lp, t, [&] { return log(t); }, gstep,
+                               a.out_score != nullptr, s);
     if (acc) {
       for (int j = 0; j < m.P; ++j) th[j] = thp[j];
       lp = lpp;
@@ -832,25 +848,9 @@ __global__ void __launch_bounds__(128) ss_walk_kernel(const NrArgs a, const __gr
       ssum[j] += th[j];
       ssq[j] = fma(th[j], th[j], ssq[j]);
     }
-    if (a.out_accept) a.out_accept[(int64_t)k * C + c] = acc ? 1 : 0;
-    if (a.out_score) a.out_score[(int64_t)k * C + c] = s;
-    if (a.out_xprop)
-      for (int j = 0; j < m.P; ++j) a.out_xprop[((int64_t)k * m.P + j) * C + c] = thp[j];
-    if (a.out_pprop) a.out_pprop[(int64_t)k * C + c] = lpp;
-    if ((k + 1) % a.thin == 0) {
-      const int64_t r = (k + 1) / a.thin - 1;
-      if (a.out_x)
-        for (int j = 0; j < m.P; ++j) a.out_x[(r * m.P + j) * C + c] = th[j];
-      if (a.out_prob) a.out_prob[r * C + c] = lp;
-    }
+    nr_record<true>(a, m, k, c, acc, s, thp, lpp, th, lp);
   }
-  for (int j = 0; j < m.P; ++j) {
-    a.state[(int64_t)j * C + c] = th[j];
-    if (a.stat_sum) a.stat_sum[(int64_t)j * C + c] += ssum[j];
-    if (a.stat_sumsq) a.stat_sumsq[(int64_t)j * C + c] += ssq[j];
-  }
-  a.state_lp[c] = lp;
-  if (a.accept_count) a.accept_count[c] += nacc;
+  nr_write_back(a, m, c, th, lp, ssum, ssq, nacc);
 }
 
 
@@ -936,32 +936,11 @@ __global__ void __launch_bounds__(32 * RW_WARPS)
     _Pragma("unroll") for (int j = 0; j < P; ++j) dl[j] = __shfl_sync(0xffffffffu, dlv[j], k & 31);
     const double t = __shfl_sync(0xffffffffu, tv, k & 31);
     const double logt = __shfl_sync(0xffffffffu, ltv, k & 31);
-    _Pragma("unroll") for (int j = 0; j < P; ++j) {
-      double v = m.log_ufun[j] ? exp(log(th[j]) + dl[j]) : th[j] + dl[j];
-      if (m.bound) {                                   // variable.py:700-727
-        const double lo = m.lims[j][0], hi = m.lims[j][1];
-        const bool olo = m.open_end[j][0] != 0, ohi = m.open_end[j][1] != 0;
-        if (!olo && !ohi) v = fmax(lo, fmin(hi, v));
-        else if (olo && ohi) v = (v > lo && v < hi) ? v : th[j];
-        else if (olo) v = (v < lo) ? th[j] : fmin(hi, v);
-        else v = (v > hi) ? th[j] : fmax(lo, v);
-      }
-      thp[j] = v;
-    }
+    _Pragma("unroll") for (int j = 0; j < P; ++j) thp[j] = nr_move<true>(m, j, th[j], dl[j]);
     const double lpp = nr_logjoint<P>(a, m, thp, rss(thp));
-    bool acc;
-    double s = nan("");
-    if (gstep == 0) {
-      acc = true;
-    } else if (m.accept_mode == PBX_ACCEPT_REFERENCE) {
-      const double num = pbx_exp_logp(lpp * m.coef), den = pbx_exp_logp(lp * m.coef);
-      s = fmin(1.0, num / fmax(PBX_TINY, den));
-      acc = (s >= t);
-    } else {
-      const double d = m.coef * (lpp - lp);
-      acc = (d >= logt);
-      if (a.out_score) s = fmin(1.0, exp(fmin(d, 0.0)));
-    }
+    double s;
+    const bool acc = nr_decide(m, lpp, lp, t, [&] { return logt; }, gstep,
+                               a.out_score != nullptr, s);
     if (acc) {
       _Pragma("unroll") for (int j = 0; j < P; ++j) th[j] = thp[j];
       lp = lpp;
@@ -971,29 +950,9 @@ __global__ void __launch_bounds__(32 * RW_WARPS)
       ssum[j] += th[j];
       ssq[j] = fma(th[j], th[j], ssq[j]);
     }
-    if (lane == 0) {
-      if (a.out_accept) a.out_accept[(int64_t)k * C + c] = acc ? 1 : 0;
-      if (a.out_score) a.out_score[(int64_t)k * C + c] = s;
-      if (a.out_xprop)
-        _Pragma("unroll") for (int j = 0; j < P; ++j) a.out_xprop[((int64_t)k * P + j) * C + c] = thp[j];
-      if (a.out_pprop) a.out_pprop[(int64_t)k * C + c] = lpp;
-      if ((k + 1) % a.thin == 0) {
-        const int64_t r = (k + 1) / a.thin - 1;
-        if (a.out_x)
-          _Pragma("unroll") for (int j = 0; j < P; ++j) a.out_x[(r * P + j) * C + c] = th[j];
-        if (a.out_prob) a.out_prob[r * C + c] = lp;
-      }
-    }
+    if (lane == 0) nr_record<true, P>(a, m, k, c, acc, s, thp, lpp, th, lp);
   }
-  if (lane == 0) {
-    _Pragma("unroll") for (int j = 0; j < P; ++j) {
-      a.state[(int64_t)j * C + c] = th[j];
-      if (a.stat_sum) a.stat_sum[(int64_t)j * C + c] += ssum[j];
-      if (a.stat_sumsq) a.stat_sumsq[(int64_t)j * C + c] += ssq[j];
-    }
-    a.state_lp[c] = lp;
-    if (a.accept_count) a.accept_count[c] += nacc;
-  }
+  if (lane == 0) nr_write_back<P>(a, m, c, th, lp, ssum, ssq, nacc);
 }
 
 static bool rw_applies(const pbx_mh_normreg_params* p) {
@@ -1049,81 +1008,11 @@ static int nr_workspace(pbx_ctx* ctx, const NrPlan& pl, int C, int P, double** p
   return PBX_OK;
 }
 
-extern "C" int pbx_mh_normreg_run(pbx_ctx* ctx, const pbx_mh_normreg_params* p) {
-  PBX_REQUIRE(ctx != nullptr, "pbx_mh_normreg_run: null ctx");
-  int rc = nr_validate(p, "pbx_mh_normreg_run", true);
-  if (rc) return rc;
-  PBX_CUDA(cudaSetDevice(ctx->device));
-  NrModel m;
-  nr_fill_model(p, m);
-  if (p->variant == 3) {                       // sufficient statistics: the walk in one launch
-    NrArgs a;
-    memset(&a, 0, sizeof(a));
-    a.C = p->n_chains; a.N = p->n_obs;
-    a.state = p->state; a.state_lp = p->state_lp;
-    a.step0 = p->step0; a.T = p->n_steps; a.thin = p->thin;
-    a.chain0 = p->chain0; a.seed = p->seed;
-    a.inj_delta = p->inj_delta; a.inj_thresh = p->inj_thresh;
-    a.out_x = p->out_x; a.out_prob = p->out_prob;
-    a.out_accept = p->out_accept; a.out_score = p->out_score;
-    a.out_xprop = p->out_xprop; a.out_pprop = p->out_pprop;
-    a.accept_count = p->accept_count; a.stat_sum = p->stat_sum; a.stat_sumsq = p->stat_sumsq;
-    PBX_CUDA(cudaEventRecord(ctx->ev0, ctx->stream));
-    if (a.T > 0) {
-      NrStats* st = nullptr;
-      rc = pbx_ss_compute(ctx, m.has_slope ? p->x_obs : nullptr, p->y_obs, p->n_obs, &st);
-      if (rc) return rc;
-      ss_walk_kernel<<<(a.C + 127) / 128, 128, 0, ctx->stream>>>(a, m, st);
-      PBX_LAUNCH_CHECK(ctx);
-    }
-    PBX_CUDA(cudaEventRecord(ctx->ev1, ctx->stream));
-    return PBX_OK;
-  }
-  if (rw_applies(p)) {                         // small problem: the walk in one launch
-    PBX_REQUIRE(p->n_obs <= RW_MAXN, "pbx_mh_normreg_run: variant 4 needs n_obs <= %d", RW_MAXN);
-    NrArgs a;
-    memset(&a, 0, sizeof(a));
-    a.C = p->n_chains; a.N = p->n_obs; a.x = p->x_obs; a.y = p->y_obs;
-    a.state = p->state; a.state_lp = p->state_lp;
-    a.step0 = p->step0; a.T = p->n_steps; a.thin = p->thin;
-    a.chain0 = p->chain0; a.seed = p->seed;
-    a.inj_delta = p->inj_delta; a.inj_thresh = p->inj_thresh;
-    a.out_x = p->out_x; a.out_prob = p->out_prob;
-    a.out_accept = p->out_accept; a.out_score = p->out_score;
-    a.out_xprop = p->out_xprop; a.out_pprop = p->out_pprop;
-    a.accept_count = p->accept_count; a.stat_sum = p->stat_sum; a.stat_sumsq = p->stat_sumsq;
-    PBX_CUDA(cudaEventRecord(ctx->ev0, ctx->stream));
-    if (a.T > 0) {
-      const size_t smem = (size_t)a.N * 8 * (m.has_slope ? 2 : 1);
-      // warps (chains) per CTA: up to RW_WARPS, fewer when there are few chains, so that they
-      // spread over the SMs (every warp re-reads the resident observations each step: four
-      // warps on one SM share its 128 B/clk of shared-memory bandwidth)
-      int wpc = (a.C + 2 * ctx->sm_count - 1) / (2 * ctx->sm_count);
-      wpc = wpc < 1 ? 1 : (wpc > RW_WARPS ? RW_WARPS : wpc);
-      const int grid = (a.C + wpc - 1) / wpc;
-      if (m.has_slope) {
-        PBX_CUDA(cudaFuncSetAttribute(rw_walk_kernel<true>,
-                                      cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        rw_walk_kernel<true><<<grid, 32 * wpc, smem, ctx->stream>>>(a, m);
-      } else {
-        PBX_CUDA(cudaFuncSetAttribute(rw_walk_kernel<false>,
-                                      cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        rw_walk_kernel<false><<<grid, 32 * wpc, smem, ctx->stream>>>(a, m);
-      }
-      PBX_LAUNCH_CHECK(ctx);
-    }
-    PBX_CUDA(cudaEventRecord(ctx->ev1, ctx->stream));
-    return PBX_OK;
-  }
-  const NrPlan pl = nr_plan(ctx, p);
+// the kernel arguments of a call, without the workspace of the one-launch-per-step kernels
+static NrArgs nr_args(const pbx_mh_normreg_params* p) {
   NrArgs a;
   memset(&a, 0, sizeof(a));
   a.C = p->n_chains; a.N = p->n_obs; a.x = p->x_obs; a.y = p->y_obs;
-  a.n_slices = pl.n_slices;
-  rc = nr_workspace(ctx, pl, a.C, m.P, &a.partial, &a.counters, &a.prop);
-  if (rc) return rc;
-  a.theta_in = a.prop;
-  a.mode = 0;
   a.state = p->state; a.state_lp = p->state_lp;
   a.step0 = p->step0; a.T = p->n_steps; a.thin = p->thin;
   a.chain0 = p->chain0; a.seed = p->seed;
@@ -1132,17 +1021,78 @@ extern "C" int pbx_mh_normreg_run(pbx_ctx* ctx, const pbx_mh_normreg_params* p) 
   a.out_accept = p->out_accept; a.out_score = p->out_score;
   a.out_xprop = p->out_xprop; a.out_pprop = p->out_pprop;
   a.accept_count = p->accept_count; a.stat_sum = p->stat_sum; a.stat_sumsq = p->stat_sumsq;
+  return a;
+}
+
+static int nr_walk_suffstat(pbx_ctx* ctx, const NrArgs& a, const NrModel& m) {
+  NrStats* st = nullptr;
+  int rc = pbx_ss_compute(ctx, m.has_slope ? a.x : nullptr, a.y, a.N, &st);
+  if (rc) return rc;
+  ss_walk_kernel<<<(a.C + 127) / 128, 128, 0, ctx->stream>>>(a, m, st);
+  PBX_LAUNCH_CHECK(ctx);
+  return PBX_OK;
+}
+
+static int nr_walk_small(pbx_ctx* ctx, const NrArgs& a, const NrModel& m) {
+  const size_t smem = (size_t)a.N * 8 * (m.has_slope ? 2 : 1);
+  // warps (chains) per CTA: up to RW_WARPS, fewer when there are few chains, so that they
+  // spread over the SMs (every warp re-reads the resident observations each step: four
+  // warps on one SM share its 128 B/clk of shared-memory bandwidth)
+  int wpc = (a.C + 2 * ctx->sm_count - 1) / (2 * ctx->sm_count);
+  wpc = wpc < 1 ? 1 : (wpc > RW_WARPS ? RW_WARPS : wpc);
+  const int grid = (a.C + wpc - 1) / wpc;
+  if (m.has_slope) {
+    PBX_CUDA(cudaFuncSetAttribute(rw_walk_kernel<true>,
+                                  cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    rw_walk_kernel<true><<<grid, 32 * wpc, smem, ctx->stream>>>(a, m);
+  } else {
+    PBX_CUDA(cudaFuncSetAttribute(rw_walk_kernel<false>,
+                                  cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    rw_walk_kernel<false><<<grid, 32 * wpc, smem, ctx->stream>>>(a, m);
+  }
+  PBX_LAUNCH_CHECK(ctx);
+  return PBX_OK;
+}
+
+static int nr_walk_per_step(pbx_ctx* ctx, const NrPlan& pl, NrArgs a, const NrModel& m) {
+  if (nr_extras(a, m)) nr_init_kernel<true><<<(a.C + 255) / 256, 256, 0, ctx->stream>>>(a, m);
+  else nr_init_kernel<false><<<(a.C + 255) / 256, 256, 0, ctx->stream>>>(a, m);
+  PBX_LAUNCH_CHECK(ctx);
+  for (int k = 0; k < a.T; ++k) {
+    a.k = k;
+    a.gstep = a.step0 + k;
+    int rc = nr_launch_step(ctx, pl, a, m);
+    if (rc) return rc;
+  }
+  return PBX_OK;
+}
+
+extern "C" int pbx_mh_normreg_run(pbx_ctx* ctx, const pbx_mh_normreg_params* p) {
+  PBX_REQUIRE(ctx != nullptr, "pbx_mh_normreg_run: null ctx");
+  int rc = nr_validate(p, "pbx_mh_normreg_run", true);
+  if (rc) return rc;
+  PBX_CUDA(cudaSetDevice(ctx->device));
+  NrModel m;
+  nr_fill_model(p, m);
+  NrArgs a = nr_args(p);
+  // variant 3: sufficient statistics, else a small problem: the walk in one launch;
+  // otherwise one launch per step
+  const bool suffstat = p->variant == 3, small = !suffstat && rw_applies(p);
+  NrPlan pl{};
+  if (small) {
+    PBX_REQUIRE(p->n_obs <= RW_MAXN, "pbx_mh_normreg_run: variant 4 needs n_obs <= %d", RW_MAXN);
+  } else if (!suffstat) {
+    pl = nr_plan(ctx, p);
+    a.n_slices = pl.n_slices;
+    rc = nr_workspace(ctx, pl, a.C, m.P, &a.partial, &a.counters, &a.prop);
+    if (rc) return rc;
+    a.theta_in = a.prop;
+  }
   PBX_CUDA(cudaEventRecord(ctx->ev0, ctx->stream));
   if (a.T > 0) {
-    if (nr_extras(a, m)) nr_init_kernel<true><<<(a.C + 255) / 256, 256, 0, ctx->stream>>>(a, m);
-    else nr_init_kernel<false><<<(a.C + 255) / 256, 256, 0, ctx->stream>>>(a, m);
-    PBX_LAUNCH_CHECK(ctx);
-    for (int k = 0; k < a.T; ++k) {
-      a.k = k;
-      a.gstep = p->step0 + k;
-      rc = nr_launch_step(ctx, pl, a, m);
-      if (rc) return rc;
-    }
+    rc = suffstat ? nr_walk_suffstat(ctx, a, m)
+                  : (small ? nr_walk_small(ctx, a, m) : nr_walk_per_step(ctx, pl, a, m));
+    if (rc) return rc;
   }
   PBX_CUDA(cudaEventRecord(ctx->ev1, ctx->stream));
   return PBX_OK;
@@ -1157,12 +1107,10 @@ extern "C" int pbx_normreg_logjoint(pbx_ctx* ctx, const pbx_mh_normreg_params* p
   PBX_CUDA(cudaSetDevice(ctx->device));
   NrModel m;
   nr_fill_model(p, m);
+  NrArgs a = nr_args(p);
+  a.theta_in = theta;
+  a.eval_out = out;
   if (p->variant == 3) {
-    NrArgs a;
-    memset(&a, 0, sizeof(a));
-    a.C = p->n_chains; a.N = p->n_obs;
-    a.theta_in = theta;
-    a.eval_out = out;
     PBX_CUDA(cudaEventRecord(ctx->ev0, ctx->stream));
     NrStats* st = nullptr;
     rc = pbx_ss_compute(ctx, m.has_slope ? p->x_obs : nullptr, p->y_obs, p->n_obs, &st);
@@ -1173,15 +1121,10 @@ extern "C" int pbx_normreg_logjoint(pbx_ctx* ctx, const pbx_mh_normreg_params* p
     return PBX_OK;
   }
   const NrPlan pl = nr_plan(ctx, p);
-  NrArgs a;
-  memset(&a, 0, sizeof(a));
-  a.C = p->n_chains; a.N = p->n_obs; a.x = p->x_obs; a.y = p->y_obs;
   a.n_slices = pl.n_slices;
   rc = nr_workspace(ctx, pl, a.C, m.P, &a.partial, &a.counters, &a.prop);
   if (rc) return rc;
-  a.theta_in = theta;
   a.mode = 1;
-  a.eval_out = out;
   a.T = 1; a.thin = 1;
   PBX_CUDA(cudaEventRecord(ctx->ev0, ctx->stream));
   rc = nr_launch_step(ctx, pl, a, m);

@@ -211,6 +211,47 @@ class Engine:
                 p.open_end[j][0], p.open_end[j][1] = int(ex[j][0]), int(ex[j][1])
         return p
 
+    def _walk_outputs(self, p, out, state, state_lp, accept_count, stats, T, thin, record,
+                      per_step, inj_delta, inj_thresh):
+        """Fills ``out`` with the output tensors of a walk of ``T`` steps and sets the
+        matching pointer fields of the ABI params ``p`` (K1 and K2 share the field names).
+        ``out`` may already hold "x" / "prob" buffers to reuse; ``stats`` is a zero-filled
+        [2, D, C] tensor (stat_sum, stat_sumsq) or None."""
+        torch = _torch()
+        D, C_ = state.shape
+        R = T // thin
+        if record:
+            if "x" not in out:
+                out["x"] = self.empty(R, D, C_)
+            if "prob" not in out:
+                out["prob"] = self.empty(R, C_)
+            self._dev(out["x"], (R, D, C_), "out['x']")
+            self._dev(out["prob"], (R, C_), "out['prob']")
+        if per_step:
+            out["accept"] = self.empty(T, C_, dtype=torch.uint8)
+            out["score"] = self.empty(T, C_)
+            out["xprop"] = self.empty(T, D, C_)
+            out["pprop"] = self.empty(T, C_)
+        out["accept_count"] = accept_count
+        if stats is not None:
+            out["stat_sum"], out["stat_sumsq"] = stats[0], stats[1]
+        out["state_lp"] = state_lp
+        if inj_delta is not None:
+            if tuple(inj_delta.shape) != (T, D, C_) or tuple(inj_thresh.shape) != (T, C_):
+                raise ValueError("injected streams must be delta[T, D, C], thresh[T, C]")
+        p.state, p.state_lp = state.data_ptr(), state_lp.data_ptr()
+        p.inj_delta = 0 if inj_delta is None else inj_delta.data_ptr()
+        p.inj_thresh = 0 if inj_thresh is None else inj_thresh.data_ptr()
+        p.out_x = out["x"].data_ptr() if record else 0
+        p.out_prob = out["prob"].data_ptr() if record else 0
+        p.out_accept = out["accept"].data_ptr() if per_step else 0
+        p.out_score = out["score"].data_ptr() if per_step else 0
+        p.out_xprop = out["xprop"].data_ptr() if per_step else 0
+        p.out_pprop = out["pprop"].data_ptr() if per_step else 0
+        p.accept_count = accept_count.data_ptr()
+        p.stat_sum = stats[0].data_ptr() if stats is not None else 0
+        p.stat_sumsq = stats[1].data_ptr() if stats is not None else 0
+
     def mh_mvn(self, state, mean, cov, steps, thin=1, seed=0, step0=0, chain0=0,
                log_pscale=False, accept="reference", prop="normal", prop_scale=1.0,
                prop_chol=None, reorder=True, inj_delta=None, inj_thresh=None,
@@ -245,39 +286,9 @@ class Engine:
         zbuf = self.zeros(C_ * (2 + (2 * D if stats else 0)))
         if state_lp is None:
             state_lp = zbuf[:C_]
-        R = T // thin
-        if record:
-            if "x" not in out:
-                out["x"] = self.empty(R, D, C_)
-            if "prob" not in out:
-                out["prob"] = self.empty(R, C_)
-            self._dev(out["x"], (R, D, C_), "out['x']")
-            self._dev(out["prob"], (R, C_), "out['prob']")
-        if per_step:
-            out["accept"] = self.empty(T, C_, dtype=torch.uint8)
-            out["score"] = self.empty(T, C_)
-            out["xprop"] = self.empty(T, D, C_)
-            out["pprop"] = self.empty(T, C_)
-        out["accept_count"] = zbuf[C_:2 * C_].view(torch.int64)
-        if stats:
-            out["stat_sum"] = zbuf[2 * C_:(2 + D) * C_].view(D, C_)
-            out["stat_sumsq"] = zbuf[(2 + D) * C_:].view(D, C_)
-        out["state_lp"] = state_lp
-        if inj_delta is not None:
-            if tuple(inj_delta.shape) != (T, D, C_) or tuple(inj_thresh.shape) != (T, C_):
-                raise ValueError("injected streams must be delta[T, D, C], thresh[T, C]")
-        p.state, p.state_lp = state.data_ptr(), state_lp.data_ptr()
-        p.inj_delta = 0 if inj_delta is None else inj_delta.data_ptr()
-        p.inj_thresh = 0 if inj_thresh is None else inj_thresh.data_ptr()
-        p.out_x = out["x"].data_ptr() if record else 0
-        p.out_prob = out["prob"].data_ptr() if record else 0
-        p.out_accept = out["accept"].data_ptr() if per_step else 0
-        p.out_score = out["score"].data_ptr() if per_step else 0
-        p.out_xprop = out["xprop"].data_ptr() if per_step else 0
-        p.out_pprop = out["pprop"].data_ptr() if per_step else 0
-        p.accept_count = out["accept_count"].data_ptr()
-        p.stat_sum = out["stat_sum"].data_ptr() if stats else 0
-        p.stat_sumsq = out["stat_sumsq"].data_ptr() if stats else 0
+        self._walk_outputs(p, out, state, state_lp, zbuf[C_:2 * C_].view(torch.int64),
+                           zbuf[2 * C_:].view(2, D, C_) if stats else None, T, thin, record,
+                           per_step, inj_delta, inj_thresh)
         if events is not None:                 # torch events bracketing the kernel launch only
             events[0].record(self.stream)
         _lib.check(self.lib.pbx_mh_mvn_run(self.ctx, C.byref(p)), "pbx_mh_mvn_run")
@@ -387,35 +398,10 @@ class Engine:
             if step0 != 0:
                 raise ValueError("state_lp is required when resuming (step0 > 0)")
             state_lp = self.zeros(C_)
-        out = {"state_lp": state_lp}
-        R = T // thin
-        if record:
-            out["x"] = self.empty(R, P, C_)
-            out["prob"] = self.empty(R, C_)
-        if per_step:
-            out["accept"] = self.empty(T, C_, dtype=torch.uint8)
-            out["score"] = self.empty(T, C_)
-            out["xprop"] = self.empty(T, P, C_)
-            out["pprop"] = self.empty(T, C_)
-        out["accept_count"] = self.zeros(C_, dtype=torch.int64)
-        if stats:
-            out["stat_sum"] = self.zeros(P, C_)
-            out["stat_sumsq"] = self.zeros(P, C_)
-        if inj_delta is not None:
-            if tuple(inj_delta.shape) != (T, P, C_) or tuple(inj_thresh.shape) != (T, C_):
-                raise ValueError("injected streams must be delta[T, P, C], thresh[T, C]")
-        p.state, p.state_lp = state.data_ptr(), state_lp.data_ptr()
-        p.inj_delta = 0 if inj_delta is None else inj_delta.data_ptr()
-        p.inj_thresh = 0 if inj_thresh is None else inj_thresh.data_ptr()
-        p.out_x = out["x"].data_ptr() if record else 0
-        p.out_prob = out["prob"].data_ptr() if record else 0
-        p.out_accept = out["accept"].data_ptr() if per_step else 0
-        p.out_score = out["score"].data_ptr() if per_step else 0
-        p.out_xprop = out["xprop"].data_ptr() if per_step else 0
-        p.out_pprop = out["pprop"].data_ptr() if per_step else 0
-        p.accept_count = out["accept_count"].data_ptr()
-        p.stat_sum = out["stat_sum"].data_ptr() if stats else 0
-        p.stat_sumsq = out["stat_sumsq"].data_ptr() if stats else 0
+        out = {}
+        self._walk_outputs(p, out, state, state_lp, self.zeros(C_, dtype=torch.int64),
+                           self.zeros(2, P, C_) if stats else None, T, thin, record, per_step,
+                           inj_delta, inj_thresh)
         _lib.check(self.lib.pbx_mh_normreg_run(self.ctx, C.byref(p)), "pbx_mh_normreg_run")
         return out
 

@@ -20,4 +20,4 @@ for C in (2048, 4096, 8192, 16384):
         ev1.record(eng.stream); torch.cuda.synchronize()
         ms.append(ev0.elapsed_time(ev1) / T)
     m = float(np.median(ms[1:]))
-    print("KC=%s C=%5d: %.4f ms per MH step, %.3e terms/s" % (os.environ.get("PBX_NR_KC", "auto"), C, m, C * N / (m * 1e-3)))
+    print("C=%5d: %.4f ms per MH step, %.3e terms/s" % (C, m, C * N / (m * 1e-3)))
