@@ -134,6 +134,19 @@ def uniforms(seed, steps, chains, ndim, step0=0):
     return out
 
 
+def spherical(seed, steps, chains, ndim, radius, scale=1.0, step0=0):
+    """Spherical proposal deltas S[T, C, D] for steps step0..step0+T-1: the cube sample
+    d = -r + 2r u (u as ``uniforms``) put on the sphere of radius r, ((d r) / |d|) * scale,
+    with |d| from a sequential sum of squares (pbx_mh_mvn.cu draw_step, field.py:509-531).
+    ``scale`` is a scalar or one factor per dimension."""
+    d = -radius + (2.0 * radius) * uniforms(seed, steps, chains, ndim, step0)
+    ss = np.zeros(d.shape[:-1])
+    for j in range(ndim):
+        ss = ss + d[..., j] * d[..., j]
+    nrm = np.where(ss >= 2.2250738585072014e-308, np.sqrt(ss), 0.0)
+    return ((d * radius) / nrm[..., None]) * np.broadcast_to(np.asarray(scale, float), (ndim,))
+
+
 def thresholds(seed, steps, chains, step0=0):
     """Accept thresholds U[T, C]."""
     t = (np.arange(steps, dtype=np.uint64) + np.uint64(step0))[:, None]
