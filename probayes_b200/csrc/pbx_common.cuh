@@ -204,20 +204,6 @@ __device__ __forceinline__ bool pbx_mbar_try_wait(void* bar, uint32_t parity) {
       : "memory");
   return ok != 0;
 }
-// non-blocking probe (try_wait may suspend the warp for a HW time slice)
-__device__ __forceinline__ bool pbx_mbar_test_wait(void* bar, uint32_t parity) {
-  uint32_t ok;
-  asm volatile(
-      "{\n"
-      ".reg .pred p;\n"
-      "mbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n"
-      "selp.u32 %0, 1, 0, p;\n"
-      "}\n"
-      : "=r"(ok)
-      : "r"(pbx_smem_u32(bar)), "r"(parity)
-      : "memory");
-  return ok != 0;
-}
 __device__ __forceinline__ void pbx_mbar_wait(void* bar, uint32_t parity) {
   while (!pbx_mbar_try_wait(bar, parity)) {
   }
@@ -232,8 +218,5 @@ __device__ __forceinline__ void pbx_bulk_g2s(void* dst_smem, const void* src_gme
 }
 __device__ __forceinline__ void pbx_fence_barrier_init() {
   asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-}
-__device__ __forceinline__ void pbx_fence_proxy_async() {
-  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
 }
 #endif

@@ -6,19 +6,25 @@
 // Layout: state[D][C], outputs [..][D][C] / [..][C] -- chain-minor so a warp of 32
 // chains reads/writes 256 contiguous bytes per dimension.
 //
-// Two kernels, identical arithmetic (bit-identical results for the same seed):
+// Three kernels, one draw per (step, chain) and the same arithmetic on the state:
 //  * mh_mvn_kernel     one thread = one chain, state + running sums in registers,
 //                      Philox4x32-10 + Box-Muller in-thread or INJECTED streams (the
-//                      bit-parity path), per-step accept/score outputs.
-//  * mh_mvn_ws_kernel  warp-specialised native-RNG fast path.  A CTA owns 32 chains:
-//                      12 (D <= 3) or 9 producer warps draw Philox blocks and turn them into
-//                      proposal deltas and log-thresholds for batches of steps (that
-//                      work does not depend on the chain state, so it parallelises
-//                      over steps), hand them through a shared-memory ring guarded
+//                      bit-parity path), per-step accept/score outputs, bound=True.
+//  * mh_mvn_ws_kernel  warp-specialised native-RNG path (reference rule, D >= 5,
+//                      kernel_variant 2).  A CTA owns 32 chains: 12 (D <= 3) or 9 producer
+//                      warps draw Philox blocks and turn them into proposal deltas and
+//                      log-thresholds for batches of steps (that work does not depend on
+//                      the chain state, so it parallelises over steps), hand them through
+//                      a shared-memory ring guarded
 //                      by mbarriers to ONE consumer warp that runs the inherently
 //                      sequential part (propose, 2-D quadratic form, accept, record)
 //                      for its 32 chains.  This takes a 4096-chain walk from one
 //                      latency-bound warp per SM to ~16 busy warps per SM.
+//  * mh_mvn_wd_kernel  whitened decisions (native RNG, log rule, D <= 4): the default.  The
+//                      producers also whiten the deltas, so the decision warp's step is one
+//                      D-term dot product and a compare (see the comment at the kernel).
+// All three record bit-identical trajectories and densities for the same seed; the
+// whitened decisions can differ only within the rounding of the tracked whitened state.
 #include <math.h>
 #include "pbx_common.cuh"
 
@@ -125,6 +131,23 @@ __device__ __noinline__ double out_exp_slow(double l) { return exp(l); }
 __device__ __forceinline__ double out_exp(double l, const PbxTables* tb) {
   return (l > -700.0 && l < 700.0) ? fast_exp(l, tb) : out_exp_slow(l);
 }
+// Density recorded for a retained state of log-density lp: lp itself under the log pscale,
+// else pdf = exp(logpdf) as scipy does -- libm's under the reference rule (bit-equal to the
+// linear density that rule decides with), the table exp under the log rule
+__device__ __forceinline__ double rec_density(double lp, bool log_pscale, bool ref,
+                                              const PbxTables* tb) {
+  return log_pscale ? lp : (ref ? exp(lp) : out_exp(lp, tb));
+}
+
+// The warp-specialised kernels read the tables from a copy in shared memory, made by all
+// kThreads threads of the CTA (the caller synchronises before the first use)
+template <int kThreads>
+__device__ __forceinline__ void stage_tables(PbxTables& s_tb) {
+  const double* src = reinterpret_cast<const double*>(&g_tables);
+  double* dst = reinterpret_cast<double*>(&s_tb);
+  for (int i = threadIdx.x; i < (int)(sizeof(PbxTables) / sizeof(double)); i += kThreads)
+    dst[i] = src[i];
+}
 
 static int init_tables(pbx_ctx* ctx) {
   // per context (one per device and process; a context is not thread-safe): no process-wide
@@ -194,36 +217,33 @@ struct MhMvnArgs {
   double* out_pprop;
 };
 
-// scipy multivariate_normal_gen._logpdf: -0.5*(rank*log(2pi) + log_pdet + maha),
-// maha = sum(square(dev @ U)).
-// kZeroMean: the target mean is exactly 0 in every dimension; x - 0.0 == x bit for
+// Whitening y = W^T (v - mean) (dev @ U in scipy's terms), handed to emit(k, y_k) one
+// component at a time in dimension order, so that a caller that only sums y_k^2 never holds
+// the whole vector (which costs the D = 7 per-thread kernel 21 registers).
+// kZeroMean: the target mean is exactly 0 in every dimension; v - 0.0 == v bit for
 // bit, so the subtraction is dropped (one FP64 op per dimension off the consumer's
-// instruction budget).
-template <int D, bool kZeroMean = false>
-__device__ __forceinline__ double mvn_maha(const double (&x)[D], const MhMvnConst& m) {
+// instruction budget).  A displacement is whitened without the mean: kZeroMean = true.
+template <int D, bool kZeroMean, class Emit>
+__device__ __forceinline__ void whiten(const double (&v)[D], const MhMvnConst& m, Emit emit) {
   double dev[D];
 #pragma unroll
-  for (int j = 0; j < D; ++j) dev[j] = kZeroMean ? x[j] : x[j] - m.mean[j];
-  double maha = 0.0;
+  for (int j = 0; j < D; ++j) dev[j] = kZeroMean ? v[j] : v[j] - m.mean[j];
 #pragma unroll
   for (int k = 0; k < D; ++k) {
-    double y = 0.0;
+    double e = 0.0;
 #pragma unroll
-    for (int j = 0; j < D; ++j) y = fma(dev[j], m.W[j * D + k], y);
-    maha = fma(y, y, maha);
+    for (int j = 0; j < D; ++j) e = fma(dev[j], m.W[j * D + k], e);
+    emit(k, e);
   }
+}
+// scipy multivariate_normal_gen._logpdf: -0.5*(rank*log(2pi) + log_pdet + maha),
+// maha = sum(square(dev @ U)).
+template <int D, bool kZeroMean = false>
+__device__ __forceinline__ double mvn_maha(const double (&x)[D], const MhMvnConst& m) {
+  double maha = 0.0;
+  whiten<D, kZeroMean>(x, m, [&](int, double y) { maha = fma(y, y, maha); });
   return maha;
 }
-template <int D>
-__device__ __forceinline__ double mvn_logpdf(const double (&x)[D], const MhMvnConst& m) {
-  return -0.5 * (m.norm_c + mvn_maha<D>(x, m));
-}
-// Log-space accept test on the Mahalanobis distance: logp' - logp >= log t with
-// logp = -0.5 (c + maha)  <=>  maha' <= maha - 2 log t.  The right-hand side depends
-// only on the CURRENT state and the threshold draw, so it is off the sequential
-// critical path (the chain per step is add, sub, mul, fma, mul, fma, setp, select)
-// and the chain never needs logp itself (the writer derives it from maha).
-__device__ __forceinline__ double neg2log(double logt) { return -2.0 * logt; }
 
 template <int D, bool kNormalOnly = false>
 __device__ __forceinline__ void draw_step(uint64_t seed, uint64_t gstep, uint32_t gchain,
@@ -281,6 +301,23 @@ __device__ __forceinline__ void colour_delta(int has_L, const MhMvnConst& m, con
 #pragma unroll
     for (int j = 0; j < D; ++j) v[j] = dl[j];
   }
+}
+
+// End of a walk for chain c: the retained state, its log-density and the accept count, and
+// the chain's running sums added to the caller's (ssum / ssq null: the caller adds them)
+template <int D>
+__device__ __forceinline__ void write_back(const MhMvnArgs& a, int c, const double (&x)[D],
+                                           double lp, int64_t nacc, const double* ssum,
+                                           const double* ssq) {
+  const int64_t C = a.C;
+#pragma unroll
+  for (int j = 0; j < D; ++j) {
+    a.state[j * C + c] = x[j];
+    if (ssum && a.stat_sum) a.stat_sum[j * C + c] += ssum[j];
+    if (ssq && a.stat_sumsq) a.stat_sumsq[j * C + c] += ssq[j];
+  }
+  a.state_lp[c] = lp;
+  if (a.accept_count) a.accept_count[c] += nacc;
 }
 
 template <int D, bool kInjected>
@@ -346,12 +383,17 @@ __global__ void __launch_bounds__(128) mh_mvn_kernel(const MhMvnArgs a,
         acc = (s >= t);
       }
     } else {
+      // Log-space accept test on the Mahalanobis distance: logp' - logp >= log t with
+      // logp = -0.5 (c + maha)  <=>  maha' <= maha - 2 log t.  The right-hand side depends
+      // only on the CURRENT state and the threshold draw, so it is off the sequential
+      // critical path (the chain per step is add, sub, mul, fma, mul, fma, setp, select)
+      // and the chain never needs logp itself (the writer derives it from maha).
       if (gstep == 0) {
         acc = true;
       } else {
         // injected thresholds go through libm's log (bit-parity with the oracle);
         // native ones through the same table log as the warp-specialised kernel
-        const double th2 = kInjected ? neg2log(log(t)) : fast_neg2log(t, &g_tables);
+        const double th2 = kInjected ? -2.0 * log(t) : fast_neg2log(t, &g_tables);
         acc = (maha <= mcur + th2);
         if (a.out_score) s = fmin(1.0, exp(fmin(lpp - lp, 0.0)));
       }
@@ -384,20 +426,10 @@ __global__ void __launch_bounds__(128) mh_mvn_kernel(const MhMvnArgs a,
 #pragma unroll
         for (int j = 0; j < D; ++j) a.out_x[(r * D + j) * C + c] = x[j];
       }
-      if (a.out_prob) {
-        double pv = a.log_pscale ? lp : (ref_mode ? lin : out_exp(lp, &g_tables));
-        a.out_prob[r * C + c] = pv;
-      }
+      if (a.out_prob) a.out_prob[r * C + c] = rec_density(lp, a.log_pscale, ref_mode, &g_tables);
     }
   }
-#pragma unroll
-  for (int j = 0; j < D; ++j) {
-    a.state[j * C + c] = x[j];
-    if (a.stat_sum) a.stat_sum[j * C + c] += ssum[j];
-    if (a.stat_sumsq) a.stat_sumsq[j * C + c] += ssq[j];
-  }
-  a.state_lp[c] = lp;
-  if (a.accept_count) a.accept_count[c] += nacc;
+  write_back(a, c, x, lp, nacc, ssum, ssq);
 }
 
 // ---------------------------------------------------------------------------
@@ -417,34 +449,9 @@ __global__ void __launch_bounds__(128) mh_mvn_kernel(const MhMvnArgs a,
 // One mbarrier pair per slot: in_full (producer -> consumer), out_full (consumer
 // -> owning producer).
 // ---------------------------------------------------------------------------
-#ifndef WS_NPROD
-#define WS_NPROD 12                      // producer warps: all warps with (warp % 4) != 0
-#endif
-#define WS_NSLOT (2 * WS_NPROD)             // two ring slots per producer warp
-#ifndef WS_PUNROLL
-#define WS_PUNROLL 4
-#endif
-constexpr int kWsPUnroll = WS_PUNROLL;
-#ifndef WS_THREADS
-#define WS_THREADS 512                   // 16 warps; warps 4, 8, 12 exit at once so that
-#endif
-                                         // the consumer (warp 0) has its SM sub-partition
-                                         // (scheduler + FP64 pipe) to itself
-#ifndef WS_G2
-#define WS_G2 8                          // steps per ring slot for D <= 2
-#endif
-#ifndef WS_BIGCTA_MAXD
-#define WS_BIGCTA_MAXD 3                 // largest D that runs the 512-thread CTA
-#endif
-#ifndef WS_BIGCTA_MIND
-#define WS_BIGCTA_MIND 99                // smallest D (beyond MAXD) that runs it again
-#endif
-#ifndef WS_SMALL_NPROD
-#define WS_SMALL_NPROD 9                 // producers of the small CTA (+ consumer + idle warps)
-#endif
 template <int D> struct WsCfg {
   // steps per ring slot: G*(D+1) doubles per lane per slot, <= 6 KB per slot
-  static constexpr int G = (D <= 2) ? WS_G2 : (D == 3 ? 6 : (D <= 5 ? 4 : (D <= 7 ? 3 : 2)));
+  static constexpr int G = (D <= 2) ? 8 : (D == 3 ? 6 : (D <= 5 ? 4 : (D <= 7 ? 3 : 2)));
   static constexpr int SLOT_DOUBLES = G * (D + 1) * 32;
   // CTA shape (measured, 4096 chains x 10^4 steps): 12 producer warps in a 512-thread CTA
   // (128 registers per thread) for D <= 3 -- 0.546 ms at D = 2 against 0.559 with 15
@@ -453,11 +460,10 @@ template <int D> struct WsCfg {
   // From D = 4 on the consumer's state + D x D quadratic form dominate and want registers:
   // 9 producers / 384 threads (up to 168 registers; D = 6: 1.70 -> 1.39 ms, D = 8: 6.5 ->
   // 3.9 ms against the 15-producer shape).
-  static constexpr bool BIG = (D <= WS_BIGCTA_MAXD) || (D >= WS_BIGCTA_MIND);
-  static constexpr int NPROD = BIG ? WS_NPROD : WS_SMALL_NPROD;
-  static constexpr int NSLOT = 2 * NPROD;
-  static constexpr int THREADS =
-      BIG ? WS_THREADS : 32 * (WS_SMALL_NPROD + 1 + (WS_SMALL_NPROD - 1) / 3);
+  // The producers are the warps with warp % 4 != 0 (see above): 12 of 16 warps, 9 of 12.
+  static constexpr int NPROD = (D <= 3) ? 12 : 9;
+  static constexpr int NSLOT = 2 * NPROD;                 // two ring slots per producer warp
+  static constexpr int THREADS = 32 * (NPROD + 1 + (NPROD - 1) / 3);
   static constexpr size_t SMEM = (size_t)NSLOT * SLOT_DOUBLES * sizeof(double);
 };
 
@@ -471,13 +477,8 @@ __global__ void __launch_bounds__(WsCfg<D>::THREADS, 1)
   constexpr int NP = WsCfg<D>::NPROD, NS = WsCfg<D>::NSLOT;
   extern __shared__ __align__(16) double ring[];          // [NS][G][D+1][32]
   __shared__ __align__(8) unsigned long long in_full[NS], out_full[NS];
-  __shared__ __align__(16) PbxTables s_tb;                // 32.5 KB of math tables
-  {
-    const double* src = reinterpret_cast<const double*>(&g_tables);
-    double* dst = reinterpret_cast<double*>(&s_tb);
-    for (int i = threadIdx.x; i < (int)(sizeof(PbxTables) / sizeof(double)); i += WsCfg<D>::THREADS)
-      dst[i] = src[i];
-  }
+  __shared__ __align__(16) PbxTables s_tb;                // 40 KB of math tables
+  stage_tables<WsCfg<D>::THREADS>(s_tb);
   const PbxTables* tb = &s_tb;
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -515,13 +516,16 @@ __global__ void __launch_bounds__(WsCfg<D>::THREADS, 1)
           if (valid) {
             double* ox = a.out_x + ((int64_t)k0 * D) * C + c;
             double* op = a.out_prob + (int64_t)k0 * C + c;
+            // the consumer leaves logp (reference rule) or the Mahalanobis distance (log
+            // rule) of the retained state in the slot
             if (a.log_pscale) {
 #pragma unroll
               for (int g = 0; g < G; ++g) {
 #pragma unroll
                 for (int j = 0; j < D; ++j) ox[(g * D + j) * C] = slot[(g * (D + 1) + j) * 32];
                 const double sv = slot[(g * (D + 1) + D) * 32];
-                op[g * C] = kRefAccept ? sv : -0.5 * (m.norm_c + sv);
+                const double lpv = kRefAccept ? sv : -0.5 * (m.norm_c + sv);
+                op[g * C] = rec_density(lpv, true, kRefAccept, tb);
               }
             } else {
 #pragma unroll
@@ -530,38 +534,35 @@ __global__ void __launch_bounds__(WsCfg<D>::THREADS, 1)
                 for (int j = 0; j < D; ++j) ox[(g * D + j) * C] = slot[(g * (D + 1) + j) * 32];
                 const double sv = slot[(g * (D + 1) + D) * 32];
                 const double lpv = kRefAccept ? sv : -0.5 * (m.norm_c + sv);
-                op[g * C] = kRefAccept ? exp(lpv) : out_exp(lpv, tb);
+                op[g * C] = rec_density(lpv, false, kRefAccept, tb);
               }
             }
           }
         } else {
-        int rem = (k0 + 1) % a.thin;                      // (k+1) % thin of step k0
-        const int64_t rec0 = (k0 + 1) / a.thin - 1 + (rem != 0);   // first record index
-        double* ox = a.out_x ? a.out_x + (rec0 * D) * C + c : nullptr;
-        double* op = a.out_prob ? a.out_prob + rec0 * C + c : nullptr;
-        if (rem == 0) rem = a.thin;                       // countdown form: record when == thin
-        for (int g = 0; g < ng; ++g) {
-          if (rem == a.thin) {
-            rem = 0;
-            if (valid) {
-              if (ox) {
+          int rem = (k0 + 1) % a.thin;                    // (k+1) % thin of step k0
+          const int64_t rec0 = (k0 + 1) / a.thin - 1 + (rem != 0);   // first record index
+          double* ox = a.out_x ? a.out_x + (rec0 * D) * C + c : nullptr;
+          double* op = a.out_prob ? a.out_prob + rec0 * C + c : nullptr;
+          if (rem == 0) rem = a.thin;                     // countdown form: record when == thin
+          for (int g = 0; g < ng; ++g) {
+            if (rem == a.thin) {
+              rem = 0;
+              if (valid) {
+                if (ox) {
 #pragma unroll
-                for (int j = 0; j < D; ++j) ox[j * C] = slot[(g * (D + 1) + j) * 32];
-                ox += D * C;
-              }
-              if (op) {
-                // the consumer leaves logp (reference rule) or the Mahalanobis distance
-                // (log rule) of the retained state in the slot
-                const double sv = slot[(g * (D + 1) + D) * 32];
-                const double lpv = kRefAccept ? sv : -0.5 * (m.norm_c + sv);
-                // linear pscale: pdf = exp(logpdf) as scipy does
-                *op = a.log_pscale ? lpv : (kRefAccept ? exp(lpv) : out_exp(lpv, tb));
-                op += C;
+                  for (int j = 0; j < D; ++j) ox[j * C] = slot[(g * (D + 1) + j) * 32];
+                  ox += D * C;
+                }
+                if (op) {
+                  const double sv = slot[(g * (D + 1) + D) * 32];
+                  const double lpv = kRefAccept ? sv : -0.5 * (m.norm_c + sv);
+                  *op = rec_density(lpv, a.log_pscale, kRefAccept, tb);
+                  op += C;
+                }
               }
             }
+            ++rem;
           }
-          ++rem;
-        }
         }
       }
       if (n >= n_mine) continue;
@@ -577,11 +578,11 @@ __global__ void __launch_bounds__(WsCfg<D>::THREADS, 1)
         slot[(g * (D + 1) + D) * 32] = kRefAccept ? t : fast_neg2log(t, tb);
       };
       if ((b + 1) * G <= a.T) {
-        // full batch: WS_PUNROLL independent steps in flight per thread (ILP), since a
+        // full batch: kUnroll independent steps in flight per thread (ILP), since a
         // producer warp is otherwise a single chain of dependent instructions
         // (D <= 3: four independent steps in flight in the 128-register shape -- 0.547 ->
         // 0.532 ms at D = 2; D = 4: two; beyond that one, the draws of a step fill the file)
-        constexpr int kUnroll = (D <= 3) ? (kRefAccept ? 2 : kWsPUnroll) : (D == 4 ? 2 : 1);
+        constexpr int kUnroll = (D <= 3) ? (kRefAccept ? 2 : 4) : (D == 4 ? 2 : 1);
 #pragma unroll kUnroll
         for (int g = 0; g < G; ++g) produce(g);
       } else {
@@ -689,12 +690,10 @@ __global__ void __launch_bounds__(WsCfg<D>::THREADS, 1)
       nacc += (int)aa + (int)ab;
 #pragma unroll
       for (int j = 0; j < D; ++j) {
-#ifndef PBX_K1_NOSTATS
         ssum[j] += s1[j];
         ssq[j] = fma(s1[j], s1[j], ssq[j]);
         ssum[j] += x[j];
         ssq[j] = fma(x[j], x[j], ssq[j]);
-#endif
         slot[(g * (D + 1) + j) * 32] = s1[j];
         slot[((g + 1) * (D + 1) + j) * 32] = x[j];
       }
@@ -717,6 +716,8 @@ __global__ void __launch_bounds__(WsCfg<D>::THREADS, 1)
     __syncwarp();
     if (lane == 0) pbx_mbar_arrive(&out_full[s]);
   }
+  // written out rather than through write_back: with the helper ptxas schedules the consumer
+  // loop differently, and the D = 6 walk of scripts/bench_k1_dims.py ran 3 % slower (B200)
   if (valid) {
 #pragma unroll
     for (int j = 0; j < D; ++j) {
@@ -760,19 +761,7 @@ __global__ void __launch_bounds__(WsCfg<D>::THREADS, 1)
 // Ring of NSLOT batches in shared memory, [field pair][item] as double2 (128-bit
 // conflict-free accesses on both sides), one mbarrier pair per slot.
 // ---------------------------------------------------------------------------
-#define WD_NPROD 14
-#define WD_ITEMS (WD_NPROD * 32)
-#define WD_THREADS 512                // 16 warps: decisions, 14 producers, one idle (see below)
-#define WD_MAXD 4
-#ifndef WD_NSLOT
-#define WD_NSLOT 3                    // ring depth in batches for D <= 2
-#endif
-#ifndef WD_IPT
-#define WD_IPT 1                      // measured: 2 (four steps in flight per thread) gains nothing
-#endif
-#ifndef WD_PF
-#define WD_PF 2                       // pairs in flight in the decision warp's registers (D <= 2)
-#endif
+constexpr int kWdMaxD = 4;
 // shared-memory accesses of the decision warp by 32-bit shared-space address (a generic
 // pointer makes the compiler rebuild the shared window base -- S2UR SR_CgaCtaId, ~100 cycles
 // -- in front of every access of the loop); volatile keeps fetches and stores in program order
@@ -785,42 +774,36 @@ __device__ __forceinline__ void pbx_sts_v2(uint32_t addr, double a, double b) {
   asm volatile("st.shared.v2.f64 [%0], {%1, %2};" ::"r"(addr), "d"(a), "d"(b) : "memory");
 }
 template <int D> struct WdCfg {
+  static constexpr int THREADS = 512;   // 16 warps: decisions, 14 producers, one idle (see below)
+  static constexpr int NPROD = 14;
+  // one item per producer thread and batch (two, i.e. four steps in flight per thread,
+  // measured no gain)
+  static constexpr int ITEMS = NPROD * 32;
   static constexpr int NF2 = 2 * D + 2;   // double2 per item: eA[D] eB[D] kA kB0 kB1 pad dA[D] dB[D]
-  // items per producer thread and batch (build-time experiment knob; 2 = four steps in
-  // flight per thread, needs the doubled slots to fit into shared memory)
-  static constexpr int IPT = (D <= 2) ? WD_IPT : 1;
-  static constexpr int ITEMS = WD_ITEMS * IPT;
-  static constexpr int NSLOT = (D <= 2 && IPT == 1) ? WD_NSLOT : 2;
+  static constexpr int NSLOT = (D <= 2) ? 3 : 2;          // ring depth in batches
   static constexpr size_t SMEM = (size_t)NSLOT * NF2 * ITEMS * sizeof(double2);
 };
 
 template <int D, bool kFast, bool kZeroMean>
-__global__ void __launch_bounds__(WD_THREADS, 1)
+__global__ void __launch_bounds__(WdCfg<D>::THREADS, 1)
     mh_mvn_wd_kernel(const MhMvnArgs a, const __grid_constant__ MhMvnConst m, const int cpc) {
   constexpr int NF2 = WdCfg<D>::NF2;
   constexpr int NS = WdCfg<D>::NSLOT;
-  constexpr int IPT = WdCfg<D>::IPT;
   constexpr int ITEMS = WdCfg<D>::ITEMS;
   extern __shared__ __align__(16) double2 ring2[];        // [NS][NF2][ITEMS]
   __shared__ __align__(8) unsigned long long in_full[NS], out_full[NS];
   __shared__ __align__(16) PbxTables s_tb;
-  {
-    const double* src = reinterpret_cast<const double*>(&g_tables);
-    double* dst = reinterpret_cast<double*>(&s_tb);
-    for (int i = threadIdx.x; i < (int)(sizeof(PbxTables) / sizeof(double)); i += WD_THREADS)
-      dst[i] = src[i];
-  }
+  stage_tables<WdCfg<D>::THREADS>(s_tb);
   const PbxTables* tb = &s_tb;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int64_t C = a.C;
-  const int P0 = WD_ITEMS / cpc;                // pairs of steps per batch and item index
-  const int P = IPT * P0;                       // pairs of steps per batch
+  const int P = ITEMS / cpc;                    // pairs of steps per batch
   const int S = 2 * P;                          // steps per batch
   const int nb = (a.T + S - 1) / S;
   const int cbase = blockIdx.x * cpc;
   if (threadIdx.x == 0) {
     for (int i = 0; i < NS; ++i) {
-      pbx_mbar_init(&in_full[i], WD_NPROD);
+      pbx_mbar_init(&in_full[i], WdCfg<D>::NPROD);
       pbx_mbar_init(&out_full[i], 1);
     }
   }
@@ -842,67 +825,63 @@ __global__ void __launch_bounds__(WD_THREADS, 1)
     const bool valid = c < a.C;
     const uint32_t gchain = (uint32_t)(a.chain0 + (valid ? c : 0));
     const bool rec_all = a.thin == 1 && a.out_x != nullptr && a.out_prob != nullptr;
-    // My items of a batch: pairs pr + k P0 (k < IPT) of chain ch.  Records of the batch being
-    // drained (thin == 1: record index = step index) through running pointers.
+    // My item of a batch: pair pr of chain ch.  Records of the batch being drained
+    // (thin == 1: record index = step index) through running pointers.
     double* px = rec_all ? a.out_x + ((int64_t)(2 * pr) * D) * C + c : nullptr;
     double* pp = rec_all ? a.out_prob + (int64_t)(2 * pr) * C + c : nullptr;
-    const int64_t kx = (int64_t)(2 * P0) * D * C, kp = (int64_t)(2 * P0) * C;
     for (int b = 0; b < nb + NS; ++b) {
       const int s = b % NS;
       double2* slot = ring2 + (size_t)s * NF2 * ITEMS + item;
       if (b >= NS) {
-        // ---- drain my items of batch b - NS: the states after steps A and B -------------
+        // ---- drain my item of batch b - NS: the states after steps A and B --------------
         const int bd = b - NS;
         pbx_mbar_wait(&out_full[s], (uint32_t)(bd / NS) & 1);
         const bool whole = rec_all && (bd + 1) * S <= a.T;
+        double r[2 * D];
 #pragma unroll
-        for (int k = 0; k < IPT; ++k) {
-          double r[2 * D];
+        for (int q = 0; q < D; ++q) {
+          const double2 t2 = slot[(D + 2 + q) * ITEMS];
+          r[2 * q] = t2.x;
+          r[2 * q + 1] = t2.y;
+        }
+        const int kA = bd * S + 2 * pr;
+        if (valid && whole) {
+          // common case (every step recorded, whole batch live): straight-line code
 #pragma unroll
-          for (int q = 0; q < D; ++q) {
-            const double2 t2 = slot[(D + 2 + q) * ITEMS + k * WD_ITEMS];
-            r[2 * q] = t2.x;
-            r[2 * q + 1] = t2.y;
+          for (int h = 0; h < 2; ++h) {
+            double xs[D];
+#pragma unroll
+            for (int j = 0; j < D; ++j) {
+              xs[j] = r[h * D + j];
+              ssum[j] += xs[j];
+              ssq[j] = fma(xs[j], xs[j], ssq[j]);
+              px[(h * D + j) * C] = xs[j];
+            }
+            const double lpv = -0.5 * (m.norm_c + mvn_maha<D, kZeroMean>(xs, m));
+            pp[h * C] = rec_density(lpv, a.log_pscale, false, tb);
           }
-          const int kA = bd * S + 2 * (pr + k * P0);
-          if (valid && whole) {
-            // common case (every step recorded, whole batch live): straight-line code
+        } else if (valid) {
 #pragma unroll
-            for (int h = 0; h < 2; ++h) {
+          for (int h = 0; h < 2; ++h) {
+            const int kk = kA + h;
+            if (kk < a.T) {
               double xs[D];
 #pragma unroll
               for (int j = 0; j < D; ++j) {
                 xs[j] = r[h * D + j];
                 ssum[j] += xs[j];
                 ssq[j] = fma(xs[j], xs[j], ssq[j]);
-                px[k * kx + (h * D + j) * C] = xs[j];
               }
-              const double lpv = -0.5 * (m.norm_c + mvn_maha<D, kZeroMean>(xs, m));
-              pp[k * kp + h * C] = a.log_pscale ? lpv : out_exp(lpv, tb);
-            }
-          } else if (valid) {
+              const bool keep = ((kk + 1) % a.thin) == 0;
+              const int64_t rec = (kk + 1) / a.thin - 1;
+              if (keep) {
+                if (a.out_x) {
 #pragma unroll
-            for (int h = 0; h < 2; ++h) {
-              const int kk = kA + h;
-              if (kk < a.T) {
-                double xs[D];
-#pragma unroll
-                for (int j = 0; j < D; ++j) {
-                  xs[j] = r[h * D + j];
-                  ssum[j] += xs[j];
-                  ssq[j] = fma(xs[j], xs[j], ssq[j]);
+                  for (int j = 0; j < D; ++j) a.out_x[(rec * D + j) * C + c] = xs[j];
                 }
-                const bool keep = ((kk + 1) % a.thin) == 0;
-                const int64_t rec = (kk + 1) / a.thin - 1;
-                if (keep) {
-                  if (a.out_x) {
-#pragma unroll
-                    for (int j = 0; j < D; ++j) a.out_x[(rec * D + j) * C + c] = xs[j];
-                  }
-                  if (a.out_prob) {
-                    const double lpv = -0.5 * (m.norm_c + mvn_maha<D, kZeroMean>(xs, m));
-                    a.out_prob[rec * C + c] = a.log_pscale ? lpv : out_exp(lpv, tb);
-                  }
+                if (a.out_prob) {
+                  const double lpv = -0.5 * (m.norm_c + mvn_maha<D, kZeroMean>(xs, m));
+                  a.out_prob[rec * C + c] = rec_density(lpv, a.log_pscale, false, tb);
                 }
               }
             }
@@ -914,49 +893,41 @@ __global__ void __launch_bounds__(WD_THREADS, 1)
         }
       }
       if (b >= nb) continue;
-      // ---- draw my pairs of steps of batch b (IPT independent pairs: ILP) ------------------
+      // ---- draw my pair of steps of batch b --------------------------------------------------
+      const int64_t gA = a.step0 + (int64_t)b * S + 2 * pr;
+      double eA[D], eB[D], dA_[D], dB_[D], kA_, kB_;
+      auto gen = [&](int64_t gstep, double (&eta)[D], double (&dv)[D], double& kap) {
+        double dl[D], t;
+        draw_step<D, kFast>(a.seed, (uint64_t)gstep, gchain, a.prop_kind, m, tb, dl, t);
+        colour_delta<D>(kFast ? 0 : a.has_L, m, dl, dv);
+        const double th = fast_neg2log(t, tb);
+        double n2 = 0.0;                         // |e|^2
+        whiten<D, true>(dv, m, [&](int k, double e) {
+          eta[k] = e;
+          n2 = fma(e, e, n2);
+        });
+        kap = 0.5 * (th - n2);
+      };
+      gen(gA, eA, dA_, kA_);
+      gen(gA + 1, eB, dB_, kB_);
+      double cross = 0.0;
 #pragma unroll
-      for (int k = 0; k < IPT; ++k) {
-        const int64_t gA = a.step0 + (int64_t)b * S + 2 * (pr + k * P0);
-        double eA[D], eB[D], dA_[D], dB_[D], kA_, kB_;
-        auto gen = [&](int64_t gstep, double (&eta)[D], double (&dv)[D], double& kap) {
-          double dl[D], t;
-          draw_step<D, kFast>(a.seed, (uint64_t)gstep, gchain, a.prop_kind, m, tb, dl, t);
-          colour_delta<D>(kFast ? 0 : a.has_L, m, dl, dv);
-          const double th = fast_neg2log(t, tb);
-          double n2 = 0.0;
+      for (int kk = 0; kk < D; ++kk) cross = fma(eA[kk], eB[kk], cross);
+      double v[4 * D + 4];
 #pragma unroll
-          for (int kk = 0; kk < D; ++kk) {
-            double e = 0.0;
-#pragma unroll
-            for (int j = 0; j < D; ++j) e = fma(dv[j], m.W[j * D + kk], e);
-            eta[kk] = e;
-            n2 = fma(e, e, n2);
-          }
-          kap = 0.5 * (th - n2);
-        };
-        gen(gA, eA, dA_, kA_);
-        gen(gA + 1, eB, dB_, kB_);
-        double cross = 0.0;
-#pragma unroll
-        for (int kk = 0; kk < D; ++kk) cross = fma(eA[kk], eB[kk], cross);
-        double v[4 * D + 4];
-#pragma unroll
-        for (int j = 0; j < D; ++j) {
-          v[j] = eA[j];
-          v[D + j] = eB[j];
-          v[2 * D + 4 + j] = dA_[j];
-          v[3 * D + 4 + j] = dB_[j];
-        }
-        v[2 * D] = kA_;
-        v[2 * D + 1] = kB_;
-        v[2 * D + 2] = kB_ - cross;
-        v[2 * D + 3] = 0.0;
-        if (gA == 0) v[2 * D] = INFINITY;        // global step 0 accepts unconditionally (sp.py:253)
-#pragma unroll
-        for (int q = 0; q < NF2; ++q)
-          slot[q * ITEMS + k * WD_ITEMS] = make_double2(v[2 * q], v[2 * q + 1]);
+      for (int j = 0; j < D; ++j) {
+        v[j] = eA[j];
+        v[D + j] = eB[j];
+        v[2 * D + 4 + j] = dA_[j];
+        v[3 * D + 4 + j] = dB_[j];
       }
+      v[2 * D] = kA_;
+      v[2 * D + 1] = kB_;
+      v[2 * D + 2] = kB_ - cross;
+      v[2 * D + 3] = 0.0;
+      if (gA == 0) v[2 * D] = INFINITY;          // global step 0 accepts unconditionally (sp.py:253)
+#pragma unroll
+      for (int q = 0; q < NF2; ++q) slot[q * ITEMS] = make_double2(v[2 * q], v[2 * q + 1]);
       __syncwarp();
       if (lane == 0) pbx_mbar_arrive(&in_full[s]);
     }
@@ -969,18 +940,7 @@ __global__ void __launch_bounds__(WD_THREADS, 1)
     double x[D], y[D];
 #pragma unroll
     for (int j = 0; j < D; ++j) x[j] = valid ? a.state[j * C + c] : 0.0;
-    {
-      double dev[D];
-#pragma unroll
-      for (int j = 0; j < D; ++j) dev[j] = kZeroMean ? x[j] : x[j] - m.mean[j];
-#pragma unroll
-      for (int k = 0; k < D; ++k) {
-        double e = 0.0;
-#pragma unroll
-        for (int j = 0; j < D; ++j) e = fma(dev[j], m.W[j * D + k], e);
-        y[k] = e;
-      }
-    }
+    whiten<D, kZeroMean>(x, m, [&](int k, double e) { y[k] = e; });
     int nacc = 0;
     // (laundered through an opaque move so that the compiler keeps the base in a register
     // instead of rematerialising it -- S2UR SR_CgaCtaId and friends -- at every use)
@@ -1094,33 +1054,31 @@ __global__ void __launch_bounds__(WD_THREADS, 1)
       __syncwarp();
       if (lane == 0) pbx_mbar_arrive(&out_full[s]);
     }
-    if (valid) {
-#pragma unroll
-      for (int j = 0; j < D; ++j) a.state[j * C + c] = x[j];
-      a.state_lp[c] = -0.5 * (m.norm_c + mvn_maha<D, kZeroMean>(x, m));
-      if (a.accept_count) a.accept_count[c] += (int64_t)nacc;
-    }
+    // the running sums are the producers' (reduced below)
+    if (valid)
+      write_back(a, c, x, -0.5 * (m.norm_c + mvn_maha<D, kZeroMean>(x, m)), nacc, nullptr,
+                 nullptr);
   }
   // ---- running sums: fixed-order reduction of the per-item partials (deterministic) -------
   if (a.stat_sum == nullptr && a.stat_sumsq == nullptr) return;
   __syncthreads();                               // every slot is drained: reuse the ring
-  double* part = reinterpret_cast<double*>(ring2);           // [2 D][WD_ITEMS]
+  double* part = reinterpret_cast<double*>(ring2);           // [2 D][ITEMS]
   if (pi >= 0) {
 #pragma unroll
     for (int j = 0; j < D; ++j) {
-      part[(2 * j) * WD_ITEMS + item] = ssum[j];
-      part[(2 * j + 1) * WD_ITEMS + item] = ssq[j];
+      part[(2 * j) * ITEMS + item] = ssum[j];
+      part[(2 * j + 1) * ITEMS + item] = ssq[j];
     }
   }
   __syncthreads();
-  for (int t = threadIdx.x; t < cpc * D; t += WD_THREADS) {
+  for (int t = threadIdx.x; t < cpc * D; t += WdCfg<D>::THREADS) {
     const int j = t / cpc, ch = t - j * cpc;
     const int c = cbase + ch;
     if (c >= a.C) continue;
     double s1 = 0.0, s2 = 0.0;
-    for (int p = 0; p < P0; ++p) {
-      s1 += part[(2 * j) * WD_ITEMS + p * cpc + ch];
-      s2 += part[(2 * j + 1) * WD_ITEMS + p * cpc + ch];
+    for (int p = 0; p < P; ++p) {
+      s1 += part[(2 * j) * ITEMS + p * cpc + ch];
+      s2 += part[(2 * j + 1) * ITEMS + p * cpc + ch];
     }
     if (a.stat_sum) a.stat_sum[j * C + c] += s1;
     if (a.stat_sumsq) a.stat_sumsq[j * C + c] += s2;
@@ -1145,62 +1103,46 @@ static int wd_pick_cpc(int C, int sms) {
   return best;
 }
 
+// Raises the kernel's dynamic shared-memory limit to smem and launches it on the context's stream
+template <class... P, class... A>
+static int launch_smem(pbx_ctx* ctx, void (*kernel)(P...), int grid, int threads, size_t smem,
+                       const A&... args) {
+  PBX_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  kernel<<<grid, threads, smem, ctx->stream>>>(args...);
+  PBX_LAUNCH_CHECK(ctx);
+  return PBX_OK;
+}
+
 template <int D>
 static int launch_mh_mvn(pbx_ctx* ctx, const MhMvnArgs& a, const MhMvnConst& m, int kernel_variant) {
   const bool injected = a.inj_delta != nullptr;
   const bool per_step = a.out_accept != nullptr || a.out_score != nullptr ||
                         a.out_xprop != nullptr || a.out_pprop != nullptr;
   const bool use_ws = !injected && !per_step && kernel_variant != 1 && !m.bound;
-  const bool wd_ok = use_ws && D <= WD_MAXD && a.accept_mode == PBX_ACCEPT_LOG;
+  const bool wd_ok = use_ws && D <= kWdMaxD && a.accept_mode == PBX_ACCEPT_LOG;
   if (kernel_variant == 4 && !wd_ok) {
     pbx_set_error("pbx_mh_mvn_run: kernel_variant 4 (whitened-decision kernel) needs the native "
-                  "RNG, the log accept rule, no per-step outputs and n_dims <= %d", WD_MAXD);
+                  "RNG, the log accept rule, no per-step outputs and n_dims <= %d", kWdMaxD);
     return PBX_ERR_UNSUPPORTED;
   }
-  if constexpr (D <= WD_MAXD) {
+  const bool fast = a.prop_kind == PBX_PROP_NORMAL && !a.has_L;      // kFast
+  bool zero_mean = true;                                               // kZeroMean
+  for (int j = 0; j < D; ++j) zero_mean = zero_mean && m.mean[j] == 0.0;
+  if constexpr (D <= kWdMaxD) {
     if (wd_ok && kernel_variant != 2) {
       const int cpc = wd_pick_cpc(a.C, ctx->sm_count);
-      const int grid = (a.C + cpc - 1) / cpc;
-      const size_t smem = WdCfg<D>::SMEM;
-      const bool fast = a.prop_kind == PBX_PROP_NORMAL && !a.has_L;
-      bool zero_mean = true;
-      for (int j = 0; j < D; ++j) zero_mean = zero_mean && m.mean[j] == 0.0;
-#define PBX_WD_LAUNCH(F, Z)                                                                   \
-  do {                                                                                        \
-    PBX_CUDA(cudaFuncSetAttribute(mh_mvn_wd_kernel<D, F, Z>,                                  \
-                                  cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));   \
-    mh_mvn_wd_kernel<D, F, Z><<<grid, WD_THREADS, smem, ctx->stream>>>(a, m, cpc);          \
-  } while (0)
-      if (fast && zero_mean) PBX_WD_LAUNCH(true, true);
-      else if (fast) PBX_WD_LAUNCH(true, false);
-      else if (zero_mean) PBX_WD_LAUNCH(false, true);
-      else PBX_WD_LAUNCH(false, false);
-#undef PBX_WD_LAUNCH
-      PBX_LAUNCH_CHECK(ctx);
-      return PBX_OK;
+      auto* k = fast ? (zero_mean ? mh_mvn_wd_kernel<D, true, true> : mh_mvn_wd_kernel<D, true, false>)
+                     : (zero_mean ? mh_mvn_wd_kernel<D, false, true> : mh_mvn_wd_kernel<D, false, false>);
+      return launch_smem(ctx, k, (a.C + cpc - 1) / cpc, WdCfg<D>::THREADS, WdCfg<D>::SMEM, a, m, cpc);
     }
   }
   if (use_ws) {
-    const int grid = (a.C + 31) / 32;
-    const size_t smem = WsCfg<D>::SMEM;
-    const bool ref = a.accept_mode == PBX_ACCEPT_REFERENCE;
-    const bool fast = a.prop_kind == PBX_PROP_NORMAL && !a.has_L;
-#define PBX_WS_LAUNCH(R, F, Z)                                                                \
-  do {                                                                                        \
-    PBX_CUDA(cudaFuncSetAttribute(mh_mvn_ws_kernel<D, R, F, Z>,                               \
-                                  cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));   \
-    mh_mvn_ws_kernel<D, R, F, Z><<<grid, WsCfg<D>::THREADS, smem, ctx->stream>>>(a, m);     \
-  } while (0)
-    bool zero_mean = true;
-    for (int j = 0; j < D; ++j) zero_mean = zero_mean && m.mean[j] == 0.0;
-    if (ref && fast) PBX_WS_LAUNCH(true, true, false);
-    else if (ref) PBX_WS_LAUNCH(true, false, false);
-    else if (fast && zero_mean) PBX_WS_LAUNCH(false, true, true);
-    else if (fast) PBX_WS_LAUNCH(false, true, false);
-    else PBX_WS_LAUNCH(false, false, false);
-#undef PBX_WS_LAUNCH
-    PBX_LAUNCH_CHECK(ctx);
-    return PBX_OK;
+    auto* k = mh_mvn_ws_kernel<D, false, false, false>;
+    if (a.accept_mode == PBX_ACCEPT_REFERENCE)
+      k = fast ? mh_mvn_ws_kernel<D, true, true, false> : mh_mvn_ws_kernel<D, true, false, false>;
+    else if (fast)
+      k = zero_mean ? mh_mvn_ws_kernel<D, false, true, true> : mh_mvn_ws_kernel<D, false, true, false>;
+    return launch_smem(ctx, k, (a.C + 31) / 32, WsCfg<D>::THREADS, WsCfg<D>::SMEM, a, m);
   }
   const int warps = (a.C + 31) / 32;
   // few chains: one warp per CTA so the warps spread over all SMs
