@@ -52,6 +52,16 @@ int pbx_ws_reserve(pbx_ctx* ctx, size_t bytes);
     PBX_CUDA(cudaGetLastError());                                               \
   } while (0)
 
+// Raises the kernel's dynamic shared-memory limit to smem and launches it on the context's stream
+template <class... P, class... A>
+static int launch_smem(pbx_ctx* ctx, void (*kernel)(P...), int grid, int threads, size_t smem,
+                       const A&... args) {
+  PBX_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  kernel<<<grid, threads, smem, ctx->stream>>>(args...);
+  PBX_LAUNCH_CHECK(ctx);
+  return PBX_OK;
+}
+
 // centred sufficient statistics of (x, y) observations for the normal likelihoods
 // (pbx_mh_normreg.cu, "variant 3"); computed into the context workspace
 struct NrStats { double N, cx, cy, Sxx, b1s, RSS, Su, Se, Seu, pad; };

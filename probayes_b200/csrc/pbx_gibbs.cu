@@ -2,33 +2,41 @@
 // and the batched mvn density.
 //
 // Gibbs step (probayes/rf.py:446-462 -> rf_utils.py:50-65 -> cond_cov.py:42-65),
-// one coordinate i = step mod d per step (tsteps=1):
+// one coordinate i = step mod d per step (tsteps=1), with the truncation limits fixed at
+// construction (cond_cov.py:38-39):
 //     u   = cdf_lo_i + (cdf_hi_i - cdf_lo_i) * r          r ~ U(0,1)  (vtypes.py:186)
 //     x_i = ndtri(u) * stdv_i + mean_i + coef_i . (x_-i - mean_-i)
+// The dot product is evaluated as c0_i + coef_i . x with c0_i = mean_i - coef_i . mean
+// folded on the host (coef_ii = 0).  ndtri is the table-driven pbx_ndtri.cuh.
 // Native uniforms: global step g takes the 52-bit uniform of words (0, 1) (bit 2 of g clear)
 // or (2, 3) (bit 2 set) of Philox block (seed, g & ~4, chain, slot 0): steps g and g + 4 --
 // consecutive coordinates of the same lane below -- share one block (oracle/philox.py
-// gibbs_uniforms replays it).  ndtri is the table-driven pbx_ndtri.cuh.
-// with the truncation limits fixed at construction (cond_cov.py:38-39).  The dot
-// product is evaluated as c0_i + coef_i . x with c0_i = mean_i - coef_i . mean
-// folded on the host (coef_ii = 0).
+// gibbs_uniforms replays it).
 //
-// Kernel: four lanes = one chain, the state vector lives in REGISTERS (DP/4 doubles
-// per lane, coordinate loop fully unrolled), the coefficient rows come from shared
-// memory with 128-bit loads, the dot product finishes with two shuffle-adds.
+// Two Gibbs kernels, both with four lanes per chain and the state vector in REGISTERS (lane q
+// of a chain holds coordinates 4m + q):
+//   gibbs_mvn_kernel      any step range, one coordinate at a time: the coefficient rows come
+//                         from shared memory with 128-bit loads, the dot product finishes with
+//                         two shuffle-adds;
+//   gibbs_mvn_mma_kernel  whole sweeps, d >= 5: blocks of 8 coordinates in closed form on the
+//                         FP64 tensor cores; at d = 64 it also evaluates the density of every
+//                         recorded state.
 //
-// Density (probayes/prob.py:347-360 -> scipy multivariate_normal): maha = |(x -
-// mean) W|^2.  For d >= 64 the [chains, d] x [d, d] whitening product runs on the
-// FP64 tensor cores (mma.sync.m8n8k4.f64 -- tcgen05 has no FP64 kind), 8 chains per
-// MMA row block; smaller d uses a plain FMA kernel.
+// Density (probayes/prob.py:347-360 -> scipy multivariate_normal): maha = |(x - mean) W|^2.
+// At d = 64 the [chains, d] x [d, d] whitening product runs on the FP64 tensor cores
+// (mma.sync.m8n8k4.f64 -- tcgen05 has no FP64 kind), 8 chains per MMA row block, with the same
+// code as the fused density; other d use a plain FMA kernel.
 #include <math.h>
 #include <vector>
 #include "pbx_common.cuh"
 #include "pbx_ndtri.cuh"
 
-#ifndef GB_THREADS
-#define GB_THREADS 256                 // measured: 0.137 / 0.116 / 0.108 ms per sweep at 64 / 128 / 256
-#endif
+// threads per CTA of both Gibbs kernels when there are enough chains (gibbs_launch); measured
+// on gibbs_mvn_kernel: 0.137 / 0.116 / 0.108 ms per sweep at 64 / 128 / 256
+constexpr int kGbThreads = 256;
+// minimum resident CTAs of 256 threads per SM for the tensor-core kernel at d <= 64 (124
+// registers); capping at 80 registers for 3 CTAs was measured slower
+constexpr int kGmMinBlocks = 2;
 
 struct GibbsArgs {
   int C, d, T, thin;
@@ -94,6 +102,61 @@ __device__ __forceinline__ double gibbs_uniform(const pbx_u4& b, int64_t gk) {
   return (gk & 4) ? pbx_u52(b.z, b.w) : pbx_u52(b.x, b.y);
 }
 
+__device__ __forceinline__ void dmma_m8n8k4(double& d0, double& d1, double a, double b) {
+  asm("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0, %1}, {%2}, {%3}, {%0, %1};"
+               : "+d"(d0), "+d"(d1)
+               : "d"(a), "d"(b));
+}
+
+// ---------------------------------------------------------------------------
+// the d = 64 density on the FP64 tensor cores: the fused density of gibbs_mvn_mma_kernel and
+// mvn_logpdf_mma64_kernel.  One warp = 8 points.  D[8 x 8] += A[8 x 4] * B[4 x 8] with
+//   A[r][k] = x[k] - mean[k] of point r   (lane T: r = T/4, k = 4 ks + T%4)
+//   B[k][n] = W[k][n]                     (lane T: k = 4 ks + T%4, n = 8 nb + T/4)
+//   D[r][n]: lane T holds (r = T/4, n = 8 nb + 2*(T%4) + {0,1})
+// ---------------------------------------------------------------------------
+// row stride of W in shared memory: 68 doubles = 4 mod 16 double-banks, so the B-fragment
+// loads are bank-conflict free per half-warp
+constexpr int kWStride = 68;
+
+__device__ __forceinline__ void stage_whiten64(double* s_W, double* s_m, const double* W,
+                                               const double* mean, int nthreads) {
+  for (int i = threadIdx.x; i < 64 * 64; i += nthreads) s_W[(i >> 6) * kWStride + (i & 63)] = W[i];
+  for (int i = threadIdx.x; i < 64; i += nthreads) s_m[i] = mean[i];
+}
+
+// |(x - mean) W|^2 of the 8 points of a warp, x[ks] = coordinate 4 ks + lane % 4 of point
+// lane / 4; the sum is returned in all four lanes of the point
+__device__ __forceinline__ double dmma_maha64(const double (&x)[16], const double* s_W,
+                                              const double* s_m, int lane) {
+  const int r = lane >> 2, q = lane & 3;
+  double av[16];
+#pragma unroll
+  for (int ks = 0; ks < 16; ++ks) av[ks] = x[ks] - s_m[4 * ks + q];
+  double maha = 0.0;
+#pragma unroll
+  for (int nb = 0; nb < 8; ++nb) {
+    double d0 = 0.0, d1 = 0.0;
+#pragma unroll
+    for (int ks = 0; ks < 16; ++ks)
+      dmma_m8n8k4(d0, d1, av[ks], s_W[(4 * ks + q) * kWStride + nb * 8 + r]);
+    maha = fma(d0, d0, maha);
+    maha = fma(d1, d1, maha);
+  }
+  maha += __shfl_xor_sync(0xffffffffu, maha, 1);
+  maha += __shfl_xor_sync(0xffffffffu, maha, 2);
+  return maha;
+}
+
+// the recorded density in log or linear pscale
+__device__ __forceinline__ double mvn_density(double norm_c, double maha, int log_pscale) {
+  const double lp = -0.5 * (norm_c + maha);
+  return log_pscale ? lp : exp(lp);
+}
+
+// ---------------------------------------------------------------------------
+// Per-coordinate Gibbs (any step range).
+//
 // One chain = FOUR lanes (a warp = 8 chains): lane q of a chain keeps coordinates
 // j = 4m + q in registers (DQ = DP/4 doubles instead of DP, so the kernel fits ~64
 // registers instead of 255 + local-memory spills), the dot product coef_i . x is DQ
@@ -102,11 +165,9 @@ __device__ __forceinline__ double gibbs_uniform(const pbx_u4& b, int64_t gk) {
 // next coordinate, i.e. four coordinates' worth in parallel with no redundancy.
 // kSweepRec: records fall on sweep boundaries only (thin % d == 0, call aligned to
 // sweeps) -> one copy of the record code per sweep instead of one per coordinate.
-// kPair (whole sweeps and d % 8 == 0): the Philox block of coordinate 4 l + q also serves
-// 4 (l + 1) + q, so it is computed on even l only.
-// NT threads per CTA (256, or 128 when there are too few chains to give every SM a CTA of
-// 64 chains: strong-scaled shards)
-template <int DQ, bool kSweepRec, bool kPair, int NT = GB_THREADS>
+// NT threads per CTA (kGbThreads, or 128 when there are too few chains to give every SM a CTA
+// of 64 chains: strong-scaled shards)
+template <int DQ, bool kSweepRec, int NT>
 __global__ void __launch_bounds__(NT)
     gibbs_mvn_kernel(const GibbsArgs a) {
   constexpr int DP = 4 * DQ;
@@ -181,8 +242,7 @@ __global__ void __launch_bounds__(NT)
           if (a.inj_runif) {
             r = a.inj_runif[(gk - k_begin) * C + c];
           } else {
-            if (!kPair || (l & 1) == 0)
-              blk = pbx_block(a.seed, (uint64_t)gk & ~(uint64_t)4, gchain, 0u);
+            blk = pbx_block(a.seed, (uint64_t)gk & ~(uint64_t)4, gchain, 0u);
             r = gibbs_uniform(blk, gk);
           }
           z = gibbs_ndtri(s_lo[i] + s_w[i] * r) * s_sd[i] + s_c0[i];
@@ -262,12 +322,6 @@ __global__ void __launch_bounds__(NT)
 // Draws: lane (r, q) draws for its own two coordinates of the block from ONE Philox block
 // (steps g and g + 4), table ndtri from shared memory, one block ahead of the MMAs.
 // ---------------------------------------------------------------------------
-__device__ __forceinline__ void dmma_m8n8k4(double& d0, double& d1, double a, double b) {
-  asm("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0, %1}, {%2}, {%3}, {%0, %1};"
-               : "+d"(d0), "+d"(d1)
-               : "d"(a), "d"(b));
-}
-
 // the model in the kernel's shared-memory layout:
 //   [NB][DQ][32] B'_b fragments | [NB][2][32] M_b fragments | c0, sd, lo, w [DP] each
 template <int DQ>
@@ -324,17 +378,15 @@ __global__ void __launch_bounds__(256) gibbs_mma_prep_kernel(const GibbsArgs a,
   }
 }
 
-#ifndef GM_MINB
-#define GM_MINB 2
-#endif
+// kPair (d % 8 == 0): the two draws of a lane in a block, steps g and g + 4 with bit 2 of g
+// clear, come from one Philox block.
 // kDens (d = 64): the target density of every recorded state -- |(x - mean) W|^2 on the tensor
 // cores, straight from the state registers (they are the A fragment of that product too) --
 // instead of a second kernel re-reading the recorded states
-#define GM_WDS 68                          // row stride of the whitening matrix in shared memory
 template <int DQ, bool kPair, int NT, bool kDens = false>
-__global__ void __launch_bounds__(NT, (DQ <= 16 ? (NT <= 128 ? 2 * GM_MINB : GM_MINB) : 1))
+__global__ void __launch_bounds__(NT, (DQ <= 16 ? (NT <= 128 ? 2 * kGmMinBlocks : kGmMinBlocks) : 1))
     gibbs_mvn_mma_kernel(const GibbsArgs a, const double* __restrict__ img) {
-  static_assert(!kDens || DQ == 16, "the fused density is the d = 64 case");
+  static_assert(!kDens || (DQ == 16 && kPair), "the fused density is the d = 64 case, a kPair one");
   constexpr int DP = 4 * DQ, NB = DQ / 2;
   extern __shared__ __align__(16) double sm[];
   double* s_B = sm;                          // [NB][DQ][32]   B'_b fragments
@@ -353,12 +405,9 @@ __global__ void __launch_bounds__(NT, (DQ <= 16 ? (NT <= 128 ? 2 * GM_MINB : GM_
     double2* hdst = reinterpret_cast<double2*>(s_nd);
     for (int i = threadIdx.x; i < NDT_NCOEF * NDT_HOT_ROWS / 2; i += NT) hdst[i] = hsrc[i];
   }
-  double* s_Wd = s_nd + NDT_NCOEF * NDT_HOT_ROWS;   // [64][GM_WDS]  whitening matrix (kDens)
-  double* s_md = s_Wd + 64 * GM_WDS;                // [64]          density mean
-  if (kDens) {
-    for (int i = threadIdx.x; i < 64 * 64; i += NT) s_Wd[(i >> 6) * GM_WDS + (i & 63)] = a.whiten[i];
-    for (int i = threadIdx.x; i < 64; i += NT) s_md[i] = a.dens_mean[i];
-  }
+  double* s_Wd = s_nd + NDT_NCOEF * NDT_HOT_ROWS;   // [64][kWStride]  whitening matrix (kDens)
+  double* s_md = s_Wd + 64 * kWStride;              // [64]            density mean
+  if (kDens) stage_whiten64(s_Wd, s_md, a.whiten, a.dens_mean, NT);
   __syncthreads();
   const int d = a.d;
   const int lane = threadIdx.x & 31, q = lane & 3;
@@ -476,28 +525,9 @@ __global__ void __launch_bounds__(NT, (DQ <= 16 ? (NT <= 128 ? 2 * GM_MINB : GM_
           }
         }
       }
-      if (kDens) {
-        // same fragments and accumulation order as mvn_logpdf_mma64_kernel: bit-identical
-        const int r8 = lane >> 2;
-        double av[DQ];
-#pragma unroll
-        for (int ks = 0; ks < DQ; ++ks) av[ks] = x[ks] - s_md[4 * ks + q];
-        double maha = 0.0;
-#pragma unroll
-        for (int nb = 0; nb < 8; ++nb) {
-          double d0 = 0.0, d1 = 0.0;
-#pragma unroll
-          for (int ks = 0; ks < DQ; ++ks)
-            dmma_m8n8k4(d0, d1, av[ks], s_Wd[(4 * ks + q) * GM_WDS + nb * 8 + r8]);
-          maha = fma(d0, d0, maha);
-          maha = fma(d1, d1, maha);
-        }
-        maha += __shfl_xor_sync(0xffffffffu, maha, 1);
-        maha += __shfl_xor_sync(0xffffffffu, maha, 2);
-        if (q == 0 && valid) {
-          const double lp = -0.5 * (a.norm_c + maha);
-          a.out_prob[rec * C + c] = a.log_pscale ? lp : exp(lp);
-        }
+      if constexpr (kDens) {
+        const double maha = dmma_maha64(x, s_Wd, s_md, lane);
+        if (q == 0 && valid) a.out_prob[rec * C + c] = mvn_density(a.norm_c, maha, a.log_pscale);
       }
       ++rec;
     }
@@ -535,28 +565,17 @@ __global__ void __launch_bounds__(128)
     for (int j = 0; j < d; ++j) y = fma(xb[(int64_t)j * C] - s_m[j], s_W[j * d + k], y);
     maha = fma(y, y, maha);
   }
-  const double lp = -0.5 * (norm_c + maha);
-  out[p] = log_pscale ? lp : exp(lp);
+  out[p] = mvn_density(norm_c, maha, log_pscale);
 }
 
-// ---------------------------------------------------------------------------
-// batched mvn density on the FP64 tensor cores, d = 64.
-// One warp = 8 points per pass.  D[8 x 8] += A[8 x 4] * B[4 x 8] with
-//   A[r][k] = x[k][c0 + r] - mean[k]   (thread T: r = T/4, k = T%4)
-//   B[k][n] = W[k][n]                  (thread T: k = T%4, n = T/4)
-//   D[r][n]: thread T holds (r = T/4, n = 2*(T%4) + {0,1})
-// ---------------------------------------------------------------------------
+// batched mvn density on the FP64 tensor cores, d = 64: one warp per 8-point row block
 __global__ void __launch_bounds__(128)
     mvn_logpdf_mma64_kernel(const double* __restrict__ x, int64_t C, int64_t R,
                             const double* __restrict__ mean, const double* __restrict__ W,
                             double norm_c, int log_pscale, double* __restrict__ out) {
-  constexpr int D = 64;
-  // W in shared memory, row stride 68 doubles (= 4 mod 16 double-banks): the B
-  // fragment load (k = 4ks + q, n = 8nb + r) is bank-conflict free per half-warp
-  __shared__ double s_W[D][D + 4];
-  __shared__ double s_m[D];
-  for (int i = threadIdx.x; i < D * D; i += blockDim.x) s_W[i / D][i % D] = W[i];
-  for (int i = threadIdx.x; i < D; i += blockDim.x) s_m[i] = mean[i];
+  __shared__ double s_W[64 * kWStride];
+  __shared__ double s_m[64];
+  stage_whiten64(s_W, s_m, W, mean, blockDim.x);
   __syncthreads();
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int r = lane >> 2, q = lane & 3;
@@ -565,30 +584,13 @@ __global__ void __launch_bounds__(128)
     const int64_t rr = blk / bpr;
     const int64_t c = (blk % bpr) * 8 + r;
     const bool valid = c < C;
-    const double* xb = x + rr * D * C;
-    // this thread's A elements for the 16 k-steps: k = 4*ks + q
-    double av[16];
+    const double* xb = x + rr * 64 * C;
+    // this lane's A elements for the 16 k-steps: k = 4*ks + q (rows past C: any finite value)
+    double xv[16];
 #pragma unroll
-    for (int ks = 0; ks < 16; ++ks) {
-      const int k = 4 * ks + q;
-      av[ks] = valid ? xb[(int64_t)k * C + c] - s_m[k] : 0.0;
-    }
-    double maha = 0.0;
-#pragma unroll
-    for (int nb = 0; nb < 8; ++nb) {
-      double d0 = 0.0, d1 = 0.0;
-#pragma unroll
-      for (int ks = 0; ks < 16; ++ks) dmma_m8n8k4(d0, d1, av[ks], s_W[4 * ks + q][nb * 8 + r]);
-      maha = fma(d0, d0, maha);
-      maha = fma(d1, d1, maha);
-    }
-    // sum the 4 threads of a row (they hold different output columns)
-    maha += __shfl_xor_sync(0xffffffffu, maha, 1);
-    maha += __shfl_xor_sync(0xffffffffu, maha, 2);
-    if (q == 0 && valid) {
-      const double lp = -0.5 * (norm_c + maha);
-      out[rr * C + c] = log_pscale ? lp : exp(lp);
-    }
+    for (int ks = 0; ks < 16; ++ks) xv[ks] = valid ? xb[(int64_t)(4 * ks + q) * C + c] : 0.0;
+    const double maha = dmma_maha64(xv, s_W, s_m, lane);
+    if (q == 0 && valid) out[rr * C + c] = mvn_density(norm_c, maha, log_pscale);
   }
 }
 
@@ -666,73 +668,42 @@ static int gibbs_init_ndtab(pbx_ctx* ctx) {
   return PBX_OK;
 }
 
+// whole: the call is whole sweeps (step0, T and thin multiples of d); dens: the density of the
+// recorded states is fused into the tensor-core kernel (whole sweeps at d = 64)
 template <int DQ, int NT>
-static int gibbs_launch_nt(pbx_ctx* ctx, const GibbsArgs& a) {
+static int gibbs_launch_nt(pbx_ctx* ctx, const GibbsArgs& a, double* img, bool whole, bool dens) {
   constexpr int DP = 4 * DQ;
   const int chains_per_cta = (NT / 32) * 8;
   const int grid = (a.C + chains_per_cta - 1) / chains_per_cta;
-  const bool sweep_rec = (a.thin % a.d == 0) && (a.step0 % a.d == 0) && (a.T % a.d == 0);
   if constexpr (DQ >= 2) {
-    if (sweep_rec) {                       // whole sweeps: conditional means on the tensor cores
-      const size_t model = gibbs_mma_model_doubles<DQ>();
-      const bool dens = DQ == 16 && a.d == 64 && a.out_prob != nullptr;
-      const size_t smem = (model + NDT_NCOEF * NDT_HOT_ROWS + (dens ? 64 * GM_WDS + 64 : 0)) *
-                          sizeof(double);
-      // workspace: [c0 (d doubles, padded to 256 B)] [model image]
-      const size_t off = ((size_t)a.d * 8 + 255) / 256 * 256;
-      int rc = pbx_ws_reserve(ctx, off + model * sizeof(double));
-      if (rc) return rc;
-      GibbsArgs a2 = a;
-      a2.c0 = (const double*)ctx->ws;                   // (the reserve above may have moved it)
-      double* img = (double*)((char*)ctx->ws + off);
-      gibbs_mma_prep_kernel<DQ><<<DQ / 2, 256, 0, ctx->stream>>>(a2, img);
+    if (whole) {                           // whole sweeps: conditional means on the tensor cores
+      const size_t smem = (gibbs_mma_model_doubles<DQ>() + NDT_NCOEF * NDT_HOT_ROWS +
+                           (dens ? 64 * kWStride + 64 : 0)) * sizeof(double);
+      gibbs_mma_prep_kernel<DQ><<<DQ / 2, 256, 0, ctx->stream>>>(a, img);
       PBX_LAUNCH_CHECK(ctx);
-#define GM_LAUNCH(PR, DN)                                                                      \
-  do {                                                                                         \
-    PBX_CUDA(cudaFuncSetAttribute(gibbs_mvn_mma_kernel<DQ, PR, NT, DN>,                        \
-                                  cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));    \
-    gibbs_mvn_mma_kernel<DQ, PR, NT, DN><<<grid, NT, smem, ctx->stream>>>(a2, img);            \
-  } while (0)
-      if constexpr (DQ == 16) {
-        if (dens) {
-          if (a.d % 8 == 0) GM_LAUNCH(true, true);
-          else GM_LAUNCH(false, true);
-          PBX_LAUNCH_CHECK(ctx);
-          return PBX_OK;
-        }
-      }
-      if (a.d % 8 == 0) GM_LAUNCH(true, false);
-      else GM_LAUNCH(false, false);
-#undef GM_LAUNCH
-      PBX_LAUNCH_CHECK(ctx);
-      return PBX_OK;
+      if constexpr (DQ == 16)
+        if (dens) return launch_smem(ctx, gibbs_mvn_mma_kernel<DQ, true, NT, true>, grid, NT, smem, a, img);
+      auto* k = a.d % 8 == 0 ? gibbs_mvn_mma_kernel<DQ, true, NT> : gibbs_mvn_mma_kernel<DQ, false, NT>;
+      return launch_smem(ctx, k, grid, NT, smem, a, img);
     }
   }
-  const size_t smem = ((size_t)DP * 4 * (DQ + 2) + 4 * DP) * sizeof(double);
-#define GB_LAUNCH(SR)                                                                          \
-  do {                                                                                         \
-    PBX_CUDA(cudaFuncSetAttribute(gibbs_mvn_kernel<DQ, SR, false, NT>,                         \
-                                  cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));    \
-    gibbs_mvn_kernel<DQ, SR, false, NT><<<grid, NT, smem, ctx->stream>>>(a);                   \
-  } while (0)
-  if constexpr (DQ == 1) {
-    if (sweep_rec) GB_LAUNCH(true);
-    else GB_LAUNCH(false);
-  } else {
-    GB_LAUNCH(false);
-  }
-#undef GB_LAUNCH
-  PBX_LAUNCH_CHECK(ctx);
-  return PBX_OK;
+  auto* k = gibbs_mvn_kernel<DQ, false, NT>;
+  if constexpr (DQ == 1)
+    if (whole) k = gibbs_mvn_kernel<DQ, true, NT>;
+  return launch_smem(ctx, k, grid, NT, ((size_t)DP * 4 * (DQ + 2) + 4 * DP) * sizeof(double), a);
 }
 
 template <int DQ>
-static int gibbs_launch(pbx_ctx* ctx, const GibbsArgs& a) {
+static int gibbs_launch(pbx_ctx* ctx, const GibbsArgs& a, double* img, bool whole, bool dens) {
   // fewer than ~3 CTAs of 64 chains per SM: halve the CTA so that the grid covers the chip
   // (a strong-scaled shard of 8192 chains is 128 CTAs of 64 on 148 SMs)
-  if ((int64_t)a.C < (int64_t)ctx->sm_count * 64 * 3) return gibbs_launch_nt<DQ, 128>(ctx, a);
-  return gibbs_launch_nt<DQ, GB_THREADS>(ctx, a);
+  if ((int64_t)a.C < (int64_t)ctx->sm_count * 64 * 3)
+    return gibbs_launch_nt<DQ, 128>(ctx, a, img, whole, dens);
+  return gibbs_launch_nt<DQ, kGbThreads>(ctx, a, img, whole, dens);
 }
+
+// workspace: c0 [d <= 128] at 0, the tensor-core kernel's model image at this offset
+constexpr size_t kGibbsImageOffset = 128 * sizeof(double);
 
 extern "C" int pbx_gibbs_mvn_run(pbx_ctx* ctx, const pbx_gibbs_mvn_params* p) {
   PBX_REQUIRE(ctx != nullptr && p != nullptr, "pbx_gibbs_mvn_run: null argument");
@@ -748,11 +719,10 @@ extern "C" int pbx_gibbs_mvn_run(pbx_ctx* ctx, const pbx_gibbs_mvn_params* p) {
   const int d = p->n_dims;
   int rc = gibbs_init_ndtab(ctx);
   if (rc) return rc;
-  // c0 [d] + the tensor-core kernel's model image (largest: d = 128), reserved in one go so
-  // that the launcher's own reserve never moves the workspace under the c0 kernel
-  rc = pbx_ws_reserve(ctx, 4096 + gibbs_mma_model_doubles<32>() * sizeof(double));
+  rc = pbx_ws_reserve(ctx, kGibbsImageOffset + gibbs_mma_model_doubles<32>() * sizeof(double));
   if (rc) return rc;
   double* c0 = (double*)ctx->ws;
+  double* img = (double*)((char*)ctx->ws + kGibbsImageOffset);
   GibbsArgs a;
   a.C = p->n_chains; a.d = d; a.T = p->n_steps; a.thin = p->thin;
   a.step0 = p->step0; a.chain0 = p->chain0; a.seed = p->seed;
@@ -761,9 +731,9 @@ extern "C" int pbx_gibbs_mvn_run(pbx_ctx* ctx, const pbx_gibbs_mvn_params* p) {
   a.stat_sum = p->stat_sum; a.stat_sumsq = p->stat_sumsq;
   // whole sweeps at d = 64: the density of the recorded states is evaluated inside the Gibbs
   // kernel; otherwise by a second launch over the recorded states (below)
+  const bool whole = (p->thin % d == 0) && (p->step0 % d == 0) && (p->n_steps % d == 0);
   const bool want_dens = p->out_prob && p->want_prob;
-  const bool fused_dens = want_dens && d == 64 && (p->thin % d == 0) && (p->step0 % d == 0) &&
-                          (p->n_steps % d == 0);
+  const bool fused_dens = want_dens && d == 64 && whole;
   a.out_prob = fused_dens ? p->out_prob : nullptr;
   a.whiten = p->whiten;
   a.dens_mean = p->dens_mean ? p->dens_mean : p->mean;
@@ -773,18 +743,17 @@ extern "C" int pbx_gibbs_mvn_run(pbx_ctx* ctx, const pbx_gibbs_mvn_params* p) {
   if (a.T > 0) {
     gibbs_c0_kernel<<<1, 128, 0, ctx->stream>>>(p->coef, p->mean, d, c0);
     PBX_LAUNCH_CHECK(ctx);
-    if (d <= 4) rc = gibbs_launch<1>(ctx, a);
-    else if (d <= 8) rc = gibbs_launch<2>(ctx, a);
-    else if (d <= 16) rc = gibbs_launch<4>(ctx, a);
-    else if (d <= 32) rc = gibbs_launch<8>(ctx, a);
-    else if (d <= 64) rc = gibbs_launch<16>(ctx, a);
-    else rc = gibbs_launch<32>(ctx, a);
+    if (d <= 4) rc = gibbs_launch<1>(ctx, a, img, whole, fused_dens);
+    else if (d <= 8) rc = gibbs_launch<2>(ctx, a, img, whole, fused_dens);
+    else if (d <= 16) rc = gibbs_launch<4>(ctx, a, img, whole, fused_dens);
+    else if (d <= 32) rc = gibbs_launch<8>(ctx, a, img, whole, fused_dens);
+    else if (d <= 64) rc = gibbs_launch<16>(ctx, a, img, whole, fused_dens);
+    else rc = gibbs_launch<32>(ctx, a, img, whole, fused_dens);
     if (rc) return rc;
     if (want_dens && !fused_dens) {
       // the target is evaluated and recorded on every kept step (sd.py:286)
-      rc = mvn_logpdf_launch(ctx, p->out_x, d, p->n_chains, p->n_steps / p->thin,
-                             p->dens_mean ? p->dens_mean : p->mean, p->whiten, p->norm_c,
-                             p->log_pscale, p->out_prob);
+      rc = mvn_logpdf_launch(ctx, p->out_x, d, p->n_chains, p->n_steps / p->thin, a.dens_mean,
+                             p->whiten, p->norm_c, p->log_pscale, p->out_prob);
       if (rc) return rc;
     }
   }

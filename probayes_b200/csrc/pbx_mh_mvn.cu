@@ -1103,16 +1103,6 @@ static int wd_pick_cpc(int C, int sms) {
   return best;
 }
 
-// Raises the kernel's dynamic shared-memory limit to smem and launches it on the context's stream
-template <class... P, class... A>
-static int launch_smem(pbx_ctx* ctx, void (*kernel)(P...), int grid, int threads, size_t smem,
-                       const A&... args) {
-  PBX_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  kernel<<<grid, threads, smem, ctx->stream>>>(args...);
-  PBX_LAUNCH_CHECK(ctx);
-  return PBX_OK;
-}
-
 template <int D>
 static int launch_mh_mvn(pbx_ctx* ctx, const MhMvnArgs& a, const MhMvnConst& m, int kernel_variant) {
   const bool injected = a.inj_delta != nullptr;

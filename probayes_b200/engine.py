@@ -566,8 +566,6 @@ class Engine:
         if stats:
             out["stat_sum"] = self.zeros(d, C_)
             out["stat_sumsq"] = self.zeros(d, C_)
-        if inj_runif is not None and tuple(inj_runif.shape) != (T, C_):
-            raise ValueError("injected uniforms must be [T, C]")
         p.state = state.data_ptr()
         p.inj_runif = 0 if inj_runif is None else inj_runif.data_ptr()
         p.out_x = out["x"].data_ptr() if record else 0

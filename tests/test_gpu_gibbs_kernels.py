@@ -1,11 +1,13 @@
 """K5 Gibbs, one compiled kernel at a time, against the numpy oracle.
 
-``pbx_gibbs_mvn_run`` picks one of 38 instantiations (36 reachable) of
-``gibbs_mvn_kernel<DQ, kSweepRec, false, NT>`` and ``gibbs_mvn_mma_kernel<DQ, kPair, NT, kDens>``
-from the dimension, the step alignment, the chain count and whether densities are recorded.
-``_instantiation`` restates that choice; the parity cases below run every reachable
-instantiation with injected uniforms, a model with real truncation limits in every draw regime
-of the table ndtri, and the native Philox stream at nonzero ``step0`` / ``chain0``."""
+``pbx_gibbs_mvn_run`` picks one of 36 instantiations of ``gibbs_mvn_kernel<DQ, kSweepRec, NT>``
+and ``gibbs_mvn_mma_kernel<DQ, kPair, NT, kDens>`` from the dimension, the step alignment, the
+chain count and whether densities are recorded.  ``_instantiation`` restates that choice, and a
+profiler test checks that each case launches the kernel it names; the parity cases below run
+every instantiation with injected uniforms, a model with real truncation limits in every draw
+regime of the table ndtri, and the native Philox stream at nonzero ``step0`` / ``chain0``."""
+import re
+
 import numpy as np
 import pytest
 from conftest import relerr
@@ -50,11 +52,17 @@ def _instantiation(d, C, T, thin, step0, want_prob, sm_count):
 
 COMPILED = {(GB, dq, sr, nt, False) for dq in (1, 2, 4, 8, 16, 32)
             for sr in ((False, True) if dq == 1 else (False,)) for nt in (128, 256)} | \
-           {(GM, dq, kp, nt, kd) for dq in (2, 4, 8, 16, 32) for kp in (False, True)
-            for nt in (128, 256) for kd in ((False, True) if dq == 16 else (False,))}
-# kDens without kPair needs d = 64 with d % 8 != 0
-UNREACHABLE = {(GM, 16, False, nt, True) for nt in (128, 256)}
-REACHABLE = COMPILED - UNREACHABLE
+           {(GM, dq, kp, nt, False) for dq in (2, 4, 8, 16, 32) for kp in (False, True)
+            for nt in (128, 256)} | \
+           {(GM, 16, True, nt, True) for nt in (128, 256)}     # fused density: d = 64, so kPair
+
+
+def _name(inst):
+    """The demangled template-id of an instantiation, e.g. gibbs_mvn_mma_kernel<16, true, 256, true>."""
+    kernel, dq, flag, nt, dens = inst
+    args = [dq, flag, nt] + ([dens] if kernel == GM else [])
+    return "%s<%s>" % (kernel, ", ".join(str(a).lower() if isinstance(a, bool) else str(a)
+                                         for a in args))
 
 
 def _chains(size, sm_count):
@@ -83,7 +91,7 @@ def _sample(C, width, n=96, seed=0):
 def test_dispatch_mirror_rules():
     sm = 148
     big = 3 * 64 * sm
-    assert len(COMPILED) == 38 and len(REACHABLE) == 36
+    assert len(COMPILED) == 36
     cases = [
         ((3, 10, 9, 3, 0, True), (GB, 1, True, 128, False)),
         ((3, 10, 9, 3, 1, True), (GB, 1, False, 128, False)),
@@ -108,15 +116,14 @@ def test_dispatch_mirror_rules():
     ]
     for args, want in cases:
         assert _instantiation(*args, sm_count=sm) == want, args
-    # exhaustively: every compiled kernel but the two kDens && !kPair ones is reached
+    # exhaustively: every compiled kernel is reached, and nothing else
     seen = set()
     for d in range(1, 129):
         for C in (1, big - 1, big):
             for T, thin, step0 in ((d, d, 0), (2 * d, d, d), (d + 1, 1, 0), (d, 1, 1), (d, d, 3)):
                 for wp in (False, True):
                     seen.add(_instantiation(d, C, T, thin, step0, wp, sm_count=sm))
-    assert seen == REACHABLE
-    assert not seen & UNREACHABLE
+    assert seen == COMPILED
 
 
 # ---------------------------------------------------------------------------------------------
@@ -252,7 +259,7 @@ def test_case_list_reaches_every_instantiation():
     sm = engine().info.sm_count
     got = {_instantiation(d, _chains(size, sm), T, thin, step0, wp, sm)
            for size in SIZES for d, T, thin, step0, wp in INJ_CASES}
-    assert got == REACHABLE, sorted(REACHABLE - got)
+    assert got == COMPILED, sorted(COMPILED - got)
 
 
 @pytest.mark.gpu
@@ -280,6 +287,70 @@ def test_injected_every_instantiation(d, T, thin, step0, want_prob, size):
                             inj_runif=Rd)
     eng.sync()
     _check(out, state, ref, thin, sel, want_prob, cov, mean, lin)
+
+
+@pytest.mark.gpu
+def test_each_case_launches_its_instantiation():
+    """Under torch.profiler, the cases launch, in order, the kernels _instantiation names."""
+    import torch
+    from torch.profiler import profile, ProfilerActivity
+    from probayes_b200.cond_cov import CondCov
+    eng = engine()
+    sm = eng.info.sm_count
+    runs = []
+    for size in SIZES:
+        C = _chains(size, sm)
+        for d, T, thin, step0, want_prob in INJ_CASES:
+            mean, cov, rng = _model(d, 7 * d)
+            cc = CondCov(mean, cov, np.tile([-10., 10.], (d, 1)))
+            runs.append((cc, dev(eng, (mean + rng.standard_normal((C, d))).T), T, thin, step0,
+                         want_prob, _instantiation(d, C, T, thin, step0, want_prob, sm)))
+    eng.sync()
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        probe = torch.ones(1024, device=eng.device, dtype=torch.float64) * 3.0
+        for cc, state, T, thin, step0, want_prob, _ in runs:
+            eng.gibbs_mvn(state, cc, T, thin=thin, step0=step0, seed=3, want_prob=want_prob)
+        eng.sync()
+        torch.cuda.synchronize()
+    del probe
+    kern = [e for e in prof.events() if e.device_type == torch.autograd.DeviceType.CUDA]
+    if not kern:
+        pytest.skip("the profiler recorded no device events, not even the probe's torch kernel")
+    kern.sort(key=lambda e: e.time_range.start)
+    names = []
+    for e in kern:
+        m = re.search(r"(gibbs_mvn(?:_mma)?_kernel<[^>]*>)", e.name)
+        if m:
+            names.append(re.sub(r"\s+", " ", m.group(1)))
+    assert names == [_name(r[-1]) for r in runs]
+    assert len(set(names)) == 36
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("log_pscale", [True, False])
+@pytest.mark.parametrize("size", SIZES)
+def test_fused_density_equals_mvn_logpdf(size, log_pscale):
+    """The density the d = 64 whole-sweep kernel evaluates at record time is bit-equal to
+    Engine.mvn_logpdf (the stand-alone tensor-core density kernel) of each recorded state."""
+    from probayes_b200.cond_cov import CondCov
+    eng = engine()
+    sm = eng.info.sm_count
+    C = _chains(size, sm)
+    d, T, thin, step0 = 64, 192, 64, 64
+    assert _instantiation(d, C, T, thin, step0, True, sm) == (GM, 16, True, _nt(C, sm), True)
+    mean, cov, rng = _model(d, 64)
+    cc = CondCov(mean, cov, np.tile([-10., 10.], (d, 1)))
+    out = eng.gibbs_mvn(dev(eng, (mean + rng.standard_normal((C, d))).T), cc, T, thin=thin,
+                        step0=step0, seed=11, log_pscale=log_pscale)
+    want = [eng.mvn_logpdf(out["x"][r], cc.mean, cc.cov, log_pscale=log_pscale)
+            for r in range(T // thin)]
+    eng.sync()
+    got = host(out["prob"])
+    assert np.isfinite(got).all()
+    if not log_pscale:
+        assert (got > 0.0).all()
+    for r in range(T // thin):
+        assert np.array_equal(got[r], host(want[r])), r
 
 
 # Band model runs: (d, T, thin, step0, want_prob) for the per-coordinate kernel and the
