@@ -170,7 +170,8 @@ PBX_API int pbx_mh_mvn_walk_host(pbx_ctx* ctx, const pbx_mh_mvn_params* p, int32
  * (probayes/rf.py:541-581, pd.py:332-370, sd.py:148-161) with scipy.stats.norm
  * .logpdf as the likelihood (examples/mcmc/metrohast_norm1d.py:30-31,
  * gibbs_linreg.py:35-36), box-uniform priors in ufun space (rv.py:153-166,
- * rv_utils.py:8-47) and ufun-space proposals (variable.py:693-697).
+ * rv_utils.py:8-47) and ufun-space proposals (variable.py:693-697), optionally coloured by
+ * the Cholesky factor of a covariance-matrix transition (has_prop_mat, rf.py:346-348).
  * ------------------------------------------------------------------------- */
 typedef struct {
   int32_t n_chains;
@@ -219,6 +220,14 @@ typedef struct {
   double* stat_sumsq;      /* [P][C] or NULL */
   double* out_xprop;       /* [T][P][C] or NULL: the proposal of every step (opqr.p values) */
   double* out_pprop;       /* [T][C] or NULL: the log-joint at the proposal (opqr.p.prob) */
+  /* set_tran(covariance) (rf.py:209-220,346-348), as K1's has_prop_mat: the delta of every
+   * step -- drawn, scaled or spherically rescaled, or injected -- is multiplied by prop_mat
+   * before the ufun move and the bound rule.  prop_mat is row-major [P][P] in its first P*P
+   * entries, lower-triangular with a positive diagonal and finite (pbx_mh_normreg_run returns
+   * PBX_ERR_INVALID otherwise); pbx_normreg_logjoint ignores both fields. */
+  int32_t has_prop_mat;
+  int32_t reserved0;
+  double prop_mat[PBX_MAX_PARAMS * PBX_MAX_PARAMS];
 } pbx_mh_normreg_params;
 
 PBX_API int pbx_mh_normreg_run(pbx_ctx* ctx, const pbx_mh_normreg_params* p);

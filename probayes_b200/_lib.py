@@ -83,6 +83,8 @@ class MhNormregParams(C.Structure):
         ("out_accept", C.c_void_p), ("out_score", C.c_void_p),
         ("accept_count", C.c_void_p), ("stat_sum", C.c_void_p), ("stat_sumsq", C.c_void_p),
         ("out_xprop", C.c_void_p), ("out_pprop", C.c_void_p),
+        ("has_prop_mat", C.c_int32), ("reserved0", C.c_int32),
+        ("prop_mat", C.c_double * (PBX_MAX_PARAMS * PBX_MAX_PARAMS)),
     ]
 
 

@@ -43,6 +43,8 @@ struct NrModel {
   double scale[PBX_MAX_PARAMS];
   double nlhv[PBX_MAX_PARAMS];      // -log(length in ufun space): rv.py:153-166
   double radius;
+  int has_L;                        // colour the delta with L (set_tran(covariance))
+  double L[PBX_MAX_PARAMS][PBX_MAX_PARAMS];   // lower-triangular, zero outside [P][P]
 };
 
 struct NrArgs {
@@ -80,12 +82,28 @@ struct NrArgs {
 };
 
 // ----------------------------------------------------------------------------
-// proposal: theta' = ufun^-1(ufun(theta) + delta)  (variable.py:693-697)
+// proposal: theta' = ufun^-1(ufun(theta) + L delta)  (variable.py:693-697, rf.py:346-348)
 // ----------------------------------------------------------------------------
+// delta <- L delta for a lower-triangular L, in place: row i reads entries j <= i only, so
+// the rows are taken from the last to the first
+__device__ __forceinline__ void nr_colour(const NrModel& m, int P, double (&dl)[PBX_MAX_PARAMS]) {
+#pragma unroll
+  for (int i = PBX_MAX_PARAMS - 1; i >= 0; --i) {
+    if (i >= P) continue;
+    double acc = 0.0;
+#pragma unroll
+    for (int j = 0; j <= i; ++j) acc = fma(m.L[i][j], dl[j], acc);
+    dl[i] = acc;
+  }
+}
+
 // kP: the parameter count at compile time (0 = read m.P): with it every index below is a
 // constant and the arrays stay in registers (runtime bounds put them into local memory, which
-// only the one-launch walk kernel -- a latency-bound chain per warp -- cares about)
-template <int kP = 0>
+// only the one-launch walk kernel -- a latency-bound chain per warp -- cares about).
+// The raw draw (injected, or Philox scaled / spherically rescaled) is coloured last, as the
+// reference multiplies its delta draw by the Cholesky factor of set_tran(covariance).
+// kColour = false compiles the colouring out (see nr_move for why the kernels care)
+template <int kP = 0, bool kColour = true>
 __device__ __forceinline__ void nr_draw_delta(const NrArgs& a, const NrModel& m, int64_t gstep,
                                               int kk, int c, double (&dl)[PBX_MAX_PARAMS]) {
   const int64_t C = a.C;
@@ -94,39 +112,40 @@ __device__ __forceinline__ void nr_draw_delta(const NrArgs& a, const NrModel& m,
 #pragma unroll
     for (int j = 0; j < PBX_MAX_PARAMS; ++j)
       if (j < P) dl[j] = a.inj_delta[((int64_t)kk * P + j) * C + c];
-    return;
-  }
-  const uint32_t gchain = (uint32_t)(a.chain0 + c);
+  } else {
+    const uint32_t gchain = (uint32_t)(a.chain0 + c);
 #pragma unroll
-  for (int s = 0; s < (PBX_MAX_PARAMS + 1) / 2; ++s) {
-    if (s >= (P + 1) / 2) break;
-    pbx_u4 w = pbx_block(a.seed, (uint64_t)gstep, gchain, (uint32_t)s);
-    double d0, d1;
-    if (m.prop_kind == PBX_PROP_NORMAL) {
-      pbx_normal_pair(w, d0, d1);
-      d0 *= m.scale[2 * s];
-      if (2 * s + 1 < P) d1 *= m.scale[2 * s + 1];
-    } else if (m.prop_kind == PBX_PROP_UNIFORM) {
-      d0 = -m.scale[2 * s] + (2.0 * m.scale[2 * s]) * pbx_u52(w.x, w.y);
-      d1 = (2 * s + 1 < P) ? -m.scale[2 * s + 1] + (2.0 * m.scale[2 * s + 1]) * pbx_u32(w.z)
-                             : 0.0;
-    } else {                       // spherical: cube sample, rescaled below
-      d0 = -m.radius + (2.0 * m.radius) * pbx_u52(w.x, w.y);
-      d1 = (2 * s + 1 < P) ? -m.radius + (2.0 * m.radius) * pbx_u32(w.z) : 0.0;
+    for (int s = 0; s < (PBX_MAX_PARAMS + 1) / 2; ++s) {
+      if (s >= (P + 1) / 2) break;
+      pbx_u4 w = pbx_block(a.seed, (uint64_t)gstep, gchain, (uint32_t)s);
+      double d0, d1;
+      if (m.prop_kind == PBX_PROP_NORMAL) {
+        pbx_normal_pair(w, d0, d1);
+        d0 *= m.scale[2 * s];
+        if (2 * s + 1 < P) d1 *= m.scale[2 * s + 1];
+      } else if (m.prop_kind == PBX_PROP_UNIFORM) {
+        d0 = -m.scale[2 * s] + (2.0 * m.scale[2 * s]) * pbx_u52(w.x, w.y);
+        d1 = (2 * s + 1 < P) ? -m.scale[2 * s + 1] + (2.0 * m.scale[2 * s + 1]) * pbx_u32(w.z)
+                               : 0.0;
+      } else {                       // spherical: cube sample, rescaled below
+        d0 = -m.radius + (2.0 * m.radius) * pbx_u52(w.x, w.y);
+        d1 = (2 * s + 1 < P) ? -m.radius + (2.0 * m.radius) * pbx_u32(w.z) : 0.0;
+      }
+      dl[2 * s] = d0;
+      if (2 * s + 1 < P) dl[2 * s + 1] = d1;
     }
-    dl[2 * s] = d0;
-    if (2 * s + 1 < P) dl[2 * s + 1] = d1;
-  }
-  if (m.prop_kind == PBX_PROP_SPHERICAL) {   // field.py:509-531
-    double ss = 0.0;
+    if (m.prop_kind == PBX_PROP_SPHERICAL) {   // field.py:509-531
+      double ss = 0.0;
 #pragma unroll
-    for (int j = 0; j < PBX_MAX_PARAMS; ++j)
-      if (j < P) ss += dl[j] * dl[j];
-    const double nrm = (ss >= PBX_TINY) ? sqrt(ss) : 0.0;
+      for (int j = 0; j < PBX_MAX_PARAMS; ++j)
+        if (j < P) ss += dl[j] * dl[j];
+      const double nrm = (ss >= PBX_TINY) ? sqrt(ss) : 0.0;
 #pragma unroll
-    for (int j = 0; j < PBX_MAX_PARAMS; ++j)
-      if (j < P) dl[j] = ((dl[j] * m.radius) / nrm) * m.scale[j];
+      for (int j = 0; j < PBX_MAX_PARAMS; ++j)
+        if (j < P) dl[j] = ((dl[j] * m.radius) / nrm) * m.scale[j];
+    }
   }
+  if (kColour && m.has_L) nr_colour(m, P, dl);
 }
 
 __device__ __forceinline__ double nr_threshold(const NrArgs& a, int64_t gstep, int kk, int c) {
@@ -140,9 +159,9 @@ __device__ __forceinline__ double nr_threshold(const NrArgs& a, int64_t gstep, i
 // ----------------------------------------------------------------------------
 // coordinate j of the proposal: ufun^-1(ufun(th) + dl) (variable.py:693-697), then the bound
 // rule.  kBound = false compiles the bound rule out: the one-launch-per-step kernels pass their
-// kExtras there, so that the rarely used per-step extras (bounded deltas, proposal outputs)
-// never perturb the register allocation of the hot likelihood loops of the common
-// configuration (a 9 % effect when it happened)
+// kExtras there (and to nr_draw_delta's kColour), so that the rarely used per-step extras
+// (bounded or coloured deltas, proposal outputs) never perturb the register allocation of the
+// hot likelihood loops of the common configuration (a 9 % effect when it happened)
 template <bool kBound>
 __device__ __forceinline__ double nr_move(const NrModel& m, int j, double th, double dl) {
   const double v = m.log_ufun[j] ? exp(log(th) + dl) : th + dl;
@@ -218,7 +237,7 @@ template <bool kExtras>
 __device__ __forceinline__ void nr_propose(const NrArgs& a, const NrModel& m, int64_t gstep,
                                            int kk, int c, const double* th) {
   double dl[PBX_MAX_PARAMS];
-  nr_draw_delta(a, m, gstep, kk, c, dl);
+  nr_draw_delta<0, kExtras>(a, m, gstep, kk, c, dl);
   for (int j = 0; j < m.P; ++j)
     a.prop[(int64_t)j * a.C + c] = nr_move<kExtras>(m, j, th[j], dl[j]);
 }
@@ -615,6 +634,18 @@ static int nr_validate(const pbx_mh_normreg_params* p, const char* who, bool nee
     PBX_REQUIRE(p->state && p->state_lp, "%s: state/state_lp are mandatory", who);
     PBX_REQUIRE((p->inj_delta == nullptr) == (p->inj_thresh == nullptr),
                 "%s: inj_delta and inj_thresh must be given together", who);
+    if (p->has_prop_mat) {
+      const int P = p->n_params;
+      for (int i = 0; i < P; ++i)
+        for (int j = 0; j < P; ++j) {
+          const double v = p->prop_mat[i * P + j];
+          PBX_REQUIRE(isfinite(v), "%s: prop_mat[%d][%d] is not finite", who, i, j);
+          PBX_REQUIRE(j <= i || v == 0.0,
+                      "%s: prop_mat must be lower-triangular (entry [%d][%d] = %g)", who, i, j, v);
+          PBX_REQUIRE(j != i || v > 0.0,
+                      "%s: prop_mat needs a positive diagonal (entry [%d][%d] = %g)", who, i, i, v);
+        }
+    }
   }
   return PBX_OK;
 }
@@ -639,10 +670,15 @@ static void nr_fill_model(const pbx_mh_normreg_params* p, NrModel& m) {
       len = p->log_ufun[j] ? log(p->lims[j][1]) - log(p->lims[j][0]) : p->lims[j][1] - p->lims[j][0];
     m.nlhv[j] = -log(len);
   }
+  // the factor is read by pbx_mh_normreg_run only (pbx_normreg_logjoint draws no proposal)
+  m.has_L = p->has_prop_mat != 0;
+  for (int i = 0; i < PBX_MAX_PARAMS; ++i)
+    for (int j = 0; j < PBX_MAX_PARAMS; ++j)
+      m.L[i][j] = (m.has_L && i < p->n_params && j <= i) ? p->prop_mat[i * p->n_params + j] : 0.0;
 }
 
 static bool nr_extras(const NrArgs& a, const NrModel& m) {
-  return m.bound != 0 || a.out_xprop != nullptr || a.out_pprop != nullptr;
+  return m.bound != 0 || m.has_L != 0 || a.out_xprop != nullptr || a.out_pprop != nullptr;
 }
 
 template <int KC>
@@ -814,8 +850,17 @@ __global__ void __launch_bounds__(256) ss_eval_kernel(const NrArgs a, const __gr
   a.eval_out[c] = nr_logjoint(a, m, th, ss_rss(st, m, th));
 }
 
+// log(t) for nr_decide where a lambda cannot be used: nvcc 12.9's front end aborts on the
+// [&] { return log(t); } of nr_phase_b inside the templated ss_walk_kernel
+struct NrLogOf {
+  double t;
+  __device__ double operator()() const { return log(t); }
+};
+
 // the whole walk of one chain in one thread (the same draws, accept rule and records as
-// nr_phase_b, with the O(1) likelihood)
+// nr_phase_b, with the O(1) likelihood); kColour as nr_draw_delta's (the runtime test alone
+// slows the uncoloured walk by 4 %)
+template <bool kColour>
 __global__ void __launch_bounds__(128) ss_walk_kernel(const NrArgs a, const __grid_constant__ NrModel m,
                                                       const NrStats* __restrict__ stp) {
   const int c = blockIdx.x * blockDim.x + threadIdx.x;
@@ -832,13 +877,12 @@ __global__ void __launch_bounds__(128) ss_walk_kernel(const NrArgs a, const __gr
   for (int k = 0; k < a.T; ++k) {
     const int64_t gstep = a.step0 + k;
     double dl[PBX_MAX_PARAMS], thp[PBX_MAX_PARAMS];
-    nr_draw_delta(a, m, gstep, k, c, dl);
+    nr_draw_delta<0, kColour>(a, m, gstep, k, c, dl);
     for (int j = 0; j < m.P; ++j) thp[j] = nr_move<true>(m, j, th[j], dl[j]);
     const double lpp = nr_logjoint(a, m, thp, ss_rss(st, m, thp));
     const double t = nr_threshold(a, gstep, k, c);
     double s;
-    const bool acc = nr_decide(m, lpp, lp, t, [&] { return log(t); }, gstep,
-                               a.out_score != nullptr, s);
+    const bool acc = nr_decide(m, lpp, lp, t, NrLogOf{t}, gstep, a.out_score != nullptr, s);
     if (acc) {
       for (int j = 0; j < m.P; ++j) th[j] = thp[j];
       lp = lpp;
@@ -868,7 +912,8 @@ __global__ void __launch_bounds__(128) ss_walk_kernel(const NrArgs a, const __gr
 // ---------------------------------------------------------------------------
 #define RW_WARPS 4
 #define RW_MAXN 8192
-template <bool kSlope>
+// kColour: as nr_draw_delta's (the colouring costs this kernel registers)
+template <bool kSlope, bool kColour>
 __global__ void __launch_bounds__(32 * RW_WARPS)
     rw_walk_kernel(const NrArgs a, const __grid_constant__ NrModel m) {
   extern __shared__ __align__(16) double rw_sm[];       // y[N], then x[N] (kSlope)
@@ -927,7 +972,7 @@ __global__ void __launch_bounds__(32 * RW_WARPS)
     if ((k & 31) == 0) {
       const int mine = k + lane;
       if (mine < a.T) {
-        nr_draw_delta<P>(a, m, a.step0 + mine, mine, c, dlv);
+        nr_draw_delta<P, kColour>(a, m, a.step0 + mine, mine, c, dlv);
         tv = nr_threshold(a, a.step0 + mine, mine, c);
         ltv = log(tv);
       }
@@ -1028,7 +1073,8 @@ static int nr_walk_suffstat(pbx_ctx* ctx, const NrArgs& a, const NrModel& m) {
   NrStats* st = nullptr;
   int rc = pbx_ss_compute(ctx, m.has_slope ? a.x : nullptr, a.y, a.N, &st);
   if (rc) return rc;
-  ss_walk_kernel<<<(a.C + 127) / 128, 128, 0, ctx->stream>>>(a, m, st);
+  if (m.has_L) ss_walk_kernel<true><<<(a.C + 127) / 128, 128, 0, ctx->stream>>>(a, m, st);
+  else ss_walk_kernel<false><<<(a.C + 127) / 128, 128, 0, ctx->stream>>>(a, m, st);
   PBX_LAUNCH_CHECK(ctx);
   return PBX_OK;
 }
@@ -1041,15 +1087,17 @@ static int nr_walk_small(pbx_ctx* ctx, const NrArgs& a, const NrModel& m) {
   int wpc = (a.C + 2 * ctx->sm_count - 1) / (2 * ctx->sm_count);
   wpc = wpc < 1 ? 1 : (wpc > RW_WARPS ? RW_WARPS : wpc);
   const int grid = (a.C + wpc - 1) / wpc;
-  if (m.has_slope) {
-    PBX_CUDA(cudaFuncSetAttribute(rw_walk_kernel<true>,
-                                  cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    rw_walk_kernel<true><<<grid, 32 * wpc, smem, ctx->stream>>>(a, m);
-  } else {
-    PBX_CUDA(cudaFuncSetAttribute(rw_walk_kernel<false>,
-                                  cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    rw_walk_kernel<false><<<grid, 32 * wpc, smem, ctx->stream>>>(a, m);
-  }
+#define RW_GO(S, L)                                                                            \
+  do {                                                                                         \
+    PBX_CUDA(cudaFuncSetAttribute(rw_walk_kernel<S, L>,                                        \
+                                  cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));    \
+    rw_walk_kernel<S, L><<<grid, 32 * wpc, smem, ctx->stream>>>(a, m);                         \
+  } while (0)
+  if (m.has_slope && m.has_L) RW_GO(true, true);
+  else if (m.has_slope) RW_GO(true, false);
+  else if (m.has_L) RW_GO(false, true);
+  else RW_GO(false, false);
+#undef RW_GO
   PBX_LAUNCH_CHECK(ctx);
   return PBX_OK;
 }

@@ -339,7 +339,7 @@ class Engine:
     # ------------------------------------------------- K2: streaming normal MH
     def _normreg_params(self, C_, P, x_obs, y_obs, lims, open_end, log_ufun, prop_scale,
                         accept="log", accept_coef=1.0, prop="uniform", variant=0,
-                        prop_radius=0.0, prop_bound=False):
+                        prop_radius=0.0, prop_bound=False, prop_chol=None):
         if P not in (2, 3):
             raise NotImplementedError("normal-likelihood MH supports (mu, sigma) or "
                                       "(b0, b1, sigma) parameters, got %d" % P)
@@ -369,16 +369,25 @@ class Engine:
             p.open_end[j][0], p.open_end[j][1] = int(open_end[j][0]), int(open_end[j][1])
             p.log_ufun[j] = int(log_ufun[j])
             p.prop_scale[j] = scale[j]
+        if prop_chol is not None:
+            L = np.asarray(prop_chol, dtype=np.float64)
+            if L.shape != (P, P):
+                raise ValueError("prop_chol must be [P, P]")
+            p.has_prop_mat = 1
+            for i, v in enumerate(L.ravel()):
+                p.prop_mat[i] = v
         return p
 
     def mh_normreg(self, state, y_obs, x_obs, steps, lims, open_end, log_ufun, prop_scale,
                    thin=1, seed=0, step0=0, chain0=0, accept="log", accept_coef=1.0,
                    prop="uniform", variant=0, inj_delta=None, inj_thresh=None, state_lp=None,
                    record=True, per_step=False, stats=True, prop_radius=0.0,
-                   prop_bound=False):
+                   prop_bound=False, prop_chol=None):
         """MH on the iid-normal posterior; ``state`` [P, C] device fp64 (in place),
         ``y_obs``/``x_obs`` device fp64 [N].  Same outputs as :meth:`mh_mvn`; the
-        recorded ``prob`` is the log-joint (log pscale)."""
+        recorded ``prob`` is the log-joint (log pscale).  ``prop_chol`` [P, P]: the
+        lower-triangular factor every delta is multiplied by before the ufun move
+        (set_tran(covariance), rf.py:346-348), injected deltas included."""
         torch = _torch()
         P, C_ = state.shape
         T = int(steps)
@@ -391,7 +400,8 @@ class Engine:
         self._dev(inj_delta, (T, P, C_), "inj_delta")
         self._dev(inj_thresh, (T, C_), "inj_thresh")
         p = self._normreg_params(C_, P, x_obs, y_obs, lims, open_end, log_ufun, prop_scale,
-                                 accept, accept_coef, prop, variant, prop_radius, prop_bound)
+                                 accept, accept_coef, prop, variant, prop_radius, prop_bound,
+                                 prop_chol)
         p.n_steps, p.thin, p.step0, p.chain0 = T, thin, step0, chain0
         p.seed = seed & 0xFFFFFFFFFFFFFFFF
         if state_lp is None:

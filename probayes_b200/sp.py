@@ -579,7 +579,7 @@ class SP(SD):
             out = eng.mh_normreg(state, y, x, T, lims, ex, lg, prop['scale'], thin=thin,
                                  seed=seed, step0=step0, accept=accept, accept_coef=coef,
                                  prop=prop['kind'], prop_radius=prop['radius'],
-                                 prop_bound=prop['bound'],
+                                 prop_bound=prop['bound'], prop_chol=prop['chol'],
                                  inj_delta=inj_d, inj_thresh=inj_t,
                                  state_lp=sampler.state_lp, per_step=per_step,
                                  variant=opts['variant'], chain0=chain0)
