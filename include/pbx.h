@@ -62,6 +62,9 @@ typedef enum {
 #define PBX_PROP_UNIFORM 1         /* delta_j = -scale_j + 2 scale_j r_j, r ~ U(0,1)  ([delta] lists) */
 #define PBX_PROP_SPHERICAL 2       /* u_j ~ U(-R, R); delta_j = (u_j R / |u|) scale_j  ((delta,) tuples,
                                       field.py:509-531; R = prop_radius) */
+/* iid likelihood family of K2 / K3 (pbx_mh_normreg_params.lik_kind) */
+#define PBX_LIK_NORMAL 0           /* scipy.stats.norm.logpdf */
+#define PBX_LIK_STUDENT_T 1        /* scipy.stats.t.logpdf (cauchy.logpdf: df = 1) */
 
 typedef struct pbx_ctx pbx_ctx;
 
@@ -228,6 +231,18 @@ typedef struct {
   int32_t has_prop_mat;
   int32_t reserved0;
   double prop_mat[PBX_MAX_PARAMS * PBX_MAX_PARAMS];
+  /* the iid likelihood of every observation, y_i ~ family(loc_i, sigma).  PBX_LIK_NORMAL (a
+   * zeroed tail) is scipy.stats.norm.logpdf; PBX_LIK_STUDENT_T is scipy.stats.t.logpdf with
+   * df = lik_df (cauchy.logpdf: lik_df = 1), per observation
+   *   lik_logc - (lik_df + 1)/2 log1p(z^2 / lik_df) - log sigma,   z = (y_i - loc_i) / sigma,
+   * where the caller computes lik_logc = log(poch(df/2, 1/2)) - (log df + log pi)/2 as scipy
+   * does (lgamma((df+1)/2) - lgamma(df/2) cancels: 9e-7 relative at df = 1e9).  Student-t needs
+   * 0 < lik_df < inf and a finite lik_logc, and refuses variant 3 (the t likelihood has no
+   * sufficient statistics); both entry points return PBX_ERR_INVALID otherwise. */
+  int32_t lik_kind;        /* PBX_LIK_* */
+  int32_t reserved1;
+  double lik_df;
+  double lik_logc;
 } pbx_mh_normreg_params;
 
 PBX_API int pbx_mh_normreg_run(pbx_ctx* ctx, const pbx_mh_normreg_params* p);
@@ -250,6 +265,14 @@ PBX_API int pbx_grid_norm_logjoint(pbx_ctx* ctx, const double* x_obs, int64_t n_
                            const double* sigma, int32_t n_sigma,
                            const double* logprior_mu, const double* logprior_sigma,
                            double* out);
+/* the same grid with a Student-t likelihood: out[m][s] = logprior_mu[m] + logprior_sigma[s]
+ * + sum_i t.logpdf(x_i; df, mu_m, sigma_s), logc as pbx_mh_normreg_params.lik_logc
+ * (0 < df < inf, logc finite; PBX_ERR_INVALID otherwise) */
+PBX_API int pbx_grid_t_logjoint(pbx_ctx* ctx, const double* x_obs, int64_t n_obs,
+                                const double* mu, int32_t n_mu, const double* sigma,
+                                int32_t n_sigma, const double* logprior_mu,
+                                const double* logprior_sigma, double* out, double df,
+                                double logc);
 /* opt-in: the same values (<= 1e-15) from centred sufficient statistics of the
  * observations: one reduction over x_obs, then O(1) per cell instead of O(N) */
 PBX_API int pbx_grid_norm_logjoint_ss(pbx_ctx* ctx, const double* x_obs, int64_t n_obs,

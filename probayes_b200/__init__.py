@@ -20,7 +20,8 @@ from .cond_cov import CondCov
 from .serial import (serialise, deserialise, write_serialised, read_serialised, write_dist,
                      read_dist)
 from . import catalogue
-from .catalogue import NormalRegression, BallIndicator, NormalProduct, BoxUniform
+from .catalogue import (NormalRegression, StudentTRegression, BallIndicator, NormalProduct,
+                        BoxUniform)
 from ._lib import PbxError
 
 __version__ = "0.1.0"

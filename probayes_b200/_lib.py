@@ -11,6 +11,7 @@ PBX_MAX_DIMS = 8
 PBX_MAX_PARAMS = 3
 ACCEPT_REFERENCE, ACCEPT_LOG = 0, 1
 PROP_NORMAL, PROP_UNIFORM, PROP_SPHERICAL = 0, 1, 2
+LIK_NORMAL, LIK_STUDENT_T = 0, 1
 
 c_double_p = C.POINTER(C.c_double)
 
@@ -85,6 +86,8 @@ class MhNormregParams(C.Structure):
         ("out_xprop", C.c_void_p), ("out_pprop", C.c_void_p),
         ("has_prop_mat", C.c_int32), ("reserved0", C.c_int32),
         ("prop_mat", C.c_double * (PBX_MAX_PARAMS * PBX_MAX_PARAMS)),
+        ("lik_kind", C.c_int32), ("reserved1", C.c_int32),
+        ("lik_df", C.c_double), ("lik_logc", C.c_double),
     ]
 
 
@@ -123,6 +126,9 @@ SIGNATURES = {
     "pbx_grid_norm_logjoint": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p,
                                          C.c_int32, C.c_void_p, C.c_int32, C.c_void_p,
                                          C.c_void_p, C.c_void_p]),
+    "pbx_grid_t_logjoint": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p,
+                                      C.c_int32, C.c_void_p, C.c_int32, C.c_void_p,
+                                      C.c_void_p, C.c_void_p, C.c_double, C.c_double]),
     "pbx_grid_norm_logjoint_ss": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p,
                                             C.c_int32, C.c_void_p, C.c_int32, C.c_void_p,
                                             C.c_void_p, C.c_void_p]),

@@ -10,9 +10,11 @@ Targets
   mvn      scipy.stats.multivariate_normal(mean, cov)        (mcmc_prob4a, gibbs_norm2d)
   norm     scipy.stats.norm.logpdf + order={'x': 0, 'mu': 'loc', 'sigma': 'scale'}
            with iid=True                                      (metrohast_norm1d, dgei_*)
+           -- or scipy.stats.t.logpdf with df=nu, or scipy.stats.cauchy.logpdf, in the
+           same call: the spec's ``lik`` entry names the family
   normreg  a Python callable that IS norm.logpdf(y, loc=b0 + b1*x, scale=s) -- verified
            numerically by probing it against every role assignment (gibbs_linreg's
-           ``norm_reg``), or an explicit ``NormalRegression`` spec
+           ``norm_reg``), or an explicit ``NormalRegression`` / ``StudentTRegression`` spec
 Proposals (field.py:220-317, variable.py:600-638, rf.py:209-220)
   [d] uniform per RV, (d,) spherical, frozen scipy.stats.norm, covariance-matrix tran
 Rejection sampling (set_prop + custom scores / thresh / update, omc_rejection_sp_circle)
@@ -24,6 +26,7 @@ Rejection sampling (set_prop + custom scores / thresh / update, omc_rejection_sp
 import inspect
 import itertools
 import numpy as np
+import scipy.special
 import scipy.stats
 
 from .pscales import iscomplex, rescale
@@ -34,6 +37,61 @@ class NormalRegression:
 
     def __init__(self, x, y, intercept, slope, scale):
         self.x, self.y, self.intercept, self.slope, self.scale = x, y, intercept, slope, scale
+
+
+class StudentTRegression:
+    """Explicit catalogue spec of y ~ t_df(intercept + slope*x, scale) (log-density,
+    scipy.stats.t.logpdf); ``df=np.inf`` is the normal regression."""
+
+    def __init__(self, x, y, intercept, slope, scale, df=None):
+        self.x, self.y, self.intercept, self.slope, self.scale = x, y, intercept, slope, scale
+        self.df = df
+
+
+def t_logc(df):
+    """The per-observation constant of scipy.stats.t.logpdf, computed as scipy's t_gen._logpdf
+    does: log(poch(df/2, 1/2)) - (log df + log pi)/2.  (lgamma((df+1)/2) - lgamma(df/2)
+    cancels: 6e-10 relative at df = 1e6, which N observations multiply.)"""
+    df = np.float64(df)
+    return float(np.log(scipy.special.poch(0.5 * df, 0.5)) - 0.5 * (np.log(df) + np.log(np.pi)))
+
+
+def likelihood(family, df=None):
+    """The ``lik`` entry of a target spec: None for the normal, else dict(family, df, logc)
+    for the Student-t (df = nu) or the Cauchy (df = 1, logc = -log pi as cauchy.logpdf).
+    A t with df = inf is the normal, as in scipy (t_gen._logpdf calls norm._logpdf)."""
+    if family == 'norm':
+        return None
+    if family == 'cauchy':
+        return dict(family='cauchy', df=1.0, logc=float(-np.log(np.pi)))
+    if df is None:
+        raise ValueError("the Student-t likelihood needs its degrees of freedom: "
+                         "set_prob(scipy.stats.t.logpdf, ..., df=nu)")
+    try:
+        df = float(df)
+    except (TypeError, ValueError):
+        raise ValueError("df must be a positive number, got {!r}".format(df))
+    if df == np.inf:
+        return None
+    if not df > 0:
+        raise ValueError("df must be positive (and not NaN), got {!r}".format(df))
+    return dict(family='t', df=df, logc=t_logc(df))
+
+
+def _with_lik(spec, lik):
+    """A normreg spec carries a ``lik`` entry for a non-normal likelihood only: the normal spec
+    (df = inf included) is the one the catalogue has always returned."""
+    if lik is not None:
+        spec['lik'] = lik
+    return spec
+
+
+def refuse_suffstat(spec, variant):
+    """suffstat=True (K2 variant 3) evaluates the normal likelihood from sufficient statistics,
+    which the Student-t likelihood does not have: refused before any device call."""
+    if variant == 3 and spec.get('lik') is not None:
+        raise NotImplementedError("suffstat=True needs the normal likelihood: the {} likelihood "
+                                  "has no sufficient statistics".format(spec['lik']['family']))
 
 
 def is_scipy_mvn(obj):
@@ -50,14 +108,19 @@ def mvn_args(args, kwds):
     return np.atleast_1d(np.asarray(mean, dtype=float)), np.atleast_2d(np.asarray(cov, dtype=float))
 
 
-def _norm_method(prob):
-    """'logpdf' / 'pdf' if prob is that bound method of scipy.stats.norm."""
+_LOC_SCALE = {'norm': scipy.stats.norm, 't': scipy.stats.t, 'cauchy': scipy.stats.cauchy}
+
+
+def _loc_scale_method(prob):
+    """(family, 'logpdf' / 'pdf') if prob is that bound method of scipy.stats.norm, .t or
+    .cauchy, else (None, None)."""
     owner = getattr(prob, '__self__', None)
-    if owner is scipy.stats.norm or type(owner).__name__ == 'norm_gen':
-        name = getattr(prob, '__name__', None)
-        if name in ('logpdf', 'pdf'):
-            return name
-    return None
+    for family, dist in _LOC_SCALE.items():
+        if owner is dist or type(owner).__name__ == family + '_gen':
+            name = getattr(prob, '__name__', None)
+            if name in ('logpdf', 'pdf'):
+                return family, name
+    return None, None
 
 
 def identify_target(holder, stats, paras):
@@ -77,12 +140,13 @@ def identify_target(holder, stats, paras):
             raise ValueError("multivariate_normal over {} variables but {} means".format(
                 len(names), len(mean)))
         return dict(kind='mvn', mean=mean, cov=cov, names=names, log_pscale=log_pscale)
-    method = _norm_method(prob)
+    family, method = _loc_scale_method(prob)
     if method is not None:
         order = holder._order
         if not isinstance(order, dict):
             raise NotImplementedError(
-                "scipy.stats.norm.{} needs order={{obs: 0, mean: 'loc', sd: 'scale'}}".format(method))
+                "scipy.stats.{}.{} needs order={{obs: 0, mean: 'loc', sd: 'scale'}}".format(
+                    family, method))
         roles = {v: k for k, v in order.items()}
         try:
             obs, loc, scale = roles[0], roles['loc'], roles['scale']
@@ -90,16 +154,24 @@ def identify_target(holder, stats, paras):
             raise NotImplementedError("unrecognised order mapping {}".format(order))
         if method == 'pdf' or not log_pscale:
             raise NotImplementedError(
-                "the iid normal likelihood is in the catalogue in log pscale only "
-                "(set_prob(scipy.stats.norm.logpdf, ..., pscale='log'))")
+                "the iid {} likelihood is in the catalogue in log pscale only "
+                "(set_prob(scipy.stats.{}.logpdf, ..., pscale='log'))".format(family, family))
         if paras is None or obs not in stats.keyset or {loc, scale} - paras.keyset:
             raise NotImplementedError("order must map a stats RV to 0 and parameter RVs "
                                       "to 'loc'/'scale'")
-        return dict(kind='normreg', has_slope=False, obs_y=obs, obs_x=None,
-                    params=[loc, scale], log_pscale=True)
-    if isinstance(prob, NormalRegression):
-        return dict(kind='normreg', has_slope=True, obs_y=prob.y, obs_x=prob.x,
-                    params=[prob.intercept, prob.slope, prob.scale], log_pscale=True)
+        return _with_lik(dict(kind='normreg', has_slope=False, obs_y=obs, obs_x=None,
+                              params=[loc, scale], log_pscale=True),
+                         likelihood(family, (kwds or {}).get('df')))
+    if isinstance(prob, (NormalRegression, StudentTRegression)):
+        lik = None
+        if isinstance(prob, StudentTRegression):
+            if not log_pscale:
+                raise NotImplementedError("StudentTRegression is in the catalogue in log pscale "
+                                          "only (set_prob(..., pscale='log'))")
+            lik = likelihood('t', prob.df)
+        return _with_lik(dict(kind='normreg', has_slope=True, obs_y=prob.y, obs_x=prob.x,
+                              params=[prob.intercept, prob.slope, prob.scale], log_pscale=True),
+                         lik)
     if callable(prob):
         spec = _probe_normreg(prob, stats, paras, log_pscale)
         if spec is not None:

@@ -2,7 +2,7 @@
 // posterior (examples/dgei/dgei_norm1d_improved.py:36-43).
 //
 // K3  log-joint[m][s] = (logprior_mu[m] + logprior_sigma[s])
-//                       + sum_i norm.logpdf(x_i; mu_m, sigma_s)
+//                       + sum_i norm.logpdf(x_i; mu_m, sigma_s)   (or t.logpdf, df nu)
 //     The reference materialises the [N, M, S] tensor and np.sum(axis=0)s it
 //     (probayes/rf.py:565-581, pd.py:368), then prod_rule adds the priors
 //     (pd_utils.py:85-328, pscales.py:160-216).  Here every CTA owns 1 mu x 1024
@@ -21,11 +21,17 @@
 #define GR_THREADS 128
 #define GR_KS 8                        // sigma cells per thread
 
+// kLik = PBX_LIK_STUDENT_T: t.logpdf with df nu, the sum N logc - N log sigma
+// - (nu+1)/2 sum_i log1p((x_i - mu)^2 / (nu sigma^2)) (logc from the host, see pbx.h).  df and
+// logc are the last arguments, unread by the normal instantiation, so that its argument
+// offsets and SASS are those of the normal-only kernel
+template <int kLik>
 __global__ void __launch_bounds__(GR_THREADS)
     grid_logjoint_kernel(const double* __restrict__ x, int64_t N, const double* __restrict__ mu,
                          const double* __restrict__ sigma, int S,
                          const double* __restrict__ lp_mu, const double* __restrict__ lp_sigma,
-                         double* __restrict__ out, int use_tma) {
+                         double* __restrict__ out, int use_tma, double df, double logc) {
+  constexpr bool kT = kLik == PBX_LIK_STUDENT_T;
   __shared__ __align__(128) double sm[GR_STAGES][GR_TILE];
   __shared__ __align__(8) unsigned long long full_bar[GR_STAGES];
   const int m = blockIdx.y;
@@ -35,7 +41,8 @@ __global__ void __launch_bounds__(GR_THREADS)
 #pragma unroll
   for (int k = 0; k < GR_KS; ++k) {
     const int s = s_base + k * GR_THREADS;
-    isg[k] = (s < S) ? 1.0 / sigma[s] : 0.0;
+    // Student-t: isg holds q = 1/(nu sigma^2)
+    isg[k] = (s < S) ? (kT ? 1.0 / (df * (sigma[s] * sigma[s])) : 1.0 / sigma[s]) : 0.0;
     acc[k] = 0.0;
   }
   const int64_t n_full = N / GR_TILE;
@@ -52,9 +59,14 @@ __global__ void __launch_bounds__(GR_THREADS)
       const double d0 = xv.x - mu_m, d1 = xv.y - mu_m;
 #pragma unroll
       for (int k = 0; k < GR_KS; ++k) {
-        const double z0 = d0 * isg[k], z1 = d1 * isg[k];
-        acc[k] = fma(z0, z0, acc[k]);
-        acc[k] = fma(z1, z1, acc[k]);
+        if (kT) {
+          acc[k] += log1p((d0 * d0) * isg[k]);
+          acc[k] += log1p((d1 * d1) * isg[k]);
+        } else {
+          const double z0 = d0 * isg[k], z1 = d1 * isg[k];
+          acc[k] = fma(z0, z0, acc[k]);
+          acc[k] = fma(z1, z1, acc[k]);
+        }
       }
     }
   };
@@ -93,8 +105,12 @@ __global__ void __launch_bounds__(GR_THREADS)
       const double d0 = sm[0][even] - mu_m;
 #pragma unroll
       for (int k = 0; k < GR_KS; ++k) {
-        const double z0 = d0 * isg[k];
-        acc[k] = fma(z0, z0, acc[k]);
+        if (kT) {
+          acc[k] += log1p((d0 * d0) * isg[k]);
+        } else {
+          const double z0 = d0 * isg[k];
+          acc[k] = fma(z0, z0, acc[k]);
+        }
       }
     }
   }
@@ -103,7 +119,8 @@ __global__ void __launch_bounds__(GR_THREADS)
   for (int k = 0; k < GR_KS; ++k) {
     const int s = s_base + k * GR_THREADS;
     if (s < S) {
-      const double ll = -acc[k] * 0.5 - n * (PBX_LOG_SQRT_2PI + log(sigma[s]));
+      const double ll = kT ? -(0.5 * (df + 1.0)) * acc[k] + n * (logc - log(sigma[s]))
+                           : -acc[k] * 0.5 - n * (PBX_LOG_SQRT_2PI + log(sigma[s]));
       out[(int64_t)m * S + s] = (lpm + lp_sigma[s]) + ll;      // prior first (prod_rule)
     }
   }
@@ -112,24 +129,45 @@ __global__ void __launch_bounds__(GR_THREADS)
 // ---------------------------------------------------------------------------
 // C ABI
 // ---------------------------------------------------------------------------
-extern "C" int pbx_grid_norm_logjoint(pbx_ctx* ctx, const double* x_obs, int64_t n_obs,
-                                      const double* mu, int32_t n_mu, const double* sigma,
-                                      int32_t n_sigma, const double* logprior_mu,
-                                      const double* logprior_sigma, double* out) {
+template <int kLik>
+static int grid_logjoint(pbx_ctx* ctx, const char* who, const double* x_obs, int64_t n_obs,
+                         const double* mu, int32_t n_mu, const double* sigma, int32_t n_sigma,
+                         const double* logprior_mu, const double* logprior_sigma, double* out,
+                         double df, double logc) {
   PBX_REQUIRE(ctx && x_obs && mu && sigma && logprior_mu && logprior_sigma && out,
-              "pbx_grid_norm_logjoint: null argument");
-  PBX_REQUIRE(n_obs >= 1 && n_mu >= 1 && n_sigma >= 1,
-              "pbx_grid_norm_logjoint: sizes must be positive");
-  PBX_REQUIRE(n_mu <= 65535, "pbx_grid_norm_logjoint: at most 65535 mu rows per call (slab it)");
+              "%s: null argument", who);
+  PBX_REQUIRE(n_obs >= 1 && n_mu >= 1 && n_sigma >= 1, "%s: sizes must be positive", who);
+  PBX_REQUIRE(n_mu <= 65535, "%s: at most 65535 mu rows per call (slab it)", who);
   PBX_CUDA(cudaSetDevice(ctx->device));
   dim3 grid((n_sigma + GR_THREADS * GR_KS - 1) / (GR_THREADS * GR_KS), n_mu);
   const int use_tma = (((uintptr_t)x_obs) % 16 == 0) ? 1 : 0;
   PBX_CUDA(cudaEventRecord(ctx->ev0, ctx->stream));
-  grid_logjoint_kernel<<<grid, GR_THREADS, 0, ctx->stream>>>(
-      x_obs, n_obs, mu, sigma, n_sigma, logprior_mu, logprior_sigma, out, use_tma);
+  grid_logjoint_kernel<kLik><<<grid, GR_THREADS, 0, ctx->stream>>>(
+      x_obs, n_obs, mu, sigma, n_sigma, logprior_mu, logprior_sigma, out, use_tma, df, logc);
   PBX_LAUNCH_CHECK(ctx);
   PBX_CUDA(cudaEventRecord(ctx->ev1, ctx->stream));
   return PBX_OK;
+}
+
+extern "C" int pbx_grid_norm_logjoint(pbx_ctx* ctx, const double* x_obs, int64_t n_obs,
+                                      const double* mu, int32_t n_mu, const double* sigma,
+                                      int32_t n_sigma, const double* logprior_mu,
+                                      const double* logprior_sigma, double* out) {
+  return grid_logjoint<PBX_LIK_NORMAL>(ctx, "pbx_grid_norm_logjoint", x_obs, n_obs, mu, n_mu,
+                                       sigma, n_sigma, logprior_mu, logprior_sigma, out, 0.0,
+                                       0.0);
+}
+
+extern "C" int pbx_grid_t_logjoint(pbx_ctx* ctx, const double* x_obs, int64_t n_obs,
+                                   const double* mu, int32_t n_mu, const double* sigma,
+                                   int32_t n_sigma, const double* logprior_mu,
+                                   const double* logprior_sigma, double* out, double df,
+                                   double logc) {
+  PBX_REQUIRE(df > 0.0 && isfinite(df), "pbx_grid_t_logjoint: needs 0 < df < inf (got %g)", df);
+  PBX_REQUIRE(isfinite(logc), "pbx_grid_t_logjoint: logc is not finite");
+  return grid_logjoint<PBX_LIK_STUDENT_T>(ctx, "pbx_grid_t_logjoint", x_obs, n_obs, mu, n_mu,
+                                          sigma, n_sigma, logprior_mu, logprior_sigma, out, df,
+                                          logc);
 }
 
 // ---------------------------------------------------------------------------

@@ -1,8 +1,10 @@
 // pbx_mh_normreg.cu -- K2: streaming normal log-likelihood Metropolis-Hastings.
 //
 // Target (log pscale, iid=True, joint=True):
-//   log p(theta, data) = sum_j boxprior_j(theta_j) + sum_i norm.logpdf(y_i; loc_i, sigma)
+//   log p(theta, data) = sum_j boxprior_j(theta_j) + sum_i lik.logpdf(y_i; loc_i, sigma)
 //   loc_i = b0 + b1 x_i (has_slope, theta = (b0, b1, sigma)) or mu (theta = (mu, sigma))
+//   lik = norm, or t with nu degrees of freedom (kLik; cauchy = t with nu = 1), whose sum is
+//   N logc - N log sigma - (nu+1)/2 sum_i log1p(r_i^2 / (nu sigma^2)), logc from the host
 // following probayes/rf.py:541-581, pd.py:332-370 (iid product = sum over the
 // observation axis), sd.py:154-161 + rf_utils.py:10-22 + rv_utils.py:8-47 (product
 // with the independent box priors, prior first), scipy.stats.norm.logpdf per term,
@@ -10,8 +12,8 @@
 // sp_utils.py:19-64 / pscales.py:219-236.
 //
 // One MH step = ONE kernel launch:
-//   phase A  every CTA accumulates S_c = sum_i (y_i - loc_i)^2 over its slice of the
-//            observations for its chains and writes a partial sum;
+//   phase A  every CTA accumulates S_c = sum_i (y_i - loc_i)^2 (Student-t: the log1p sum)
+//            over its slice of the observations for its chains and writes a partial sum;
 //   phase B  the last CTA to finish (per chain group) reduces the partials in a
 //            fixed order, adds -N(log sqrt(2pi) + log sigma) and the priors, runs
 //            the accept test, records the sample and draws the NEXT proposal.
@@ -45,6 +47,14 @@ struct NrModel {
   double radius;
   int has_L;                        // colour the delta with L (set_tran(covariance))
   double L[PBX_MAX_PARAMS][PBX_MAX_PARAMS];   // lower-triangular, zero outside [P][P]
+};
+
+// the Student-t likelihood of a call (PBX_LIK_STUDENT_T; unread by the normal instantiations).
+// A kernel argument of its own, after the others, so that the normal kernels' argument
+// offsets -- and with them their SASS -- are those of the normal-only build
+struct NrLik {
+  double df;                   // nu
+  double logc;                 // log(poch(nu/2, 1/2)) - (log nu + log pi)/2, from the host
 };
 
 struct NrArgs {
@@ -242,14 +252,32 @@ __device__ __forceinline__ void nr_propose(const NrArgs& a, const NrModel& m, in
     a.prop[(int64_t)j * a.C + c] = nr_move<kExtras>(m, j, th[j], dl[j]);
 }
 
-// log-joint from the residual sum of squares S (see file header)
-template <int kP = 0>
+// one observation's term of the likelihood sum, residual r: r^2 (normal), or
+// log1p(r^2 q) with q = 1/(nu sigma^2) (Student-t)
+template <int kLik>
+__device__ __forceinline__ double nr_term(double acc, double r, double q) {
+  if (kLik == PBX_LIK_STUDENT_T) return acc + log1p((r * r) * q);
+  return fma(r, r, acc);
+}
+
+// q of nr_term for scale sg
+template <int kLik>
+__device__ __forceinline__ double nr_q(const NrLik& lik, double sg) {
+  return kLik == PBX_LIK_STUDENT_T ? 1.0 / (lik.df * (sg * sg)) : 0.0;
+}
+
+// log-joint from the likelihood sum S (see file header; for Student-t S = sum log1p(z^2/nu))
+template <int kP = 0, int kLik = PBX_LIK_NORMAL>
 __device__ __forceinline__ double nr_logjoint(const NrArgs& a, const NrModel& m, const double* th,
-                                              double S) {
+                                              double S, const NrLik& lik = NrLik{}) {
   const int P = kP ? kP : m.P;
   const double sg = th[P - 1];
   const double n = (double)a.N;
-  double ll = -(S / (sg * sg)) * 0.5 - n * (PBX_LOG_SQRT_2PI + log(sg));
+  double ll;
+  if (kLik == PBX_LIK_STUDENT_T)
+    ll = -(0.5 * (lik.df + 1.0)) * S + n * (lik.logc - log(sg));
+  else
+    ll = -(S / (sg * sg)) * 0.5 - n * (PBX_LOG_SQRT_2PI + log(sg));
   double prior = 0.0;
 #pragma unroll
   for (int j = 0; j < PBX_MAX_PARAMS; ++j) {
@@ -263,12 +291,12 @@ __device__ __forceinline__ double nr_logjoint(const NrArgs& a, const NrModel& m,
 }
 
 // phase B for one chain: S is the complete residual sum of squares of the proposal
-template <bool kExtras>
-__device__ void nr_phase_b(const NrArgs& a, const NrModel& m, int c, double S) {
+template <bool kExtras, int kLik>
+__device__ void nr_phase_b(const NrArgs& a, const NrModel& m, int c, double S, const NrLik& lik) {
   const int64_t C = a.C;
   double thp[PBX_MAX_PARAMS];
   for (int j = 0; j < m.P; ++j) thp[j] = a.theta_in[(int64_t)j * C + c];
-  const double lpp = nr_logjoint(a, m, thp, S);
+  const double lpp = nr_logjoint<0, kLik>(a, m, thp, S, lik);
   if (a.mode == 1) {
     a.eval_out[c] = lpp;
     return;
@@ -327,22 +355,24 @@ __device__ __forceinline__ bool nr_arrive_last(unsigned int* counter, unsigned i
 // phase A, "tiles": chains in registers, observation tiles via TMA bulk copies
 // grid = (n_slices, n_groups); group = NR_THREADS*KC chains
 // ----------------------------------------------------------------------------
-template <int KC, bool kSlope, bool kExtras>
+template <int KC, bool kSlope, bool kExtras, int kLik>
 __global__ void __launch_bounds__(NR_THREADS)
-    nr_tiles_kernel(const NrArgs a, const __grid_constant__ NrModel m, int use_tma) {
+    nr_tiles_kernel(const NrArgs a, const __grid_constant__ NrModel m, int use_tma,
+                    const NrLik lik) {
   extern __shared__ __align__(128) double sm[];            // [NR_STAGES][2][NR_TILE]
   __shared__ __align__(8) unsigned long long full_bar[NR_STAGES];
   const int slice = blockIdx.x, group = blockIdx.y;
   const int64_t C = a.C;
   const int cbase = group * (NR_THREADS * KC) + threadIdx.x;
 
-  double b0[KC], b1[KC], acc[KC];
+  double b0[KC], b1[KC], q[KC], acc[KC];
 #pragma unroll
   for (int k = 0; k < KC; ++k) {
     const int c = cbase + k * NR_THREADS;
     const bool v = c < a.C;
     b0[k] = v ? a.theta_in[c] : 0.0;
     b1[k] = (v && kSlope) ? a.theta_in[C + c] : 0.0;
+    q[k] = (kLik && v) ? nr_q<kLik>(lik, a.theta_in[(kSlope ? 2 : 1) * C + c]) : 0.0;
     acc[k] = 0.0;
   }
 
@@ -382,8 +412,8 @@ __global__ void __launch_bounds__(NR_THREADS)
       for (int k = 0; k < KC; ++k) {
         const double r0 = yv.x - (kSlope ? fma(b1[k], xv.x, b0[k]) : b0[k]);
         const double r1 = yv.y - (kSlope ? fma(b1[k], xv.y, b0[k]) : b0[k]);
-        acc[k] = fma(r0, r0, acc[k]);
-        acc1[k] = fma(r1, r1, acc1[k]);
+        acc[k] = nr_term<kLik>(acc[k], r0, q[k]);
+        acc1[k] = nr_term<kLik>(acc1[k], r1, q[k]);
       }
     }
   };
@@ -431,7 +461,7 @@ __global__ void __launch_bounds__(NR_THREADS)
 #pragma unroll
         for (int k = 0; k < KC; ++k) {
           const double r0 = yv - (kSlope ? fma(b1[k], xv, b0[k]) : b0[k]);
-          acc[k] = fma(r0, r0, acc[k]);
+          acc[k] = nr_term<kLik>(acc[k], r0, q[k]);
         }
       }
     }
@@ -449,7 +479,7 @@ __global__ void __launch_bounds__(NR_THREADS)
     if (c >= a.C) continue;
     double S = 0.0;
     for (int s = 0; s < a.n_slices; ++s) S += __ldcg(&a.partial[(int64_t)s * C + c]);
-    nr_phase_b<kExtras>(a, m, c, S);
+    nr_phase_b<kExtras, kLik>(a, m, c, S, lik);
   }
 }
 
@@ -463,17 +493,20 @@ __global__ void __launch_bounds__(NR_THREADS)
 // block reduction; phase B in the last CTA.
 // ----------------------------------------------------------------------------
 #define NRS_THREADS 256
-template <int KS, bool kSlope, bool kExtras>
+template <int KS, bool kSlope, bool kExtras, int kLik>
 __global__ void __launch_bounds__(NRS_THREADS)
-    nr_stream_kernel(const NrArgs a, const __grid_constant__ NrModel m, int use_tma) {
+    nr_stream_kernel(const NrArgs a, const __grid_constant__ NrModel m, int use_tma,
+                     const NrLik lik) {
   extern __shared__ __align__(128) double sm[];            // [NR_STAGES][2][NRS_TILE]
   __shared__ __align__(8) unsigned long long full_bar[NR_STAGES];
   __shared__ double s_red[NRS_THREADS / 32][KS];
-  double b0[KS], b1[KS], acc[KS];
+  double b0[KS], b1[KS], q[KS], acc[KS];
 #pragma unroll
   for (int k = 0; k < KS; ++k) {
     b0[k] = (k < a.C) ? a.theta_in[k] : 0.0;
     b1[k] = (k < a.C && kSlope) ? a.theta_in[(int64_t)a.C + k] : 0.0;
+    q[k] = (kLik && k < a.C) ? nr_q<kLik>(lik, a.theta_in[(int64_t)(kSlope ? 2 : 1) * a.C + k])
+                             : 0.0;
     acc[k] = 0.0;
   }
   const int64_t n_full = a.N / NRS_TILE;
@@ -503,8 +536,8 @@ __global__ void __launch_bounds__(NRS_THREADS)
       for (int k = 0; k < KS; ++k) {
         const double r0 = yv.x - (kSlope ? fma(b1[k], xv.x, b0[k]) : b0[k]);
         const double r1 = yv.y - (kSlope ? fma(b1[k], xv.y, b0[k]) : b0[k]);
-        acc[k] = fma(r0, r0, acc[k]);
-        acc[k] = fma(r1, r1, acc[k]);
+        acc[k] = nr_term<kLik>(acc[k], r0, q[k]);
+        acc[k] = nr_term<kLik>(acc[k], r1, q[k]);
       }
     }
   };
@@ -538,7 +571,7 @@ __global__ void __launch_bounds__(NRS_THREADS)
 #pragma unroll
       for (int k = 0; k < KS; ++k) {
         const double r0 = yv - (kSlope ? fma(b1[k], xv, b0[k]) : b0[k]);
-        acc[k] = fma(r0, r0, acc[k]);
+        acc[k] = nr_term<kLik>(acc[k], r0, q[k]);
       }
     }
   }
@@ -563,7 +596,7 @@ __global__ void __launch_bounds__(NRS_THREADS)
     const int c = threadIdx.x;
     double S = 0.0;
     for (int s = 0; s < (int)gridDim.x; ++s) S += __ldcg(&a.partial[(int64_t)s * a.C + c]);
-    nr_phase_b<kExtras>(a, m, c, S);
+    nr_phase_b<kExtras, kLik>(a, m, c, S, lik);
   }
 }
 
@@ -623,6 +656,15 @@ static int nr_validate(const pbx_mh_normreg_params* p, const char* who, bool nee
               "%s: unknown accept_mode", who);
   PBX_REQUIRE(p->prop_kind >= PBX_PROP_NORMAL && p->prop_kind <= PBX_PROP_SPHERICAL,
               "%s: unknown prop_kind", who);
+  PBX_REQUIRE(p->lik_kind == PBX_LIK_NORMAL || p->lik_kind == PBX_LIK_STUDENT_T,
+              "%s: unknown lik_kind %d", who, p->lik_kind);
+  if (p->lik_kind == PBX_LIK_STUDENT_T) {
+    PBX_REQUIRE(p->lik_df > 0.0 && isfinite(p->lik_df),
+                "%s: the Student-t likelihood needs 0 < lik_df < inf (got %g)", who, p->lik_df);
+    PBX_REQUIRE(isfinite(p->lik_logc), "%s: lik_logc is not finite", who);
+    PBX_REQUIRE(p->variant != 3,
+                "%s: variant 3 (sufficient statistics) needs the normal likelihood", who);
+  }
   for (int j = 0; j < p->n_params; ++j) {
     PBX_REQUIRE(p->lims[j][1] > p->lims[j][0], "%s: empty prior box for parameter %d", who, j);
     PBX_REQUIRE(!p->log_ufun[j] || p->lims[j][0] > 0.0,
@@ -681,14 +723,16 @@ static bool nr_extras(const NrArgs& a, const NrModel& m) {
   return m.bound != 0 || m.has_L != 0 || a.out_xprop != nullptr || a.out_pprop != nullptr;
 }
 
-template <int KC>
-static int nr_launch_tiles(pbx_ctx* ctx, const NrPlan& pl, const NrArgs& a, const NrModel& m) {
+template <int KC, int kLik>
+static int nr_launch_tiles(pbx_ctx* ctx, const NrPlan& pl, const NrArgs& a, const NrModel& m,
+                           const NrLik& lik) {
   dim3 grid(pl.n_slices, pl.n_groups);
 #define NR_TILES_GO(S, E)                                                                      \
   do {                                                                                         \
-    PBX_CUDA(cudaFuncSetAttribute(nr_tiles_kernel<KC, S, E>,                                   \
+    PBX_CUDA(cudaFuncSetAttribute(nr_tiles_kernel<KC, S, E, kLik>,                             \
                                   cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl.smem)); \
-    nr_tiles_kernel<KC, S, E><<<grid, NR_THREADS, pl.smem, ctx->stream>>>(a, m, pl.use_tma);   \
+    nr_tiles_kernel<KC, S, E, kLik><<<grid, NR_THREADS, pl.smem, ctx->stream>>>(a, m,          \
+                                                                               pl.use_tma, lik); \
   } while (0)
   const bool ex = nr_extras(a, m);
   if (m.has_slope && ex) NR_TILES_GO(true, true);
@@ -700,14 +744,15 @@ static int nr_launch_tiles(pbx_ctx* ctx, const NrPlan& pl, const NrArgs& a, cons
   return PBX_OK;
 }
 
-template <int KS>
-static int nr_launch_stream(pbx_ctx* ctx, const NrPlan& pl, const NrArgs& a, const NrModel& m) {
+template <int KS, int kLik>
+static int nr_launch_stream(pbx_ctx* ctx, const NrPlan& pl, const NrArgs& a, const NrModel& m,
+                            const NrLik& lik) {
 #define NR_STREAM_GO(S, E)                                                                     \
   do {                                                                                         \
-    PBX_CUDA(cudaFuncSetAttribute(nr_stream_kernel<KS, S, E>,                                  \
+    PBX_CUDA(cudaFuncSetAttribute(nr_stream_kernel<KS, S, E, kLik>,                            \
                                   cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl.smem)); \
-    nr_stream_kernel<KS, S, E><<<pl.n_slices, NRS_THREADS, pl.smem, ctx->stream>>>(a, m,       \
-                                                                                  pl.use_tma); \
+    nr_stream_kernel<KS, S, E, kLik><<<pl.n_slices, NRS_THREADS, pl.smem, ctx->stream>>>(      \
+        a, m, pl.use_tma, lik);                                                                \
   } while (0)
   const bool ex = nr_extras(a, m);
   if (m.has_slope && ex) NR_STREAM_GO(true, true);
@@ -719,20 +764,29 @@ static int nr_launch_stream(pbx_ctx* ctx, const NrPlan& pl, const NrArgs& a, con
   return PBX_OK;
 }
 
-static int nr_launch_step(pbx_ctx* ctx, const NrPlan& pl, const NrArgs& a, const NrModel& m) {
+template <int kLik>
+static int nr_launch_step_lik(pbx_ctx* ctx, const NrPlan& pl, const NrArgs& a, const NrModel& m,
+                              const NrLik& lik) {
   if (pl.variant == 1) {
     switch (pl.kc) {
-      case 4: return nr_launch_tiles<4>(ctx, pl, a, m);
-      case 2: return nr_launch_tiles<2>(ctx, pl, a, m);
-      default: return nr_launch_tiles<1>(ctx, pl, a, m);
+      case 4: return nr_launch_tiles<4, kLik>(ctx, pl, a, m, lik);
+      case 2: return nr_launch_tiles<2, kLik>(ctx, pl, a, m, lik);
+      default: return nr_launch_tiles<1, kLik>(ctx, pl, a, m, lik);
     }
   }
   switch (pl.kc) {
-    case 1: return nr_launch_stream<1>(ctx, pl, a, m);
-    case 2: return nr_launch_stream<2>(ctx, pl, a, m);
-    case 4: return nr_launch_stream<4>(ctx, pl, a, m);
-    default: return nr_launch_stream<8>(ctx, pl, a, m);
+    case 1: return nr_launch_stream<1, kLik>(ctx, pl, a, m, lik);
+    case 2: return nr_launch_stream<2, kLik>(ctx, pl, a, m, lik);
+    case 4: return nr_launch_stream<4, kLik>(ctx, pl, a, m, lik);
+    default: return nr_launch_stream<8, kLik>(ctx, pl, a, m, lik);
   }
+}
+
+static int nr_launch_step(pbx_ctx* ctx, const NrPlan& pl, const NrArgs& a, const NrModel& m,
+                          int lik_kind, const NrLik& lik) {
+  return lik_kind == PBX_LIK_STUDENT_T
+             ? nr_launch_step_lik<PBX_LIK_STUDENT_T>(ctx, pl, a, m, lik)
+             : nr_launch_step_lik<PBX_LIK_NORMAL>(ctx, pl, a, m, lik);
 }
 
 // ============================================================================
@@ -913,9 +967,9 @@ __global__ void __launch_bounds__(128) ss_walk_kernel(const NrArgs a, const __gr
 #define RW_WARPS 4
 #define RW_MAXN 8192
 // kColour: as nr_draw_delta's (the colouring costs this kernel registers)
-template <bool kSlope, bool kColour>
+template <bool kSlope, bool kColour, int kLik>
 __global__ void __launch_bounds__(32 * RW_WARPS)
-    rw_walk_kernel(const NrArgs a, const __grid_constant__ NrModel m) {
+    rw_walk_kernel(const NrArgs a, const __grid_constant__ NrModel m, const NrLik lik) {
   extern __shared__ __align__(16) double rw_sm[];       // y[N], then x[N] (kSlope)
   double* sy = rw_sm;
   double* sx = rw_sm + a.N;
@@ -942,7 +996,10 @@ __global__ void __launch_bounds__(32 * RW_WARPS)
     double s0 = 0.0, s1 = 0.0, s2 = 0.0, s3 = 0.0;
     auto term = [&](int i) {
       const double r = kSlope ? (sy[i] - b0) - b1 * sx[i] : sy[i] - b0;
-      return r * r;
+      // if constexpr: the normal instantiation captures no more than the normal-only kernel
+      // did, which keeps its SASS byte-identical (a runtime-dead capture reorders registers)
+      if constexpr (kLik == PBX_LIK_STUDENT_T) return log1p((r * r) * nr_q<kLik>(lik, t[P - 1]));
+      else return r * r;
     };
     int i = lane;
     for (; i + 96 < n; i += 128) {
@@ -982,7 +1039,7 @@ __global__ void __launch_bounds__(32 * RW_WARPS)
     const double t = __shfl_sync(0xffffffffu, tv, k & 31);
     const double logt = __shfl_sync(0xffffffffu, ltv, k & 31);
     _Pragma("unroll") for (int j = 0; j < P; ++j) thp[j] = nr_move<true>(m, j, th[j], dl[j]);
-    const double lpp = nr_logjoint<P>(a, m, thp, rss(thp));
+    const double lpp = nr_logjoint<P, kLik>(a, m, thp, rss(thp), lik);
     double s;
     const bool acc = nr_decide(m, lpp, lp, t, [&] { return logt; }, gstep,
                                a.out_score != nullptr, s);
@@ -1079,7 +1136,8 @@ static int nr_walk_suffstat(pbx_ctx* ctx, const NrArgs& a, const NrModel& m) {
   return PBX_OK;
 }
 
-static int nr_walk_small(pbx_ctx* ctx, const NrArgs& a, const NrModel& m) {
+template <int kLik>
+static int nr_walk_small(pbx_ctx* ctx, const NrArgs& a, const NrModel& m, const NrLik& lik) {
   const size_t smem = (size_t)a.N * 8 * (m.has_slope ? 2 : 1);
   // warps (chains) per CTA: up to RW_WARPS, fewer when there are few chains, so that they
   // spread over the SMs (every warp re-reads the resident observations each step: four
@@ -1089,9 +1147,9 @@ static int nr_walk_small(pbx_ctx* ctx, const NrArgs& a, const NrModel& m) {
   const int grid = (a.C + wpc - 1) / wpc;
 #define RW_GO(S, L)                                                                            \
   do {                                                                                         \
-    PBX_CUDA(cudaFuncSetAttribute(rw_walk_kernel<S, L>,                                        \
+    PBX_CUDA(cudaFuncSetAttribute(rw_walk_kernel<S, L, kLik>,                                  \
                                   cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));    \
-    rw_walk_kernel<S, L><<<grid, 32 * wpc, smem, ctx->stream>>>(a, m);                         \
+    rw_walk_kernel<S, L, kLik><<<grid, 32 * wpc, smem, ctx->stream>>>(a, m, lik);              \
   } while (0)
   if (m.has_slope && m.has_L) RW_GO(true, true);
   else if (m.has_slope) RW_GO(true, false);
@@ -1102,14 +1160,15 @@ static int nr_walk_small(pbx_ctx* ctx, const NrArgs& a, const NrModel& m) {
   return PBX_OK;
 }
 
-static int nr_walk_per_step(pbx_ctx* ctx, const NrPlan& pl, NrArgs a, const NrModel& m) {
+static int nr_walk_per_step(pbx_ctx* ctx, const NrPlan& pl, NrArgs a, const NrModel& m,
+                            int lik_kind, const NrLik& lik) {
   if (nr_extras(a, m)) nr_init_kernel<true><<<(a.C + 255) / 256, 256, 0, ctx->stream>>>(a, m);
   else nr_init_kernel<false><<<(a.C + 255) / 256, 256, 0, ctx->stream>>>(a, m);
   PBX_LAUNCH_CHECK(ctx);
   for (int k = 0; k < a.T; ++k) {
     a.k = k;
     a.gstep = a.step0 + k;
-    int rc = nr_launch_step(ctx, pl, a, m);
+    int rc = nr_launch_step(ctx, pl, a, m, lik_kind, lik);
     if (rc) return rc;
   }
   return PBX_OK;
@@ -1123,6 +1182,8 @@ extern "C" int pbx_mh_normreg_run(pbx_ctx* ctx, const pbx_mh_normreg_params* p) 
   NrModel m;
   nr_fill_model(p, m);
   NrArgs a = nr_args(p);
+  const NrLik lik{p->lik_df, p->lik_logc};
+  const bool t_lik = p->lik_kind == PBX_LIK_STUDENT_T;
   // variant 3: sufficient statistics, else a small problem: the walk in one launch;
   // otherwise one launch per step
   const bool suffstat = p->variant == 3, small = !suffstat && rw_applies(p);
@@ -1138,8 +1199,11 @@ extern "C" int pbx_mh_normreg_run(pbx_ctx* ctx, const pbx_mh_normreg_params* p) 
   }
   PBX_CUDA(cudaEventRecord(ctx->ev0, ctx->stream));
   if (a.T > 0) {
-    rc = suffstat ? nr_walk_suffstat(ctx, a, m)
-                  : (small ? nr_walk_small(ctx, a, m) : nr_walk_per_step(ctx, pl, a, m));
+    if (suffstat) rc = nr_walk_suffstat(ctx, a, m);
+    else if (small)
+      rc = t_lik ? nr_walk_small<PBX_LIK_STUDENT_T>(ctx, a, m, lik)
+                 : nr_walk_small<PBX_LIK_NORMAL>(ctx, a, m, lik);
+    else rc = nr_walk_per_step(ctx, pl, a, m, p->lik_kind, lik);
     if (rc) return rc;
   }
   PBX_CUDA(cudaEventRecord(ctx->ev1, ctx->stream));
@@ -1175,7 +1239,7 @@ extern "C" int pbx_normreg_logjoint(pbx_ctx* ctx, const pbx_mh_normreg_params* p
   a.mode = 1;
   a.T = 1; a.thin = 1;
   PBX_CUDA(cudaEventRecord(ctx->ev0, ctx->stream));
-  rc = nr_launch_step(ctx, pl, a, m);
+  rc = nr_launch_step(ctx, pl, a, m, p->lik_kind, NrLik{p->lik_df, p->lik_logc});
   if (rc) return rc;
   PBX_CUDA(cudaEventRecord(ctx->ev1, ctx->stream));
   return PBX_OK;

@@ -115,18 +115,18 @@ def gather_slabs(local, counts, group=None):
     return torch.cat([p[:c] for p, c in zip(parts, counts)])
 
 
-def dgei_sharded(engine, x_obs, mu, sigma, logprior_mu, logprior_sigma, group=None):
+def dgei_sharded(engine, x_obs, mu, sigma, logprior_mu, logprior_sigma, group=None, lik=None):
     """Slab-sharded discrete grid exact inference: every rank evaluates the
     log-joint of its mu rows, the ranks agree on the normaliser, and each returns
     dict(post=[M_local, S] slab, marg_mu=[M] (gathered), marg_sigma=[S], rows=(start,
-    count)).  All inputs are full-size host arrays."""
+    count)).  All inputs are full-size host arrays; ``lik`` as Engine.mh_normreg's."""
     rank, ws = world()
     M = len(mu)
     start, count = shard_range(M, rank, ws)
     sl = slice(start, start + count)
     lj = engine.grid_norm_logjoint(engine.to_device(x_obs), engine.to_device(mu[sl]),
                                    engine.to_device(sigma), engine.to_device(logprior_mu[sl]),
-                                   engine.to_device(logprior_sigma))
+                                   engine.to_device(logprior_sigma), lik=lik)
     dist = _sharded(group)
     if dist is not None and group is None:
         group = dist.group.WORLD
@@ -151,18 +151,19 @@ def allreduce_expectation(sums, group=None):
 
 
 def omc_sharded(engine, y_obs, lims, open_end, log_ufun, n_samples, seed=0, x_obs=None,
-                group=None):
+                group=None, lik=None):
     """Sample-sharded ordinary Monte Carlo random sampling of a normal-likelihood
     posterior: rank r draws samples [start, start + count) of the global Philox stream,
     evaluates their log-joint, the ranks agree on the normaliser, and the posterior
     means of the parameters are all-reduced.  Returns dict(theta [P, count], logpost
-    [count] (normalised over ALL ranks), expectation [P], samples=(start, count))."""
+    [count] (normalised over ALL ranks), expectation [P], samples=(start, count)).  ``lik``
+    as Engine.mh_normreg's."""
     rank, ws = world()
     start, count = shard_range(n_samples, rank, ws)
     theta = engine.box_sample(lims, log_ufun, count, seed=seed, sample0=start)
     y = engine.to_device(np.ravel(np.asarray(y_obs, dtype=np.float64)))
     x = None if x_obs is None else engine.to_device(np.ravel(np.asarray(x_obs, np.float64)))
-    logp = engine.normreg_logjoint(theta, y, x, lims, open_end, log_ufun)
+    logp = engine.normreg_logjoint(theta, y, x, lims, open_end, log_ufun, lik=lik)
     ms = engine.grid_max_sumexp(logp)
     gmax, gsum = allreduce_max_sumexp(ms[0:1], ms[1:2], engine.grid_rescale_sumexp_,
                                       group=group)

@@ -339,7 +339,7 @@ class Engine:
     # ------------------------------------------------- K2: streaming normal MH
     def _normreg_params(self, C_, P, x_obs, y_obs, lims, open_end, log_ufun, prop_scale,
                         accept="log", accept_coef=1.0, prop="uniform", variant=0,
-                        prop_radius=0.0, prop_bound=False, prop_chol=None):
+                        prop_radius=0.0, prop_bound=False, prop_chol=None, lik=None):
         if P not in (2, 3):
             raise NotImplementedError("normal-likelihood MH supports (mu, sigma) or "
                                       "(b0, b1, sigma) parameters, got %d" % P)
@@ -376,18 +376,23 @@ class Engine:
             p.has_prop_mat = 1
             for i, v in enumerate(L.ravel()):
                 p.prop_mat[i] = v
+        if lik is not None:
+            p.lik_kind = _lib.LIK_STUDENT_T
+            p.lik_df, p.lik_logc = float(lik["df"]), float(lik["logc"])
         return p
 
     def mh_normreg(self, state, y_obs, x_obs, steps, lims, open_end, log_ufun, prop_scale,
                    thin=1, seed=0, step0=0, chain0=0, accept="log", accept_coef=1.0,
                    prop="uniform", variant=0, inj_delta=None, inj_thresh=None, state_lp=None,
                    record=True, per_step=False, stats=True, prop_radius=0.0,
-                   prop_bound=False, prop_chol=None):
+                   prop_bound=False, prop_chol=None, lik=None):
         """MH on the iid-normal posterior; ``state`` [P, C] device fp64 (in place),
         ``y_obs``/``x_obs`` device fp64 [N].  Same outputs as :meth:`mh_mvn`; the
         recorded ``prob`` is the log-joint (log pscale).  ``prop_chol`` [P, P]: the
         lower-triangular factor every delta is multiplied by before the ufun move
-        (set_tran(covariance), rf.py:346-348), injected deltas included."""
+        (set_tran(covariance), rf.py:346-348), injected deltas included.  ``lik``: the
+        likelihood family, None (normal) or a Student-t dict(df=nu, logc=...) as
+        ``catalogue.likelihood`` returns; the t has no sufficient statistics (no variant 3)."""
         torch = _torch()
         P, C_ = state.shape
         T = int(steps)
@@ -401,7 +406,7 @@ class Engine:
         self._dev(inj_thresh, (T, C_), "inj_thresh")
         p = self._normreg_params(C_, P, x_obs, y_obs, lims, open_end, log_ufun, prop_scale,
                                  accept, accept_coef, prop, variant, prop_radius, prop_bound,
-                                 prop_chol)
+                                 prop_chol, lik)
         p.n_steps, p.thin, p.step0, p.chain0 = T, thin, step0, chain0
         p.seed = seed & 0xFFFFFFFFFFFFFFFF
         if state_lp is None:
@@ -415,14 +420,16 @@ class Engine:
         _lib.check(self.lib.pbx_mh_normreg_run(self.ctx, C.byref(p)), "pbx_mh_normreg_run")
         return out
 
-    def normreg_logjoint(self, theta, y_obs, x_obs, lims, open_end, log_ufun, variant=0):
-        """log-joint (likelihood + box priors) of theta [P, C] -> [C] device."""
+    def normreg_logjoint(self, theta, y_obs, x_obs, lims, open_end, log_ufun, variant=0,
+                         lik=None):
+        """log-joint (likelihood + box priors) of theta [P, C] -> [C] device; ``lik`` as
+        :meth:`mh_normreg`'s."""
         P, C_ = theta.shape
         self._dev(theta, (P, C_), "theta")
         self._dev(y_obs, None, "y_obs")
         self._dev(x_obs, None, "x_obs")
         p = self._normreg_params(C_, P, x_obs, y_obs, lims, open_end, log_ufun, 0.0,
-                                 variant=variant)
+                                 variant=variant, lik=lik)
         out = self.empty(C_)
         _lib.check(self.lib.pbx_normreg_logjoint(self.ctx, C.byref(p), self._ptr(theta),
                                                  self._ptr(out)), "pbx_normreg_logjoint")
@@ -430,13 +437,23 @@ class Engine:
 
     # ------------------------------------------------------ K3/K4: grid (DGEI)
     def grid_norm_logjoint(self, x_obs, mu, sigma, logprior_mu, logprior_sigma, out=None,
-                           suffstat=False):
+                           suffstat=False, lik=None):
         """log-joint [M, S] = priors + sum_i norm.logpdf(x_i; mu_m, sigma_s); all
         arguments device fp64 vectors.  ``suffstat=True`` (opt-in) evaluates it from
-        centred sufficient statistics of the observations: O(M S) instead of O(N M S)."""
+        centred sufficient statistics of the observations: O(M S) instead of O(N M S).
+        ``lik``: as :meth:`mh_normreg`'s; a Student-t sums t.logpdf and has no suffstat."""
         M, S = int(mu.numel()), int(sigma.numel())
-        fn, what = (self.lib.pbx_grid_norm_logjoint_ss, "pbx_grid_norm_logjoint_ss") \
-            if suffstat else (self.lib.pbx_grid_norm_logjoint, "pbx_grid_norm_logjoint")
+        extra = ()
+        if lik is not None:
+            if suffstat:
+                raise ValueError("suffstat=True needs the normal likelihood: the Student-t "
+                                 "likelihood has no sufficient statistics")
+            fn, what = self.lib.pbx_grid_t_logjoint, "pbx_grid_t_logjoint"
+            extra = (float(lik["df"]), float(lik["logc"]))
+        elif suffstat:
+            fn, what = self.lib.pbx_grid_norm_logjoint_ss, "pbx_grid_norm_logjoint_ss"
+        else:
+            fn, what = self.lib.pbx_grid_norm_logjoint, "pbx_grid_norm_logjoint"
         if out is None:
             out = self.empty(M, S)
         row_cap = 65535
@@ -445,7 +462,7 @@ class Engine:
             _lib.check(fn(
                 self.ctx, self._ptr(x_obs), int(x_obs.numel()), self._ptr(mu[m0:m1]), m1 - m0,
                 self._ptr(sigma), S, self._ptr(logprior_mu[m0:m1]), self._ptr(logprior_sigma),
-                self._ptr(out[m0:m1])), what)
+                self._ptr(out[m0:m1]), *extra), what)
         return out
 
     def log_prob_(self, v):

@@ -169,11 +169,12 @@ class SD:
         values = self.parse_values(values)
         spec = catalogue.identify_target(self, self._leafs, self._roots)
         if spec['kind'] != 'normreg' or spec['has_slope']:
-            raise NotImplementedError("grid evaluation is in the catalogue for the iid normal "
-                                      "(mu, sigma) likelihood only")
+            raise NotImplementedError("grid evaluation is in the catalogue for the iid normal, "
+                                      "Student-t or Cauchy (mu, sigma) likelihood only")
         if not iid:
             raise NotImplementedError("the un-reduced [N, M, S] likelihood tensor is never "
                                       "materialised on the device: call with iid=True")
+        catalogue.refuse_suffstat(spec, 3 if suffstat else 0)
         obs, (kmu, ksg) = spec['obs_y'], spec['params']
         data = np.ascontiguousarray(np.ravel(np.asarray(values[obs], dtype=np.float64)))
         grids = {}
@@ -194,7 +195,7 @@ class SD:
         eng = get_engine()
         lj = eng.grid_norm_logjoint(eng.to_device(data), eng.to_device(grids[kmu]),
                                     eng.to_device(grids[ksg]), eng.to_device(lpm),
-                                    eng.to_device(lps), suffstat=suffstat)
+                                    eng.to_device(lps), suffstat=suffstat, lik=spec.get('lik'))
         order = [k for k in self._roots.keylist if k in (kmu, ksg)]
         vals = collections.OrderedDict()
         dims = collections.OrderedDict()

@@ -402,8 +402,10 @@ class SP(SD):
         if seed is None:
             seed = int(np.random.randint(0, 2 ** 31 - 1))
         theta = eng.box_sample(lims, lg, T, seed=seed, sample0=sampler.counter, inj_unif=inj)
+        catalogue.refuse_suffstat(spec, opts['variant'])
         logp = eng.normreg_logjoint(theta, y, x, lims, ex, lg,
-                                    variant=3 if opts['variant'] == 3 else 0)
+                                    variant=3 if opts['variant'] == 3 else 0,
+                                    lik=spec.get('lik'))
         return dict(omc=True, keys=keys, T=T, spec=spec, theta=theta, logp=logp,
                     n_obs=int(y.numel()), pscale=self._pscale, chains=None)
 
@@ -557,6 +559,7 @@ class SP(SD):
         else:
             if not opts['iid']:
                 raise NotImplementedError("the normal-likelihood target needs iid=True")
+            catalogue.refuse_suffstat(spec, opts['variant'])
             if sampler.obs is None or spec['obs_y'] not in sampler.obs:
                 raise ValueError("observations for '{}' are required".format(spec['obs_y']))
             assert spec['params'] == keys, \
@@ -582,7 +585,7 @@ class SP(SD):
                                  prop_bound=prop['bound'], prop_chol=prop['chol'],
                                  inj_delta=inj_d, inj_thresh=inj_t,
                                  state_lp=sampler.state_lp, per_step=per_step,
-                                 variant=opts['variant'], chain0=chain0)
+                                 variant=opts['variant'], chain0=chain0, lik=spec.get('lik'))
             res['n_obs'] = int(y.numel())
         sampler.state_lp = out['state_lp']
         res.update(x=out['x'], prob=out['prob'], accept_count=out['accept_count'],
