@@ -65,6 +65,8 @@ typedef enum {
 /* iid likelihood family of K2 / K3 (pbx_mh_normreg_params.lik_kind) */
 #define PBX_LIK_NORMAL 0           /* scipy.stats.norm.logpdf */
 #define PBX_LIK_STUDENT_T 1        /* scipy.stats.t.logpdf (cauchy.logpdf: df = 1) */
+#define PBX_LIK_STUDENT_T_NU 2     /* scipy.stats.t.logpdf with df = nu a model parameter:
+                                      params (mu, sigma, nu) */
 
 typedef struct pbx_ctx pbx_ctx;
 
@@ -169,6 +171,7 @@ PBX_API int pbx_mh_mvn_walk_host(pbx_ctx* ctx, const pbx_mh_mvn_params* p, int32
  * K2  streaming normal log-likelihood MH (iid=True, joint=True, log pscale).
  *   y_i ~ N(b0 + b1 x_i, sigma)   params (b0, b1, sigma)   has_slope = 1
  *   y_i ~ N(mu, sigma)            params (mu, sigma)       has_slope = 0
+ *   y_i ~ t_nu(mu, sigma)         params (mu, sigma, nu)   has_slope = 0  (PBX_LIK_STUDENT_T_NU)
  * Replaces RF.__call__(iid=True) + SD.__call__(joint=True) evaluated every step
  * (probayes/rf.py:541-581, pd.py:332-370, sd.py:148-161) with scipy.stats.norm
  * .logpdf as the likelihood (examples/mcmc/metrohast_norm1d.py:30-31,
@@ -178,7 +181,7 @@ PBX_API int pbx_mh_mvn_walk_host(pbx_ctx* ctx, const pbx_mh_mvn_params* p, int32
  * ------------------------------------------------------------------------- */
 typedef struct {
   int32_t n_chains;
-  int32_t n_params;        /* 2 or 3 */
+  int32_t n_params;        /* 2 or 3 (3: has_slope, or PBX_LIK_STUDENT_T_NU) */
   int32_t n_steps;
   int32_t thin;
   int64_t step0;
@@ -238,7 +241,13 @@ typedef struct {
    * where the caller computes lik_logc = log(poch(df/2, 1/2)) - (log df + log pi)/2 as scipy
    * does (lgamma((df+1)/2) - lgamma(df/2) cancels: 9e-7 relative at df = 1e9).  Student-t needs
    * 0 < lik_df < inf and a finite lik_logc, and refuses variant 3 (the t likelihood has no
-   * sufficient statistics); both entry points return PBX_ERR_INVALID otherwise. */
+   * sufficient statistics); both entry points return PBX_ERR_INVALID otherwise.
+   * PBX_LIK_STUDENT_T_NU is the same density with df = nu sampled as the model's third
+   * parameter, theta = (mu, sigma, nu): n_params = 3, has_slope = 0, lik_df = lik_logc = 0
+   * (unread: the kernels compute logc(nu) of every chain and step, as
+   * lgamma((nu+1)/2) - lgamma(nu/2) - log(nu pi)/2 below nu = 16 and an asymptotic series
+   * above, which does not cancel), nu's prior box admitting nu > 0 only (lims[2][0] > 0, or
+   * lims[2][0] = 0 with an open lower end), and no variant 3. */
   int32_t lik_kind;        /* PBX_LIK_* */
   int32_t reserved1;
   double lik_df;

@@ -11,7 +11,7 @@ PBX_MAX_DIMS = 8
 PBX_MAX_PARAMS = 3
 ACCEPT_REFERENCE, ACCEPT_LOG = 0, 1
 PROP_NORMAL, PROP_UNIFORM, PROP_SPHERICAL = 0, 1, 2
-LIK_NORMAL, LIK_STUDENT_T = 0, 1
+LIK_NORMAL, LIK_STUDENT_T, LIK_STUDENT_T_NU = 0, 1, 2
 
 c_double_p = C.POINTER(C.c_double)
 

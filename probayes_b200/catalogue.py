@@ -11,7 +11,8 @@ Targets
   norm     scipy.stats.norm.logpdf + order={'x': 0, 'mu': 'loc', 'sigma': 'scale'}
            with iid=True                                      (metrohast_norm1d, dgei_*)
            -- or scipy.stats.t.logpdf with df=nu, or scipy.stats.cauchy.logpdf, in the
-           same call: the spec's ``lik`` entry names the family
+           same call: the spec's ``lik`` entry names the family; or t.logpdf with order
+           mapping a parameter RV nu to 1 or 'df': nu is sampled, params (loc, scale, nu)
   normreg  a Python callable that IS norm.logpdf(y, loc=b0 + b1*x, scale=s) -- verified
            numerically by probing it against every role assignment (gibbs_linreg's
            ``norm_reg``), or an explicit ``NormalRegression`` / ``StudentTRegression`` spec
@@ -76,6 +77,37 @@ def likelihood(family, df=None):
     if not df > 0:
         raise ValueError("df must be positive (and not NaN), got {!r}".format(df))
     return dict(family='t', df=df, logc=t_logc(df))
+
+
+def _df_role(order, family, kwds, stats, paras):
+    """The parameter RV an order of t.logpdf maps to df (positional 1 or 'df'), or None.  Only
+    t.logpdf takes a df; for the normal, whose catalogue entry predates this, a role 1 stays
+    unread as before."""
+    names = [k for k, v in order.items() if isinstance(v, (int, str)) and not isinstance(v, bool)
+             and v in (1, 'df')]
+    if not names or family == 'norm':
+        return None
+    if family == 'cauchy':
+        raise NotImplementedError("scipy.stats.cauchy.logpdf has no degrees of freedom: use "
+                                  "scipy.stats.t.logpdf to sample nu (order maps {!r} to {!r})"
+                                  .format(names[0], order[names[0]]))
+    if len(names) > 1:
+        raise NotImplementedError("order maps more than one RV to the degrees of freedom: "
+                                  "{}".format(names))
+    nu = names[0]
+    if 'df' in (kwds or {}):
+        raise ValueError("the degrees of freedom are given twice: by df= and by order "
+                         "({!r} -> {!r}); drop one".format(nu, order[nu]))
+    if paras is None or nu not in paras.keyset:
+        where = "a stats (observation) RV" if nu in stats.keyset else "not a parameter RV"
+        raise NotImplementedError("order maps {!r} to the degrees of freedom, but {!r} is {}: a "
+                                  "sampled nu must be a parameter RV".format(nu, nu, where))
+    lo, (lo_open, _) = float(paras[nu].vlims[0]), paras[nu].open_ends
+    if not (lo > 0 or (lo == 0 and lo_open)):
+        raise ValueError("the prior box of the degrees of freedom {!r} must admit nu > 0 only: "
+                         "its lower end is {} ({}); use vset=[a, b] with a > 0, or (0, b)"
+                         .format(nu, lo, "open" if lo_open else "closed"))
+    return nu
 
 
 def _with_lik(spec, lik):
@@ -159,6 +191,12 @@ def identify_target(holder, stats, paras):
         if paras is None or obs not in stats.keyset or {loc, scale} - paras.keyset:
             raise NotImplementedError("order must map a stats RV to 0 and parameter RVs "
                                       "to 'loc'/'scale'")
+        nu = _df_role(order, family, kwds, stats, paras)
+        if nu is not None:
+            # theta = (loc, scale, nu): the parameter order of the kernels' sampled-nu t
+            return dict(kind='normreg', has_slope=False, obs_y=obs, obs_x=None,
+                        params=[loc, scale, nu], log_pscale=True,
+                        lik=dict(family='t', df_param=nu))
         return _with_lik(dict(kind='normreg', has_slope=False, obs_y=obs, obs_x=None,
                               params=[loc, scale], log_pscale=True),
                          likelihood(family, (kwds or {}).get('df')))

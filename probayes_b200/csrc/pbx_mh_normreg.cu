@@ -4,7 +4,9 @@
 //   log p(theta, data) = sum_j boxprior_j(theta_j) + sum_i lik.logpdf(y_i; loc_i, sigma)
 //   loc_i = b0 + b1 x_i (has_slope, theta = (b0, b1, sigma)) or mu (theta = (mu, sigma))
 //   lik = norm, or t with nu degrees of freedom (kLik; cauchy = t with nu = 1), whose sum is
-//   N logc - N log sigma - (nu+1)/2 sum_i log1p(r_i^2 / (nu sigma^2)), logc from the host
+//   N logc - N log sigma - (nu+1)/2 sum_i log1p(r_i^2 / (nu sigma^2)), logc from the host;
+//   or that t with nu sampled (PBX_LIK_STUDENT_T_NU, theta = (mu, sigma, nu)), logc(nu) on
+//   the device (nr_t_logc)
 // following probayes/rf.py:541-581, pd.py:332-370 (iid product = sum over the
 // observation axis), sd.py:154-161 + rf_utils.py:10-22 + rv_utils.py:8-47 (product
 // with the independent box priors, prior first), scipy.stats.norm.logpdf per term,
@@ -49,7 +51,8 @@ struct NrModel {
   double L[PBX_MAX_PARAMS][PBX_MAX_PARAMS];   // lower-triangular, zero outside [P][P]
 };
 
-// the Student-t likelihood of a call (PBX_LIK_STUDENT_T; unread by the normal instantiations).
+// the Student-t likelihood of a call (PBX_LIK_STUDENT_T; unread by the normal and the
+// sampled-nu instantiations).
 // A kernel argument of its own, after the others, so that the normal kernels' argument
 // offsets -- and with them their SASS -- are those of the normal-only build
 struct NrLik {
@@ -253,17 +256,50 @@ __device__ __forceinline__ void nr_propose(const NrArgs& a, const NrModel& m, in
 }
 
 // one observation's term of the likelihood sum, residual r: r^2 (normal), or
-// log1p(r^2 q) with q = 1/(nu sigma^2) (Student-t)
+// log1p(r^2 q) with q = 1/(nu sigma^2) (Student-t, nu fixed or sampled)
 template <int kLik>
 __device__ __forceinline__ double nr_term(double acc, double r, double q) {
-  if (kLik == PBX_LIK_STUDENT_T) return acc + log1p((r * r) * q);
+  if (kLik != PBX_LIK_NORMAL) return acc + log1p((r * r) * q);
   return fma(r, r, acc);
 }
 
-// q of nr_term for scale sg
-template <int kLik>
-__device__ __forceinline__ double nr_q(const NrLik& lik, double sg) {
-  return kLik == PBX_LIK_STUDENT_T ? 1.0 / (lik.df * (sg * sg)) : 0.0;
+// q of nr_term for scale sg and nu degrees of freedom
+__device__ __forceinline__ double nr_q(double sg, double nu) { return 1.0 / (nu * (sg * sg)); }
+
+// theta index of sigma: the last parameter, but for the sampled-nu t's (mu, sigma, nu)
+template <int kLik, bool kSlope>
+constexpr int nr_isg() { return kLik == PBX_LIK_STUDENT_T_NU ? 1 : (kSlope ? 2 : 1); }
+
+// logc(nu) = lgamma((nu+1)/2) - lgamma(nu/2) - log(nu pi)/2, the per-observation constant of
+// the t density, for a sampled nu, as R(z) - log sqrt(2 pi) with z = nu/2 and
+// R(z) = lgamma(z + 1/2) - lgamma(z) - log(z)/2.  Below z = 8 the lgamma difference (both
+// terms < 10 there); from z = 8 on the asymptotic series R(z) = sum_k c_k z^-k over odd k,
+// c_k = -(2 - 2^-k) B_{k+1} / (k (k+1)) (B: Bernoulli), up to k = 17 (the first term left out
+// is < 2e-17 at z = 8).  The series never cancels, where the lgamma difference would at large nu
+// (which is why the host's t_logc uses poch), and R -> -1/(8z) -> 0 gives the normal's constant
+// as nu -> inf.  Within 1.2e-15 absolute of mpmath over nu in [1e-3, 1e12], measured on a B200
+// (tests/test_gpu_studentt_nu.py).  nu <= 0 gives NaN, as scipy's t.logpdf does.
+// Once per chain and step.  __noinline__: inlined, the lgamma calls kept the epilogue's state
+// live across libm's subroutine calls and spilled it in the tiles and stream kernels.
+__device__ __noinline__ double nr_t_logc(double nu) {
+  const double z = 0.5 * nu;
+  double R;
+  if (z < 8.0) {
+    R = lgamma(z + 0.5) - lgamma(z) - 0.5 * log(z);
+  } else {
+    const double w = 1.0 / (z * z);
+    double s = -3202291.0 / 8912896.0;                    // c_17
+    s = fma(s, w, 929569.0 / 15728640.0);                 // c_15
+    s = fma(s, w, -5461.0 / 425984.0);                    // c_13
+    s = fma(s, w, 691.0 / 180224.0);                      // c_11
+    s = fma(s, w, -31.0 / 18432.0);                       // c_9
+    s = fma(s, w, 17.0 / 14336.0);                        // c_7
+    s = fma(s, w, -1.0 / 640.0);                          // c_5
+    s = fma(s, w, 1.0 / 192.0);                           // c_3
+    s = fma(s, w, -0.125);                                // c_1
+    R = s / z;
+  }
+  return R - PBX_LOG_SQRT_2PI;
 }
 
 // log-joint from the likelihood sum S (see file header; for Student-t S = sum log1p(z^2/nu))
@@ -271,10 +307,13 @@ template <int kP = 0, int kLik = PBX_LIK_NORMAL>
 __device__ __forceinline__ double nr_logjoint(const NrArgs& a, const NrModel& m, const double* th,
                                               double S, const NrLik& lik = NrLik{}) {
   const int P = kP ? kP : m.P;
-  const double sg = th[P - 1];
+  const double sg = kLik == PBX_LIK_STUDENT_T_NU ? th[1] : th[P - 1];
   const double n = (double)a.N;
   double ll;
-  if (kLik == PBX_LIK_STUDENT_T)
+  if constexpr (kLik == PBX_LIK_STUDENT_T_NU) {
+    const double nu = th[2];
+    ll = -(0.5 * (nu + 1.0)) * S + n * (nr_t_logc(nu) - log(sg));
+  } else if (kLik == PBX_LIK_STUDENT_T)
     ll = -(0.5 * (lik.df + 1.0)) * S + n * (lik.logc - log(sg));
   else
     ll = -(S / (sg * sg)) * 0.5 - n * (PBX_LOG_SQRT_2PI + log(sg));
@@ -372,7 +411,10 @@ __global__ void __launch_bounds__(NR_THREADS)
     const bool v = c < a.C;
     b0[k] = v ? a.theta_in[c] : 0.0;
     b1[k] = (v && kSlope) ? a.theta_in[C + c] : 0.0;
-    q[k] = (kLik && v) ? nr_q<kLik>(lik, a.theta_in[(kSlope ? 2 : 1) * C + c]) : 0.0;
+    if constexpr (kLik == PBX_LIK_STUDENT_T_NU)
+      q[k] = v ? nr_q(a.theta_in[C + c], a.theta_in[2 * C + c]) : 0.0;
+    else
+      q[k] = (kLik && v) ? nr_q(a.theta_in[nr_isg<kLik, kSlope>() * C + c], lik.df) : 0.0;
     acc[k] = 0.0;
   }
 
@@ -505,8 +547,12 @@ __global__ void __launch_bounds__(NRS_THREADS)
   for (int k = 0; k < KS; ++k) {
     b0[k] = (k < a.C) ? a.theta_in[k] : 0.0;
     b1[k] = (k < a.C && kSlope) ? a.theta_in[(int64_t)a.C + k] : 0.0;
-    q[k] = (kLik && k < a.C) ? nr_q<kLik>(lik, a.theta_in[(int64_t)(kSlope ? 2 : 1) * a.C + k])
-                             : 0.0;
+    if constexpr (kLik == PBX_LIK_STUDENT_T_NU)
+      q[k] = k < a.C ? nr_q(a.theta_in[(int64_t)a.C + k], a.theta_in[2 * (int64_t)a.C + k]) : 0.0;
+    else
+      q[k] = (kLik && k < a.C)
+                 ? nr_q(a.theta_in[(int64_t)nr_isg<kLik, kSlope>() * a.C + k], lik.df)
+                 : 0.0;
     acc[k] = 0.0;
   }
   const int64_t n_full = a.N / NRS_TILE;
@@ -647,8 +693,22 @@ static int nr_validate(const pbx_mh_normreg_params* p, const char* who, bool nee
   PBX_REQUIRE(p != nullptr, "%s: null params", who);
   PBX_REQUIRE(p->n_chains >= 1, "%s: n_chains must be >= 1", who);
   PBX_REQUIRE(p->n_params == 2 || p->n_params == 3, "%s: n_params must be 2 or 3", who);
-  PBX_REQUIRE((p->has_slope != 0) == (p->n_params == 3),
-              "%s: has_slope needs 3 params (b0, b1, sigma), otherwise 2 (mu, sigma)", who);
+  PBX_REQUIRE(p->lik_kind == PBX_LIK_NORMAL || p->lik_kind == PBX_LIK_STUDENT_T ||
+                  p->lik_kind == PBX_LIK_STUDENT_T_NU,
+              "%s: unknown lik_kind %d", who, p->lik_kind);
+  if (p->lik_kind == PBX_LIK_STUDENT_T_NU) {
+    PBX_REQUIRE(p->n_params == 3 && p->has_slope == 0,
+                "%s: the sampled-nu Student-t needs 3 params (mu, sigma, nu) and no slope", who);
+    PBX_REQUIRE(p->lik_df == 0.0 && p->lik_logc == 0.0,
+                "%s: the sampled-nu Student-t reads nu from theta: lik_df and lik_logc must be 0",
+                who);
+    PBX_REQUIRE(p->lims[2][0] > 0.0 || (p->lims[2][0] == 0.0 && p->open_end[2][0]),
+                "%s: nu's prior box must admit nu > 0 only (got lower limit %g, %s)", who,
+                p->lims[2][0], p->open_end[2][0] ? "open" : "closed");
+  } else {
+    PBX_REQUIRE((p->has_slope != 0) == (p->n_params == 3),
+                "%s: has_slope needs 3 params (b0, b1, sigma), otherwise 2 (mu, sigma)", who);
+  }
   PBX_REQUIRE(p->n_obs >= 1, "%s: n_obs must be >= 1", who);
   PBX_REQUIRE(p->y_obs != nullptr && (!p->has_slope || p->x_obs != nullptr),
               "%s: observation arrays missing", who);
@@ -656,15 +716,13 @@ static int nr_validate(const pbx_mh_normreg_params* p, const char* who, bool nee
               "%s: unknown accept_mode", who);
   PBX_REQUIRE(p->prop_kind >= PBX_PROP_NORMAL && p->prop_kind <= PBX_PROP_SPHERICAL,
               "%s: unknown prop_kind", who);
-  PBX_REQUIRE(p->lik_kind == PBX_LIK_NORMAL || p->lik_kind == PBX_LIK_STUDENT_T,
-              "%s: unknown lik_kind %d", who, p->lik_kind);
   if (p->lik_kind == PBX_LIK_STUDENT_T) {
     PBX_REQUIRE(p->lik_df > 0.0 && isfinite(p->lik_df),
                 "%s: the Student-t likelihood needs 0 < lik_df < inf (got %g)", who, p->lik_df);
     PBX_REQUIRE(isfinite(p->lik_logc), "%s: lik_logc is not finite", who);
-    PBX_REQUIRE(p->variant != 3,
-                "%s: variant 3 (sufficient statistics) needs the normal likelihood", who);
   }
+  PBX_REQUIRE(p->lik_kind == PBX_LIK_NORMAL || p->variant != 3,
+              "%s: variant 3 (sufficient statistics) needs the normal likelihood", who);
   for (int j = 0; j < p->n_params; ++j) {
     PBX_REQUIRE(p->lims[j][1] > p->lims[j][0], "%s: empty prior box for parameter %d", who, j);
     PBX_REQUIRE(!p->log_ufun[j] || p->lims[j][0] > 0.0,
@@ -735,10 +793,15 @@ static int nr_launch_tiles(pbx_ctx* ctx, const NrPlan& pl, const NrArgs& a, cons
                                                                                pl.use_tma, lik); \
   } while (0)
   const bool ex = nr_extras(a, m);
-  if (m.has_slope && ex) NR_TILES_GO(true, true);
-  else if (m.has_slope) NR_TILES_GO(true, false);
-  else if (ex) NR_TILES_GO(false, true);
-  else NR_TILES_GO(false, false);
+  if constexpr (kLik == PBX_LIK_STUDENT_T_NU) {         // (mu, sigma, nu): never a slope
+    if (ex) NR_TILES_GO(false, true);
+    else NR_TILES_GO(false, false);
+  } else {
+    if (m.has_slope && ex) NR_TILES_GO(true, true);
+    else if (m.has_slope) NR_TILES_GO(true, false);
+    else if (ex) NR_TILES_GO(false, true);
+    else NR_TILES_GO(false, false);
+  }
 #undef NR_TILES_GO
   PBX_LAUNCH_CHECK(ctx);
   return PBX_OK;
@@ -755,10 +818,15 @@ static int nr_launch_stream(pbx_ctx* ctx, const NrPlan& pl, const NrArgs& a, con
         a, m, pl.use_tma, lik);                                                                \
   } while (0)
   const bool ex = nr_extras(a, m);
-  if (m.has_slope && ex) NR_STREAM_GO(true, true);
-  else if (m.has_slope) NR_STREAM_GO(true, false);
-  else if (ex) NR_STREAM_GO(false, true);
-  else NR_STREAM_GO(false, false);
+  if constexpr (kLik == PBX_LIK_STUDENT_T_NU) {
+    if (ex) NR_STREAM_GO(false, true);
+    else NR_STREAM_GO(false, false);
+  } else {
+    if (m.has_slope && ex) NR_STREAM_GO(true, true);
+    else if (m.has_slope) NR_STREAM_GO(true, false);
+    else if (ex) NR_STREAM_GO(false, true);
+    else NR_STREAM_GO(false, false);
+  }
 #undef NR_STREAM_GO
   PBX_LAUNCH_CHECK(ctx);
   return PBX_OK;
@@ -784,9 +852,11 @@ static int nr_launch_step_lik(pbx_ctx* ctx, const NrPlan& pl, const NrArgs& a, c
 
 static int nr_launch_step(pbx_ctx* ctx, const NrPlan& pl, const NrArgs& a, const NrModel& m,
                           int lik_kind, const NrLik& lik) {
-  return lik_kind == PBX_LIK_STUDENT_T
-             ? nr_launch_step_lik<PBX_LIK_STUDENT_T>(ctx, pl, a, m, lik)
-             : nr_launch_step_lik<PBX_LIK_NORMAL>(ctx, pl, a, m, lik);
+  switch (lik_kind) {
+    case PBX_LIK_STUDENT_T: return nr_launch_step_lik<PBX_LIK_STUDENT_T>(ctx, pl, a, m, lik);
+    case PBX_LIK_STUDENT_T_NU: return nr_launch_step_lik<PBX_LIK_STUDENT_T_NU>(ctx, pl, a, m, lik);
+    default: return nr_launch_step_lik<PBX_LIK_NORMAL>(ctx, pl, a, m, lik);
+  }
 }
 
 // ============================================================================
@@ -983,7 +1053,8 @@ __global__ void __launch_bounds__(32 * RW_WARPS)
   if (c >= a.C) return;
   const int64_t C = a.C;
   const int n = (int)a.N;
-  constexpr int P = kSlope ? 3 : 2;           // has_slope <=> (b0, b1, sigma), validated by the host
+  // (b0, b1, sigma) with a slope, (mu, sigma, nu) for the sampled-nu t, else (mu, sigma)
+  constexpr int P = (kSlope || kLik == PBX_LIK_STUDENT_T_NU) ? 3 : 2;
   double th[PBX_MAX_PARAMS], ssum[PBX_MAX_PARAMS], ssq[PBX_MAX_PARAMS];
   _Pragma("unroll") for (int j = 0; j < P; ++j) {
     th[j] = a.state[(int64_t)j * C + c];
@@ -998,7 +1069,8 @@ __global__ void __launch_bounds__(32 * RW_WARPS)
       const double r = kSlope ? (sy[i] - b0) - b1 * sx[i] : sy[i] - b0;
       // if constexpr: the normal instantiation captures no more than the normal-only kernel
       // did, which keeps its SASS byte-identical (a runtime-dead capture reorders registers)
-      if constexpr (kLik == PBX_LIK_STUDENT_T) return log1p((r * r) * nr_q<kLik>(lik, t[P - 1]));
+      if constexpr (kLik == PBX_LIK_STUDENT_T_NU) return log1p((r * r) * nr_q(t[1], t[2]));
+      else if constexpr (kLik == PBX_LIK_STUDENT_T) return log1p((r * r) * nr_q(t[P - 1], lik.df));
       else return r * r;
     };
     int i = lane;
@@ -1151,10 +1223,15 @@ static int nr_walk_small(pbx_ctx* ctx, const NrArgs& a, const NrModel& m, const 
                                   cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));    \
     rw_walk_kernel<S, L, kLik><<<grid, 32 * wpc, smem, ctx->stream>>>(a, m, lik);              \
   } while (0)
-  if (m.has_slope && m.has_L) RW_GO(true, true);
-  else if (m.has_slope) RW_GO(true, false);
-  else if (m.has_L) RW_GO(false, true);
-  else RW_GO(false, false);
+  if constexpr (kLik == PBX_LIK_STUDENT_T_NU) {
+    if (m.has_L) RW_GO(false, true);
+    else RW_GO(false, false);
+  } else {
+    if (m.has_slope && m.has_L) RW_GO(true, true);
+    else if (m.has_slope) RW_GO(true, false);
+    else if (m.has_L) RW_GO(false, true);
+    else RW_GO(false, false);
+  }
 #undef RW_GO
   PBX_LAUNCH_CHECK(ctx);
   return PBX_OK;
@@ -1183,7 +1260,6 @@ extern "C" int pbx_mh_normreg_run(pbx_ctx* ctx, const pbx_mh_normreg_params* p) 
   nr_fill_model(p, m);
   NrArgs a = nr_args(p);
   const NrLik lik{p->lik_df, p->lik_logc};
-  const bool t_lik = p->lik_kind == PBX_LIK_STUDENT_T;
   // variant 3: sufficient statistics, else a small problem: the walk in one launch;
   // otherwise one launch per step
   const bool suffstat = p->variant == 3, small = !suffstat && rw_applies(p);
@@ -1201,8 +1277,9 @@ extern "C" int pbx_mh_normreg_run(pbx_ctx* ctx, const pbx_mh_normreg_params* p) 
   if (a.T > 0) {
     if (suffstat) rc = nr_walk_suffstat(ctx, a, m);
     else if (small)
-      rc = t_lik ? nr_walk_small<PBX_LIK_STUDENT_T>(ctx, a, m, lik)
-                 : nr_walk_small<PBX_LIK_NORMAL>(ctx, a, m, lik);
+      rc = p->lik_kind == PBX_LIK_STUDENT_T      ? nr_walk_small<PBX_LIK_STUDENT_T>(ctx, a, m, lik)
+           : p->lik_kind == PBX_LIK_STUDENT_T_NU ? nr_walk_small<PBX_LIK_STUDENT_T_NU>(ctx, a, m, lik)
+                                                 : nr_walk_small<PBX_LIK_NORMAL>(ctx, a, m, lik);
     else rc = nr_walk_per_step(ctx, pl, a, m, p->lik_kind, lik);
     if (rc) return rc;
   }

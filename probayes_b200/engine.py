@@ -345,7 +345,11 @@ class Engine:
                                       "(b0, b1, sigma) parameters, got %d" % P)
         if accept not in _ACCEPT or prop not in _PROP:
             raise ValueError("unknown accept/prop mode: %r / %r" % (accept, prop))
-        has_slope = P == 3
+        # a sampled nu is the third parameter of (mu, sigma, nu); otherwise three are a slope's
+        sampled_nu = lik is not None and lik.get("df_param") is not None
+        has_slope = P == 3 and not sampled_nu
+        if sampled_nu and P != 3:
+            raise ValueError("the sampled-nu Student-t needs parameters (mu, sigma, nu)")
         if has_slope and x_obs is None:
             raise ValueError("x_obs is required for the regression likelihood")
         p = MhNormregParams()
@@ -376,7 +380,9 @@ class Engine:
             p.has_prop_mat = 1
             for i, v in enumerate(L.ravel()):
                 p.prop_mat[i] = v
-        if lik is not None:
+        if sampled_nu:
+            p.lik_kind = _lib.LIK_STUDENT_T_NU          # nu and logc(nu) per chain, on the device
+        elif lik is not None:
             p.lik_kind = _lib.LIK_STUDENT_T
             p.lik_df, p.lik_logc = float(lik["df"]), float(lik["logc"])
         return p
@@ -392,7 +398,9 @@ class Engine:
         lower-triangular factor every delta is multiplied by before the ufun move
         (set_tran(covariance), rf.py:346-348), injected deltas included.  ``lik``: the
         likelihood family, None (normal) or a Student-t dict(df=nu, logc=...) as
-        ``catalogue.likelihood`` returns; the t has no sufficient statistics (no variant 3)."""
+        ``catalogue.likelihood`` returns, or dict(family='t', df_param=name) for a t whose nu
+        is sampled as the third parameter of (mu, sigma, nu); the t has no sufficient
+        statistics (no variant 3)."""
         torch = _torch()
         P, C_ = state.shape
         T = int(steps)
@@ -444,6 +452,9 @@ class Engine:
         ``lik``: as :meth:`mh_normreg`'s; a Student-t sums t.logpdf and has no suffstat."""
         M, S = int(mu.numel()), int(sigma.numel())
         extra = ()
+        if lik is not None and lik.get("df_param") is not None:
+            raise NotImplementedError("the (mu, sigma) grid needs a fixed nu: a grid over nu "
+                                      "would be a three-axis grid")
         if lik is not None:
             if suffstat:
                 raise ValueError("suffstat=True needs the normal likelihood: the Student-t "

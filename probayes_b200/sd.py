@@ -161,6 +161,8 @@ class SD:
     def __call__(self, values=None, iid=False, joint=False, **kwds):
         """model({x: data, 'mu': {M}, 'sigma': {S}}, iid=True, joint=True) -> PD of the
         log-joint over the (mu, sigma) grid (examples/dgei/dgei_norm1d_improved.py:36-37).
+        A Student-t whose nu is a model parameter takes nu as a scalar value ('nu': 4.) and
+        gives the (mu, sigma) grid at that nu, its prior included when ``joint``.
         ``suffstat=True`` (new, opt-in): evaluate it from centred sufficient statistics of
         the observations -- O(M S) instead of O(N M S), same values to fp64 round-off."""
         suffstat = bool(kwds.pop('suffstat', False))
@@ -175,7 +177,18 @@ class SD:
             raise NotImplementedError("the un-reduced [N, M, S] likelihood tensor is never "
                                       "materialised on the device: call with iid=True")
         catalogue.refuse_suffstat(spec, 3 if suffstat else 0)
-        obs, (kmu, ksg) = spec['obs_y'], spec['params']
+        obs, (kmu, ksg) = spec['obs_y'], spec['params'][:2]
+        lik = spec.get('lik')
+        knu = (lik or {}).get('df_param')
+        if knu is not None:
+            nu = values.get(knu)
+            if nu is None:
+                raise ValueError("values must give the degrees of freedom '{}' a scalar".format(knu))
+            if isunitsetint(nu) or np.ndim(nu) > 0:
+                raise NotImplementedError("a grid over '{}' would be a three-axis (mu, sigma, nu) "
+                                          "grid: give it a scalar value".format(knu))
+            nu = float(nu)
+            lik = catalogue.likelihood('t', nu)        # the fixed-nu grid at this nu
         data = np.ascontiguousarray(np.ravel(np.asarray(values[obs], dtype=np.float64)))
         grids = {}
         for key in (kmu, ksg):
@@ -190,12 +203,15 @@ class SD:
             from .pscales import rescale
             lpm = rescale(lpm, self._roots[kmu].pscale, 'log')
             lps = rescale(lps, self._roots[ksg].pscale, 'log')
+            if knu is not None:                        # nu's prior: the same for every cell
+                lpm = lpm + float(rescale(self._roots[knu].eval_prob(nu),
+                                          self._roots[knu].pscale, 'log'))
         else:
             lpm, lps = np.zeros(M), np.zeros(S)
         eng = get_engine()
         lj = eng.grid_norm_logjoint(eng.to_device(data), eng.to_device(grids[kmu]),
                                     eng.to_device(grids[ksg]), eng.to_device(lpm),
-                                    eng.to_device(lps), suffstat=suffstat, lik=spec.get('lik'))
+                                    eng.to_device(lps), suffstat=suffstat, lik=lik)
         order = [k for k in self._roots.keylist if k in (kmu, ksg)]
         vals = collections.OrderedDict()
         dims = collections.OrderedDict()
@@ -205,9 +221,13 @@ class SD:
         if order[0] != kmu:
             lj = lj.t().contiguous()
             dims = collections.OrderedDict((k, 1 - d) for k, d in dims.items())
+        fixed = []
+        if knu is not None:
+            vals[knu], dims[knu] = nu, None
+            fixed = ["{}={}".format(knu, nu)]
         vals[obs] = {len(data)}
         dims[obs] = None
-        names = [k + "=[]" for k in order] + ["{}={{{}}}".format(obs, len(data))]
-        cond = "" if joint else "|" + ",".join(k + "=[]" for k in order)
+        names = [k + "=[]" for k in order] + fixed + ["{}={{{}}}".format(obs, len(data))]
+        cond = "" if joint else "|" + ",".join([k + "=[]" for k in order] + fixed)
         name = ",".join(names) if joint else names[-1] + cond
         return PD(name, vals, dims=dims, prob=lj, pscale=self._pscale)
